@@ -2,6 +2,7 @@
 """bench.py -- RA-LENet training-step throughput on B200 (BASELINE.json metric: ECG windows/s).
 
     python bench.py --gpus N --steps K --warmup W            # one rank per GPU under torchrun for N > 1
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/*.npy
     python bench.py --impl reference ...                     # the UNMODIFIED reference on this box's host cores
     python bench.py --impl reference-gpu ...                 # the UNMODIFIED reference, eager PyTorch, on the B200
 
@@ -53,6 +54,8 @@ WORKLOAD = ("configs[1]: RA-LENet training step (fwd+bwd+Adam, MSE, lr 1e-3), {b
 FLOPS_PER_WINDOW_TRAIN = 184_665_984       # torch.utils.flop_counter on the reference, SURVEY 8d
 BYTES_PER_WINDOW_TRAIN = 2_347_008         # fp32 activations, per-half-block schedule, SURVEY 8d
 ADAM_BYTES_PER_STEP = 7 * 4 * 1_087_282
+# --dump-outputs writes at most this many windows (32 MiB of `out`), so that a dump stays under 64 MB with the model state
+DUMP_MAX_WINDOWS = 16384
 
 
 def workload_config(world: int, B: int, graph: bool = True):
@@ -615,6 +618,24 @@ def dropin_record(dev, sd, B, steps, warmup):
                           "what": "the same loop, optimizer line changed to ecg_denoise_b200.optim.Adam(model, lr=1e-3)"}}
 
 
+def dump_outputs(path, loss, rmse, snr, out, model):
+    """--dump-outputs: what the last timed step returned (loss, per-window RMSE and SNR, the denoised windows) and the
+    model state it left (every floating-point state_dict tensor, flattened and concatenated in state_dict order), as
+    <path>/<name>.npy.  Above DUMP_MAX_WINDOWS windows, the same seeded sample of windows is written every run."""
+    import numpy as np
+    import torch
+    arrays = {"loss": loss, "rmse": rmse, "snr": snr, "out": out}
+    if out.shape[0] > DUMP_MAX_WINDOWS:
+        idx = np.sort(np.random.default_rng(0).choice(out.shape[0], DUMP_MAX_WINDOWS, replace=False))
+        idx = torch.from_numpy(idx).to(out.device)
+        arrays.update({k: arrays[k].index_select(0, idx) for k in ("rmse", "snr", "out")})
+    arrays["model_state"] = torch.cat([t.detach().reshape(-1) for t in model.state_dict().values()
+                                       if t.is_floating_point()])
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().cpu().numpy())
+
+
 def timed_train(trainer, dx, dt, steps, warmup, barrier):
     import torch
     NB = dx.shape[0]
@@ -728,7 +749,14 @@ def main():
     ap.add_argument("--workload", default="train", choices=["train", "infer", "train12"],
                     help="train = configs[1] (default, the headline); infer = configs[4] record inference; "
                          "train12 = configs[2] 12-lead fine-tuning")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed (loss, rmse, snr, out, model_state) "
+                         "as DIR/<name>.npy; the inputs depend only on the arguments, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "train"):
+        ap.error("--dump-outputs applies to the default training workload (--impl b200 --workload train)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -793,6 +821,8 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     final_loss = float(loss.item())
+    if args.dump_outputs and rank == 0:           # before the end-to-end loop below trains the model further
+        dump_outputs(args.dump_outputs, loss, rmse, snr, out, model)
 
     # ---- end to end: pinned host batch -> H2D -> step -> D2H loss ---------------------------------------
     for i in range(3):                            # warm-up of the same loop (staging buffers, copy stream, pinned slots)

@@ -3,7 +3,8 @@ from the reference root) driven for 2 epochs on synthetic loaders.  TEST INFRAST
 
 Used twice: by `oracle/make_golden_dropin.py` with the reference's model on the CPU (-> tests/golden/dropin_golden.json)
 and by `tests/test_dropin_driver.py` with `ecg_denoise_b200.install()` on the B200.  `global_utils` (un-vendored by the
-reference) comes from the test-only shim in tests/shim/.
+reference) comes from the test-only shim in tests/shim/.  `stock_train` restates the same loop so that the numbers of
+the golden file are also checked where the reference is not at hand.
 """
 from __future__ import annotations
 
@@ -56,3 +57,45 @@ def run_train(ref_root: str, model, use_gpu: bool):
         finally:
             os.chdir(cwd)
     return [list(map(float, r)) for r in res], line
+
+
+def stock_train(model):
+    """the loop of denoise_train.train on the GPU, restated: model.cuda(), Adam(lr 1e-3); every epoch, train mode over
+    the training batches (zero_grad, model(data), F.mse_loss, loss.item(), backward, step, per-window SNR / RMSE of
+    that output), then eval mode over the test batches (without torch.no_grad, as the reference runs it).  Returns
+    (train_snr, test_snr, train_rmse, test_rmse), each the per-epoch mean over windows, like run_train."""
+    import torch.nn.functional as F
+    from oracle.ralenet_oracle import RMSE, SNR
+    tr, te = loaders()
+    model = model.cuda()
+    opt = torch.optim.Adam(model.parameters(), lr=0.001)
+
+    def metrics(target, pre):
+        t, p = target.double(), pre.detach().cpu().double()
+        return SNR(t, p), RMSE(t, p)
+
+    res = [[], [], [], []]
+    for _ in range(EPOCHS):
+        model.train()
+        snr, rmse = [], []
+        for data, target in tr:
+            opt.zero_grad()
+            pre = model(data.cuda())
+            loss = F.mse_loss(pre, target.cuda())
+            loss.item()
+            loss.backward()
+            opt.step()
+            s, r = metrics(target, pre)
+            snr.append(s)
+            rmse.append(r)
+        res[0].append(float(torch.cat(snr).mean()))
+        res[2].append(float(torch.cat(rmse).mean()))
+        model.eval()
+        snr, rmse = [], []
+        for data, target in te:
+            s, r = metrics(target, model(data.cuda()))
+            snr.append(s)
+            rmse.append(r)
+        res[1].append(float(torch.cat(snr).mean()))
+        res[3].append(float(torch.cat(rmse).mean()))
+    return res
