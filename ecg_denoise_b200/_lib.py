@@ -97,6 +97,8 @@ def load():
     lib.ralenet_abi_version.restype = ctypes.c_int
     lib.ralenet_net_workspace_bytes.restype = ctypes.c_uint64
     lib.ralenet_net_workspace_bytes.argtypes = [ctypes.c_int32] * 3
+    lib.ralenet_net_workspace_bytes_ex.restype = ctypes.c_uint64
+    lib.ralenet_net_workspace_bytes_ex.argtypes = [ctypes.c_int32] * 4
     lib.ralenet_launch_count.restype = ctypes.c_int64
     lib.ralenet_launch_count.argtypes = [ctypes.c_int32]
     lib.ralenet_check_device.argtypes = [ctypes.c_int]
@@ -130,6 +132,23 @@ _checked_devices = set()
 def check(rc: int):
     if rc != 0:
         raise RalenetError(f"libralenet_b200 error {rc}: {load().ralenet_last_error().decode()}")
+
+
+def deterministic_guard(what: str) -> None:
+    """Behave like a PyTorch op without a deterministic implementation when `what` (a path of this package whose
+    parameter gradients are accumulated with floating-point atomics) runs under torch.use_deterministic_algorithms(True):
+    raise RuntimeError, or warn when the flag was set with warn_only=True.  Does nothing when the flag is off."""
+    import torch
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = (f"{what} does not have a deterministic implementation, but you set "
+           "'torch.use_deterministic_algorithms(True)'. The whole-network paths (ralenet modules, FusedTrainer on one "
+           "GPU) are deterministic under that flag; see INTEGRATION.md section 4.")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        import warnings
+        warnings.warn(msg)
+    else:
+        raise RuntimeError(msg)
 
 
 def check_device(index: int):

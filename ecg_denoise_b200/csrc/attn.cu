@@ -179,7 +179,7 @@ size_t attn_bwd_smem(int L) {
   return sizeof(float) * (8 * (size_t)L * ld_mk(C) + 2 * ((size_t)L * C / 4) + attn_bwd_swf<C>() + 256 + 2 * C);
 }
 
-template <int C, int WIN>
+template <int C, int WIN, bool DET>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_bwd_kernel(const rl_attn_bwd_args a) {
   extern __shared__ __align__(16) float smem[];
   constexpr int L = 2048 * WIN / C, H = C / RL_HD;
@@ -279,7 +279,8 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_bwd_kernel(const rl_attn_
     static_assert(CtaWgrad<C, C, L>::SCRATCH <= LP, "attn_bwd: scratch");
     CtaWgrad<C, C, L>::partial(sdq, LDC, sdk, LDC, su);
     __syncthreads();
-    CtaWgrad<C, C, L>::reduce(su, a.d_wp, a.d_bp);
+    CtaWgrad<C, C, L>::template reduce<DET>(su, grad_slot<DET>(a.d_wp, C * C, blockIdx.x),
+                                            grad_slot<DET>(a.d_bp, C, blockIdx.x));
   }
   RL_TS(attn, 4);
 
@@ -296,14 +297,16 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_bwd_kernel(const rl_attn_
   float* sds_c = (a.d_table != nullptr && W > 0) ? su : nullptr;      // su is free until step 6 (H * W * W <= LP floats)
   attn_core_bwd_single<C, L>(sq, sk, sv, sdo, sD, sLse, sdq, sdk, sdv, stab, sds_c, W, c0, 1.0f / do_scale);
   __syncthreads();
-  if (sds_c != nullptr)           // d_table[i - j + W - 1][h] += sum over the diagonal of the central block of dS
+  if (sds_c != nullptr) {         // d_table[i - j + W - 1][h] += sum over the diagonal of the central block of dS
+    float* d_table = grad_slot<DET>(a.d_table, (2 * W - 1) * H, blockIdx.x);
     for (int idx = tid; idx < (2 * W - 1) * H; idx += RL_NT) {
       const int rel = idx / H - (W - 1), h = idx % H;
       const int jlo = (rel < 0) ? -rel : 0, jhi = (rel > 0) ? W - rel : W;
       float s = 0.f;
       for (int j = jlo; j < jhi; ++j) s += sds_c[(h * W + j + rel) * W + j];
-      atomicAdd(a.d_table + idx, s);
+      grad_add<DET>(d_table + idx, s);
     }
+  }
   RL_TS(attn, 6);
 
   // 5. dqkv scratch [t][dq | dk | dv] for the weight-gradient GEMMs
@@ -357,7 +360,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_bwd_kernel(const rl_attn_
           *reinterpret_cast<float4*>(FW ? su + t * LDC + c : uw + t * C + c) = u;
         });
     __syncthreads();
-    ln_backward_finish<C>(sq, a.d_ln_w, a.d_ln_b);
+    ln_backward_finish<C, DET>(sq, grad_slot<DET>(a.d_ln_w, C, blockIdx.x), grad_slot<DET>(a.d_ln_b, C, blockIdx.x));
   } else {
     for (int i = tid; i < LC; i += RL_NT) {
       const int t = i / C, c = i % C;
@@ -374,9 +377,11 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_bwd_kernel(const rl_attn_
     WG::partial(sdk, LDC, su, LDC, sv);
     WG::partial(sdv, LDC, su, LDC, sdo);
     __syncthreads();
-    WG::reduce(sk, a.d_wq, a.d_bq);
-    WG::reduce(sv, a.d_wkv, a.d_bkv);
-    WG::reduce(sdo, a.d_wkv ? a.d_wkv + C * C : nullptr, a.d_bkv ? a.d_bkv + C : nullptr);
+    float* d_wkv = grad_slot<DET>(a.d_wkv, 2 * C * C, blockIdx.x);
+    float* d_bkv = grad_slot<DET>(a.d_bkv, 2 * C, blockIdx.x);
+    WG::template reduce<DET>(sk, grad_slot<DET>(a.d_wq, C * C, blockIdx.x), grad_slot<DET>(a.d_bq, C, blockIdx.x));
+    WG::template reduce<DET>(sv, d_wkv, d_bkv);
+    WG::template reduce<DET>(sdo, d_wkv ? d_wkv + C * C : nullptr, d_bkv ? d_bkv + C : nullptr);
   }
   RL_TS(attn, 10);
 }
@@ -431,18 +436,31 @@ int launch_fwd(const rl_attn_fwd_args* a, cudaStream_t st) {
   return launch_fwd_groups<C, 1>(&rest, st, &d1);
 }
 
-template <int C>
-int launch_bwd(const rl_attn_bwd_args* a, cudaStream_t st) {
-  const int win = a->L * C / 2048;
+template <int C, int WIN, bool DET>
+int launch_bwd_one(const rl_attn_bwd_args* a, cudaStream_t st) {
   const size_t smem = attn_bwd_smem<C>(a->L);
-  if (win == 1) {
-    if (int rc = rl_set_smem(attn_bwd_kernel<C, 1>, smem)) return rc;
-    rl_launch_pdl(attn_bwd_kernel<C, 1>, dim3(a->B), dim3(RL_NT), smem, st, *a);
-  } else {
-    if (int rc = rl_set_smem(attn_bwd_kernel<C, 2>, smem)) return rc;
-    rl_launch_pdl(attn_bwd_kernel<C, 2>, dim3(a->B), dim3(RL_NT), smem, st, *a);
-  }
+  if (int rc = rl_set_smem(attn_bwd_kernel<C, WIN, DET>, smem)) return rc;
+  rl_launch_pdl(attn_bwd_kernel<C, WIN, DET>, dim3(a->B), dim3(RL_NT), smem, st, *a);
   return rl_check_launch("attn_bwd_kernel", C);
+}
+
+// det: one partial slot per window (CTA) for the in-CTA gradients (LayerNorm, R-wave table; every weight at C <= 16)
+template <int C>
+int launch_bwd(const rl_attn_bwd_args* a, cudaStream_t st, RlDet* det) {
+  const int win = a->L * C / 2048;
+  if (det == nullptr) return win == 1 ? launch_bwd_one<C, 1, false>(a, st) : launch_bwd_one<C, 2, false>(a, st);
+  rl_attn_bwd_args d = *a;
+  const int B = a->B;
+  d.d_ln_w = rl_det_take(det, a->d_ln_w, C, B);
+  d.d_ln_b = rl_det_take(det, a->d_ln_b, C, B);
+  d.d_table = (a->W > 0) ? rl_det_take(det, a->d_table, (2 * a->W - 1) * (C / RL_HD), B) : nullptr;
+  if (C <= RL_FW_MAXC) {
+    d.d_wq = rl_det_take(det, a->d_wq, C * C, B);   d.d_bq = rl_det_take(det, a->d_bq, C, B);
+    d.d_wkv = rl_det_take(det, a->d_wkv, 2 * C * C, B); d.d_bkv = rl_det_take(det, a->d_bkv, 2 * C, B);
+    d.d_wp = rl_det_take(det, a->d_wp, C * C, B);   d.d_bp = rl_det_take(det, a->d_bp, C, B);
+  }
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "attn_bwd: deterministic-mode workspace too small");
+  return win == 1 ? launch_bwd_one<C, 1, true>(&d, st) : launch_bwd_one<C, 2, true>(&d, st);
 }
 
 int check_shape(int B, int L, int C, int H, int W, int c0) {
@@ -534,7 +552,7 @@ extern "C" int ralenet_attn_fwd(const rl_attn_fwd_args* a, void* stream) {
 }
 
 // the data-gradient kernel (also writes the dqkv / u scratch of the weight gradients)
-int rl_attn_bwd_main(const rl_attn_bwd_args* a, cudaStream_t st) {
+int rl_attn_bwd_main(const rl_attn_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(a, RL_ERR_NULL, "attn_bwd: args is NULL");
   if (int rc = check_shape(a->B, a->L, a->C, a->H, a->W, a->c0)) return rc;
   RL_REQUIRE(a->g && a->x && a->wq && a->wkv && a->wp && a->q && a->k && a->v && a->o && a->lse && a->dx && a->dqkv &&
@@ -547,11 +565,11 @@ int rl_attn_bwd_main(const rl_attn_bwd_args* a, cudaStream_t st) {
                      a->dqkv, a->u),
              RL_ERR_SHAPE, "attn_bwd: tensors must be 16-byte aligned");
   switch (a->C) {
-    case 8: return launch_bwd<8>(a, st);
-    case 16: return launch_bwd<16>(a, st);
-    case 32: return launch_bwd<32>(a, st);
-    case 64: return launch_bwd<64>(a, st);
-    case 128: return launch_bwd<128>(a, st);
+    case 8: return launch_bwd<8>(a, st, det);
+    case 16: return launch_bwd<16>(a, st, det);
+    case 32: return launch_bwd<32>(a, st, det);
+    case 64: return launch_bwd<64>(a, st, det);
+    case 128: return launch_bwd<128>(a, st, det);
   }
   return RL_ERR_SHAPE;
 }
@@ -562,13 +580,13 @@ bool rl_attn_bwd_has_wgrad(const rl_attn_bwd_args* a) {
 }
 
 // weight gradients from (g, o) and the scratch tensors; may run on another stream once the main kernel is done
-int rl_attn_bwd_wgrad(const rl_attn_bwd_args* a, cudaStream_t st) {
+int rl_attn_bwd_wgrad(const rl_attn_bwd_args* a, cudaStream_t st, RlDet* det) {
   const int M = a->B * a->L, C = a->C;
   if (C <= RL_FW_MAXC) return RL_OK;        // narrow stages accumulate their weight gradients inside the kernel
   const RlWgradDesc d[3] = {{a->g, C, a->o, C, C, C, a->d_wp, a->d_bp},
                             {a->dqkv, 3 * C, a->u, C, C, C, a->d_wq, a->d_bq},
                             {a->dqkv + C, 3 * C, a->u, C, 2 * C, C, a->d_wkv, a->d_bkv}};
-  return rl_launch_wgrad_group(d, 3, M, st);
+  return rl_launch_wgrad_group(d, 3, M, st, det);
 }
 
 extern "C" int ralenet_attn_bwd(const rl_attn_bwd_args* a, void* stream) {

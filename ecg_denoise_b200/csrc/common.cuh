@@ -257,6 +257,22 @@ __device__ __forceinline__ void copy_s2g(float* __restrict__ dst, const float* s
 }
 
 // ---------------------------------------------------------------------------------------------
+// Parameter-gradient output of a backward kernel.  Default: fp32 atomics into the gradient, so the low bits depend on
+// the order in which CTAs arrive.  Deterministic mode (DET, RL_NET_DETERMINISTIC): the gradient pointer handed to the
+// kernel is a partial slab [slots][n] (rl_det_take), every slot is written by exactly one CTA with plain stores, and
+// rl_launch_grad_reduce() later adds the slots up in slot order.  grad_slot() moves a slab pointer to the slot of the
+// calling CTA; the slot is a function of the work item only (window, tile, token slice), never of timing.
+template <bool DET>
+__device__ __forceinline__ void grad_add(float* p, float v) {
+  if constexpr (DET) *p = v;
+  else atomicAdd(p, v);
+}
+template <bool DET>
+__device__ __forceinline__ float* grad_slot(float* p, size_t n, int slot) {
+  return (DET && p != nullptr) ? p + (size_t)slot * n : p;
+}
+
+// ---------------------------------------------------------------------------------------------
 // LayerNorm over C channels of `rows` tokens (eps 1e-5, biased variance, like nn.LayerNorm).
 // A group of GS = min(C,32) lanes owns one token; each lane holds CPL = C/GS channels.
 // load(t, c) returns the pre-norm value; store(t, c, zhat, rstd_is_unused) receives zhat.
@@ -390,7 +406,8 @@ __device__ __forceinline__ void ln_backward_rows(int rows, const float* __restri
       });
 }
 // after a CTA barrier behind ln_backward_rows<C, true>: d_ln_w / d_ln_b += the per-warp partial rows
-template <int C>
+// (DET: d_ln_w / d_ln_b are this CTA's slots of partial slabs, see grad_add)
+template <int C, bool DET = false>
 __device__ __forceinline__ void ln_backward_finish(const float* s_part, float* __restrict__ d_ln_w,
                                                    float* __restrict__ d_ln_b) {
   if (d_ln_w == nullptr) return;
@@ -398,7 +415,7 @@ __device__ __forceinline__ void ln_backward_finish(const float* s_part, float* _
     float s = 0.f;
 #pragma unroll
     for (int w = 0; w < RL_NT / 32; ++w) s += s_part[w * 2 * C + i];
-    atomicAdd((i < C) ? d_ln_w + i : d_ln_b + i - C, s);
+    grad_add<DET>((i < C) ? d_ln_w + i : d_ln_b + i - C, s);
   }
 }
 
@@ -840,7 +857,7 @@ __device__ __forceinline__ void cta_wgrad(const float* A, int lda, const float* 
 //     (A(m = n_out, k = token) = A[t*lda + n], B(k = token, n = k_in) = B[t*ldb + k]) and leaves its fragment in
 //     `scratch`; the warps of the first column tile also sum their A fragments over the tokens: the bias gradient.
 //   reduce(): (after the barrier) adds the KS fragments of every element and issues one red.global per element of dW /
-//     db and CTA.  No shared-memory atomics anywhere.
+//     db and CTA (DET: one store into the CTA's slab slot).  No shared-memory atomics anywhere.
 // Several partial()s into different scratch regions can share the barrier.
 template <int N, int K, int L>
 struct CtaWgrad {
@@ -884,6 +901,7 @@ struct CtaWgrad {
     }
   }
 
+  template <bool DET = false>
   __device__ static __forceinline__ void reduce(const float* scratch, float* __restrict__ dW, float* __restrict__ db) {
     if (dW != nullptr) {
       for (int e = threadIdx.x; e < TILES * 128; e += RL_NT) {
@@ -892,7 +910,7 @@ struct CtaWgrad {
 #pragma unroll
         for (int ks = 0; ks < KS; ++ks) s += scratch[(ks * TILES + tile) * ITEM + idx];
         const int m = (tile / NT) * 16 + (ln >> 2) + ((j & 2) ? 8 : 0), n = (tile % NT) * 8 + 2 * (ln & 3) + (j & 1);
-        if (m < N) atomicAdd(dW + m * K + n, s);
+        if (m < N) grad_add<DET>(dW + m * K + n, s);
       }
     }
     if (db != nullptr) {
@@ -901,7 +919,7 @@ struct CtaWgrad {
         float s = 0.f;
 #pragma unroll
         for (int ks = 0; ks < KS; ++ks) s += scratch[(ks * TILES + tile) * ITEM + 128 + (m % 16)];
-        atomicAdd(db + m, s);
+        grad_add<DET>(db + m, s);
       }
     }
   }
@@ -915,23 +933,49 @@ inline bool rl_al16(P... p) { return (((uintptr_t)p | ...) & 15) == 0; }
 // generic weight-gradient GEMM launcher (wgrad.cu):
 //   dW[n*K + k] += sum_m dY[m*ldy + n] * X[m*ldx + k]      n < N, k < K, m < M
 //   db[n]       += sum_m dY[m*ldy + n]                     (db may be NULL)
+struct RlDet;
 int rl_launch_wgrad(const float* dY, int ldy, const float* X, int ldx, int M, int N, int K, float* dW, float* db,
-                    cudaStream_t st);
+                    cudaStream_t st, RlDet* det = nullptr);
 // grouped form: all weight matrices of one half-block in one launch (tensor-core path when every dim % 32 == 0)
 struct RlWgradDesc {
   const float* dY; int ldy; const float* X; int ldx; int N, K; float* dW; float* db;
 };
-int rl_launch_wgrad_group(const RlWgradDesc* d, int n, int M, cudaStream_t st);
+int rl_launch_wgrad_group(const RlWgradDesc* d, int n, int M, cudaStream_t st, RlDet* det = nullptr);
+
+// Deterministic-mode bookkeeping of one backward kernel and its weight-gradient GEMMs (net.cu): the partial slabs
+// are carved from `slab` (cap floats) and every slab is recorded with the gradient it stands in for.
+constexpr int RL_DET_MAXRED = 16;
+constexpr int RL_DET_MAX_SPLIT = 148;   // token slices of a weight-gradient GEMM at most (bounds the slab size)
+struct RlGradRed {
+  const float* src;   // [slots][n]
+  float* dst;         // [n] += sum over the slots, in slot order
+  int n, slots;
+};
+struct RlDet {
+  float* slab;
+  size_t cap, used;
+  RlGradRed red[RL_DET_MAXRED];
+  int nred;
+};
+// slab region of slots x n floats standing in for gradient g (nullptr when g is nullptr or on overflow, with an error
+// set: check rl_det_ok()); slab regions are 16-byte aligned
+float* rl_det_take(RlDet* d, float* g, size_t n, int slots);
+bool rl_det_ok(const RlDet* d);
+// dst += sum over slots for every recorded slab, in one launch; clears the record
+int rl_launch_grad_reduce(RlDet* d, cudaStream_t st);
 
 // backward halves split into the data-gradient kernel and the weight-gradient GEMMs (net.cu runs the latter on a
-// side stream, off the critical path of the backward chain)
-int rl_attn_bwd_main(const rl_attn_bwd_args* a, cudaStream_t st);
-int rl_attn_bwd_wgrad(const rl_attn_bwd_args* a, cudaStream_t st);
+// side stream, off the critical path of the backward chain).  det != nullptr: deterministic mode, the parameter
+// gradients go to partial slabs recorded in *det (main and wgrad of one kernel share it)
+int rl_attn_bwd_main(const rl_attn_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
+int rl_attn_bwd_wgrad(const rl_attn_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
 bool rl_attn_bwd_has_wgrad(const rl_attn_bwd_args* a);
-int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st);
-int rl_ffn_bwd_wgrad(const rl_ffn_bwd_args* a, cudaStream_t st);
+int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
+int rl_ffn_bwd_wgrad(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
 bool rl_ffn_bwd_has_wgrad(const rl_ffn_bwd_args* a);
-int rl_patch_bwd_main(const rl_patch_bwd_args* a, cudaStream_t st);
-int rl_patch_bwd_wgrad(const rl_patch_bwd_args* a, cudaStream_t st);
+int rl_patch_bwd_main(const rl_patch_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
+int rl_patch_bwd_wgrad(const rl_patch_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
 bool rl_patch_bwd_has_wgrad(const rl_patch_bwd_args* a);
+int rl_head_bwd(const rl_head_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
+int rl_stem_bwd_apply(const rl_stem_bwd_args* a, cudaStream_t st, RlDet* det = nullptr);
 bool rl_prof_active();                 // per-launch profiling is on: keep every launch on the profiled stream

@@ -13,7 +13,7 @@
 
 // cluster kernels for the wide stages (ffn_cluster.cu); return 1 when the shape/mode is not handled there
 int rl_ffn_fwd_umma(const rl_ffn_fwd_args* a, cudaStream_t st);      // tcgen05 kernels (ffn_umma.cu)
-int rl_ffn_bwd_umma(const rl_ffn_bwd_args* a, cudaStream_t st);
+int rl_ffn_bwd_umma(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det);
 int rl_ffn_fwd_cluster(const rl_ffn_fwd_args* a, cudaStream_t st);
 int rl_ffn_bwd_cluster(const rl_ffn_bwd_args* a, cudaStream_t st);
 
@@ -45,7 +45,7 @@ size_t ffn_bwd_smem(int L, bool dw) {
                           ffn_bwd_swf<C>() + 3 * (size_t)L + 2 * C + 64);
 }
 
-template <int C, int WIN, bool DW>
+template <int C, int WIN, bool DW, bool DET>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_kernel(const rl_ffn_bwd_args a) {
   extern __shared__ __align__(16) float smem[];
   constexpr int L = 2048 * WIN / C;
@@ -189,7 +189,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_kernel(const rl_ffn_bw
         float s = 0.f;
 #pragma unroll
         for (int w = 0; w < RL_NT / 32; ++w) s += s_red[3 * w + tid];
-        atomicAdd(a.d_lew + tid, s);
+        grad_add<DET>(grad_slot<DET>(a.d_lew, 3, blockIdx.x) + tid, s);
       }
     } else if (DW) {
       for (int c = tid; c < HC; c += RL_NT) {
@@ -209,9 +209,10 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_kernel(const rl_ffn_bw
           dcur = dnxt;
         }
         if (a.d_lew) {
-          atomicAdd(a.d_lew + 3 * c, a0);
-          atomicAdd(a.d_lew + 3 * c + 1, a1);
-          atomicAdd(a.d_lew + 3 * c + 2, a2);
+          float* d_lew = grad_slot<DET>(a.d_lew, 3 * HC, blockIdx.x);
+          grad_add<DET>(d_lew + 3 * c, a0);
+          grad_add<DET>(d_lew + 3 * c + 1, a1);
+          grad_add<DET>(d_lew + 3 * c + 2, a2);
         }
       }
       __syncthreads();
@@ -250,7 +251,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_kernel(const rl_ffn_bw
           *reinterpret_cast<float4*>(FW ? su + t * LDC + c : uw + t * C + c) = fma4(zh, ldg4(lw + c), ldg4(lb + c));
         });
     __syncthreads();
-    ln_backward_finish<C>(sw, a.d_ln_w, a.d_ln_b);
+    ln_backward_finish<C, DET>(sw, grad_slot<DET>(a.d_ln_w, C, blockIdx.x), grad_slot<DET>(a.d_ln_b, C, blockIdx.x));
     if (FW) __syncthreads();                                        // sw is the weight-gradient scratch next
   } else {
     for (int i = tid; i < L * C; i += RL_NT) {
@@ -266,11 +267,11 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_kernel(const rl_ffn_bw
     static_assert(W2::SCRATCH <= ffn_bwd_swf<C>() && W1::SCRATCH <= ffn_bwd_swf<C>(), "ffn_bwd: scratch");
     W2::partial(sg, LDC, sg2, LDH, sw);
     __syncthreads();
-    W2::reduce(sw, a.d_w2, a.d_b2);
+    W2::template reduce<DET>(sw, grad_slot<DET>(a.d_w2, C * HC, blockIdx.x), grad_slot<DET>(a.d_b2, C, blockIdx.x));
     __syncthreads();
     W1::partial(sd, LDH, su, LDC, sw);
     __syncthreads();
-    W1::reduce(sw, a.d_w1, a.d_b1);
+    W1::template reduce<DET>(sw, grad_slot<DET>(a.d_w1, HC * C, blockIdx.x), grad_slot<DET>(a.d_b1, HC, blockIdx.x));
   }
 }
 
@@ -287,19 +288,38 @@ int launch_fwd(const rl_ffn_fwd_args* a, cudaStream_t st) {
   return rl_check_launch("ffn_fwd_kernel", C);
 }
 
-template <int C, int WIN, bool DW>
+template <int C, int WIN, bool DW, bool DET>
 int launch_bwd_one(const rl_ffn_bwd_args* a, cudaStream_t st) {
   const size_t smem = ffn_bwd_smem<C>(a->L, DW);
-  if (int rc = rl_set_smem(ffn_bwd_kernel<C, WIN, DW>, smem)) return rc;
-  rl_launch_pdl(ffn_bwd_kernel<C, WIN, DW>, dim3(a->B), dim3(RL_NT), smem, st, *a);
+  if (int rc = rl_set_smem(ffn_bwd_kernel<C, WIN, DW, DET>, smem)) return rc;
+  rl_launch_pdl(ffn_bwd_kernel<C, WIN, DW, DET>, dim3(a->B), dim3(RL_NT), smem, st, *a);
   return rl_check_launch("ffn_bwd_kernel", C);
 }
 
-template <int C>
-int launch_bwd(const rl_ffn_bwd_args* a, cudaStream_t st) {
+template <int C, bool DET>
+int launch_bwd_det(const rl_ffn_bwd_args* a, cudaStream_t st) {
   const bool dw = a->le_mode == RL_LE_DEPTHWISE;
-  if (a->L * C == 2048) return dw ? launch_bwd_one<C, 1, true>(a, st) : launch_bwd_one<C, 1, false>(a, st);
-  return dw ? launch_bwd_one<C, 2, true>(a, st) : launch_bwd_one<C, 2, false>(a, st);
+  if (a->L * C == 2048) return dw ? launch_bwd_one<C, 1, true, DET>(a, st) : launch_bwd_one<C, 1, false, DET>(a, st);
+  return dw ? launch_bwd_one<C, 2, true, DET>(a, st) : launch_bwd_one<C, 2, false, DET>(a, st);
+}
+
+// det: one partial slot per window (CTA) for the in-CTA gradients (LayerNorm, local enhancement; every weight at
+// C <= 16)
+template <int C>
+int launch_bwd(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
+  if (det == nullptr) return launch_bwd_det<C, false>(a, st);
+  rl_ffn_bwd_args d = *a;
+  const int B = a->B;
+  d.d_ln_w = rl_det_take(det, a->d_ln_w, C, B);
+  d.d_ln_b = rl_det_take(det, a->d_ln_b, C, B);
+  d.d_lew = (a->le_mode == RL_LE_NONE) ? nullptr
+                                       : rl_det_take(det, a->d_lew, a->le_mode == RL_LE_DEPTHWISE ? 12 * C : 3, B);
+  if (C <= RL_FW_MAXC) {
+    d.d_w1 = rl_det_take(det, a->d_w1, 4 * C * C, B); d.d_b1 = rl_det_take(det, a->d_b1, 4 * C, B);
+    d.d_w2 = rl_det_take(det, a->d_w2, 4 * C * C, B); d.d_b2 = rl_det_take(det, a->d_b2, C, B);
+  }
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "ffn_bwd: deterministic-mode workspace too small");
+  return launch_bwd_det<C, true>(&d, st);
 }
 
 int check_shape(int B, int L, int C, int le) {
@@ -337,7 +357,7 @@ extern "C" int ralenet_ffn_fwd(const rl_ffn_fwd_args* a, void* stream) {
   return RL_ERR_SHAPE;
 }
 
-int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st) {
+int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(a, RL_ERR_NULL, "ffn_bwd: args is NULL");
   if (int rc = check_shape(a->B, a->L, a->C, a->le_mode)) return rc;
   RL_REQUIRE(a->g && a->x && a->w1 && a->w2 && a->h && a->dx && a->dh && a->g2 && a->u, RL_ERR_NULL,
@@ -347,16 +367,16 @@ int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st) {
   RL_REQUIRE(!a->d_ln_w == !a->d_ln_b, RL_ERR_NULL, "ffn_bwd: d_ln_w/d_ln_b must be both set or both NULL");
   RL_REQUIRE(rl_al16(a->g, a->x, a->w1, a->w2, a->ln_w, a->ln_b, a->h, a->dx, a->dh, a->g2, a->u), RL_ERR_SHAPE,
              "ffn_bwd: tensors must be 16-byte aligned");
-  int rc = rl_ffn_bwd_umma(a, st);
+  int rc = rl_ffn_bwd_umma(a, st, det);
   if (rc < 0) return rc;
-  if (rc == 1) rc = rl_ffn_bwd_cluster(a, st);
+  if (rc == 1 && det == nullptr) rc = rl_ffn_bwd_cluster(a, st);   // (never reached: the tcgen05 kernels take its shapes)
   if (rc < 0) return rc;
   if (rc == 1) switch (a->C) {
-    case 8: rc = launch_bwd<8>(a, st); break;
-    case 16: rc = launch_bwd<16>(a, st); break;
-    case 32: rc = launch_bwd<32>(a, st); break;
-    case 64: rc = launch_bwd<64>(a, st); break;
-    case 128: rc = launch_bwd<128>(a, st); break;
+    case 8: rc = launch_bwd<8>(a, st, det); break;
+    case 16: rc = launch_bwd<16>(a, st, det); break;
+    case 32: rc = launch_bwd<32>(a, st, det); break;
+    case 64: rc = launch_bwd<64>(a, st, det); break;
+    case 128: rc = launch_bwd<128>(a, st, det); break;
   }
   return rc;
 }
@@ -364,12 +384,12 @@ int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st) {
 bool rl_ffn_bwd_has_wgrad(const rl_ffn_bwd_args* a) { return a->C > RL_FW_MAXC && (a->d_w1 || a->d_w2); }
 
 // weight gradients from (g, g2) and (dh, u); may run on another stream once the main kernel is done
-int rl_ffn_bwd_wgrad(const rl_ffn_bwd_args* a, cudaStream_t st) {
+int rl_ffn_bwd_wgrad(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   const int M = a->B * a->L, C = a->C;
   if (C <= RL_FW_MAXC) return RL_OK;        // narrow stages accumulate their weight gradients inside the kernel
   const RlWgradDesc d[2] = {{a->g, C, a->g2, 4 * C, C, 4 * C, a->d_w2, a->d_b2},
                             {a->dh, 4 * C, a->u, C, 4 * C, C, a->d_w1, a->d_b1}};
-  return rl_launch_wgrad_group(d, 2, M, st);
+  return rl_launch_wgrad_group(d, 2, M, st, det);
 }
 
 extern "C" int ralenet_ffn_bwd(const rl_ffn_bwd_args* a, void* stream) {

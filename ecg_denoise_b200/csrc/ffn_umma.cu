@@ -404,7 +404,7 @@ struct BwdSmem {
   static constexpr size_t BYTES = sizeof(float) * (2 * A_FLOATS + 4 * B_FLOATS + 2 * TM + 2 * C + 64) + 64;
 };
 
-template <int C>
+template <int C, bool DET>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_ffn_bwd_args a) {
   constexpr int L = 2048 / C, HC = 4 * C, NSL = HC / TS;
   // dgrad operand of fc2, B(n = hidden, k = c) = W2[c][128 r + n]: prefetched before the dependency wait
@@ -600,9 +600,10 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
         a1 = block_sum(a1, s_red);
         a2 = block_sum(a2, s_red);
         if (tid == 0) {
-          atomicAdd(a.d_lew, a0);
-          atomicAdd(a.d_lew + 1, a1);
-          atomicAdd(a.d_lew + 2, a2);
+          float* d_lew = grad_slot<DET>(a.d_lew, 3, tile);   // one slot per token tile (its rank-0 CTA)
+          grad_add<DET>(d_lew, a0);
+          grad_add<DET>(d_lew + 1, a1);
+          grad_add<DET>(d_lew + 2, a2);
         }
       }
     }
@@ -687,7 +688,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
             *reinterpret_cast<float4*>(uw + t * C + c) = fma4(zh, ldg4(lw + c), ldg4(lb + c));
           });
       __syncthreads();
-      ln_backward_finish<C>(sB, a.d_ln_w, a.d_ln_b);
+      ln_backward_finish<C, DET>(sB, grad_slot<DET>(a.d_ln_w, C, blockIdx.x), grad_slot<DET>(a.d_ln_b, C, blockIdx.x));
     } else {
       for (int i = tid; i < rows_here * C / 4; i += RL_NT) {
         const int t = (4 * i) / C, c = (4 * i) % C;
@@ -785,12 +786,24 @@ int rl_ffn_fwd_umma(const rl_ffn_fwd_args* a, cudaStream_t st) {
   return 1;
 }
 
-int rl_ffn_bwd_umma(const rl_ffn_bwd_args* a, cudaStream_t st) {
+template <int C>
+static int launch_bwd(const rl_ffn_bwd_args* a, int tiles, cudaStream_t st, RlDet* det) {
+  constexpr int NSL = 4 * C / TS;
+  if (det == nullptr)
+    return launch_cluster(ffn_bwd_umma_kernel<C, false>, BwdSmem<C>::BYTES, tiles * NSL, NSL, *a, st, "ffn_bwd_umma", C);
+  // det: LayerNorm partials one slot per CTA, local-enhancement taps one slot per token tile
+  rl_ffn_bwd_args d = *a;
+  d.d_ln_w = rl_det_take(det, a->d_ln_w, C, tiles * NSL);
+  d.d_ln_b = rl_det_take(det, a->d_ln_b, C, tiles * NSL);
+  d.d_lew = (a->le_mode == RL_LE_PARTIAL) ? rl_det_take(det, a->d_lew, 3, tiles) : nullptr;
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "ffn_bwd: deterministic-mode workspace too small");
+  return launch_cluster(ffn_bwd_umma_kernel<C, true>, BwdSmem<C>::BYTES, tiles * NSL, NSL, d, st, "ffn_bwd_umma", C);
+}
+
+int rl_ffn_bwd_umma(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   if (a->L * a->C != 2048 || a->le_mode == RL_LE_DEPTHWISE) return 1;
   const int tiles = (a->B * a->L + TM - 1) / TM;
-  if (a->C == 128)
-    return launch_cluster(ffn_bwd_umma_kernel<128>, BwdSmem<128>::BYTES, tiles * 4, 4, *a, st, "ffn_bwd_umma", 128);
-  if (a->C == 64)
-    return launch_cluster(ffn_bwd_umma_kernel<64>, BwdSmem<64>::BYTES, tiles * 2, 2, *a, st, "ffn_bwd_umma", 64);
+  if (a->C == 128) return launch_bwd<128>(a, tiles, st, det);
+  if (a->C == 64) return launch_bwd<64>(a, tiles, st, det);
   return 1;
 }

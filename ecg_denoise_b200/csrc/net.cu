@@ -6,9 +6,10 @@
 //        -> [2 @ s1] -> ps1 -> (+stem) head
 //
 // stage s: C = 8<<s channels, L = L0>>s tokens, H = 2<<s heads; every activation is L*C = 8*L0 floats
-// per window.  The workspace is carved deterministically from (B, L0, save) so forward and backward
+// per window.  The workspace is carved deterministically from (B, L0, save, flags) so forward and backward
 // agree on where each saved tensor lives.
 #include "common.cuh"
+#include <algorithm>
 
 namespace {
 
@@ -32,10 +33,39 @@ struct Ws {
   // weight-gradient GEMMs run on a side stream up to three kernels behind the data-gradient chain
   float *dqkv[2], *ua[2], *dh[2], *g2[2], *uf[2], *gsum, *grot[4], *gskip[5], *gx0, *gfirst, *partials;
   float *ping, *pong;   // inference only
+  // RL_NET_DETERMINISTIC: partial slabs of the attention / feed-forward backward kernels (two sets, alternating per
+  // block like dqkv / dh), of the patch kernels, and of the head / stem kernels (reduced on the main stream)
+  float *det_attn[2], *det_ffn[2], *det_patch, *det_ends;
+  size_t det_attn_n, det_ffn_n, det_patch_n, det_ends_n;
   size_t floats;
 };
 
-Ws carve(float* base, int B, int L0, int save) {
+// Partial-slab floats of one backward kernel (with its weight-gradient GEMMs) of each kind: upper bounds over the
+// stages, a function of (B, L0) alone; rl_det_take() checks every slab against them.  Slots: one per CTA of the
+// in-CTA gradients (B windows, or ceil(B L / 128) * NSL <= B / 2 + 4 token-tile CTAs at the tcgen05 feed-forward
+// stages), one per token slice of the GEMMs (<= min(RL_DET_MAX_SPLIT, ceil(M / 64)) in every GEMM family).
+struct DetSizes {
+  size_t attn, ffn, patch, ends;
+};
+DetSizes det_sizes(int B, int L0) {
+  const size_t cta = (size_t)B + 4, slack = 4 * RL_DET_MAXRED;
+  auto gemm = [](size_t M) { return std::min<size_t>(RL_DET_MAX_SPLIT, (M + 63) / 64); };
+  DetSizes d = {0, 0, 0, slack + 56 * (size_t)B};
+  for (int s = 0; s < 5; ++s) {
+    const size_t C = 8u << s, L = (size_t)L0 >> s, M = (size_t)B * L;
+    const size_t wslots = (C <= RL_FW_MAXC) ? cta : gemm(M);
+    d.attn = std::max(d.attn, slack + (2 * C + 128) * cta + (4 * C * C + 4 * C) * wslots);   // LN, R-wave table | weights
+    d.ffn = std::max(d.ffn, slack + (2 * C + 12 * C) * cta + (8 * C * C + 5 * C) * wslots);  // LN, lew | weights
+    for (int mode = 0; mode < 2; ++mode) {                                                  // merge 2C / separate C/2
+      const size_t CN = mode == 0 ? 2 * C : C / 2;
+      if (CN < 8 || CN > 128) continue;
+      d.patch = std::max(d.patch, slack + 2 * CN * cta + CN * CN * gemm(M * C / CN));
+    }
+  }
+  return d;
+}
+
+Ws carve(float* base, int B, int L0, int save, int flags) {
   Ws w;
   const size_t N = (size_t)B * 8 * L0;
   size_t off = 0;
@@ -64,6 +94,13 @@ Ws carve(float* base, int B, int L0, int save) {
     w.gx0 = take(N);
     w.gfirst = take(N);
     w.ping = w.pong = nullptr;
+    if (flags & RL_NET_DETERMINISTIC) {
+      const DetSizes d = det_sizes(B, L0);
+      for (int p = 0; p < 2; ++p) { w.det_attn[p] = take(d.attn); w.det_ffn[p] = take(d.ffn); }
+      w.det_patch = take(d.patch);
+      w.det_ends = take(d.ends);
+      w.det_attn_n = d.attn; w.det_ffn_n = d.ffn; w.det_patch_n = d.patch; w.det_ends_n = d.ends;
+    }
   } else {
     w.ping = take(N);
     w.pong = take(N);
@@ -78,8 +115,9 @@ int check_cfg(const rl_net_cfg* cfg, const rl_net_ptrs* P) {
              cfg->L0);
   RL_REQUIRE(!(P->table[0] && cfg->L0 != 256), RL_ERR_SHAPE,
              "net: the R-wave bias tables are defined for 256-sample windows only (model/transformer.py:568-579)");
-  RL_REQUIRE(cfg->ws && cfg->ws_bytes >= ralenet_net_workspace_bytes(cfg->B, cfg->L0, cfg->save), RL_ERR_NULL,
-             "net: workspace missing or too small (%llu bytes given)", (unsigned long long)cfg->ws_bytes);
+  RL_REQUIRE((cfg->flags & ~RL_NET_DETERMINISTIC) == 0, RL_ERR_SHAPE, "net: unknown flags 0x%x", cfg->flags);
+  RL_REQUIRE(cfg->ws && cfg->ws_bytes >= ralenet_net_workspace_bytes_ex(cfg->B, cfg->L0, cfg->save, cfg->flags),
+             RL_ERR_NULL, "net: workspace missing or too small (%llu bytes given)", (unsigned long long)cfg->ws_bytes);
   RL_REQUIRE(cfg->running_mean && cfg->running_var && cfg->bn_stats, RL_ERR_NULL, "net: BN buffers missing");
   for (int s = 0; s < 5; ++s) RL_REQUIRE(cfg->pe[s], RL_ERR_NULL, "net: positional table %d missing", s);
   return RL_OK;
@@ -127,15 +165,19 @@ void fill_stem(rl_stem_args* sa, const rl_net_cfg* cfg, const rl_net_ptrs* P, co
 
 }  // namespace
 
-extern "C" uint64_t ralenet_net_workspace_bytes(int32_t B, int32_t L0, int32_t save) {
+extern "C" uint64_t ralenet_net_workspace_bytes_ex(int32_t B, int32_t L0, int32_t save, int32_t flags) {
   if (B <= 0 || L0 <= 0) return 0;
-  return (uint64_t)carve(nullptr, B, L0, save).floats * sizeof(float);
+  return (uint64_t)carve(nullptr, B, L0, save, flags).floats * sizeof(float);
+}
+
+extern "C" uint64_t ralenet_net_workspace_bytes(int32_t B, int32_t L0, int32_t save) {
+  return ralenet_net_workspace_bytes_ex(B, L0, save, 0);
 }
 
 extern "C" int ralenet_net_fwd_stats(const rl_net_cfg* cfg, const rl_net_ptrs* P, const float* x, void* stream) {
   if (int rc = check_cfg(cfg, P)) return rc;
   RL_REQUIRE(x, RL_ERR_NULL, "net_fwd_stats: x is NULL");
-  const Ws w = carve((float*)cfg->ws, cfg->B, cfg->L0, cfg->save);
+  const Ws w = carve((float*)cfg->ws, cfg->B, cfg->L0, cfg->save, cfg->flags);
   rl_stem_args sa;
   fill_stem(&sa, cfg, P, x, w);
   return ralenet_stem_stats(&sa, stream);
@@ -145,7 +187,7 @@ extern "C" int ralenet_net_fwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
   if (int rc = check_cfg(cfg, P)) return rc;
   RL_REQUIRE(x && out, RL_ERR_NULL, "net_fwd: x/out is NULL");
   const int B = cfg->B, L0 = cfg->L0, save = cfg->save;
-  const Ws w = carve((float*)cfg->ws, B, L0, save);
+  const Ws w = carve((float*)cfg->ws, B, L0, save, cfg->flags);
   int rc;
   {
     rl_stem_args sa;
@@ -223,7 +265,14 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
   RL_REQUIRE(G && x && dout, RL_ERR_NULL, "net_bwd: NULL argument");
   RL_REQUIRE(cfg->save, RL_ERR_SHAPE, "net_bwd: forward was run without save");
   const int B = cfg->B, L0 = cfg->L0;
-  const Ws w = carve((float*)cfg->ws, B, L0, 1);
+  const Ws w = carve((float*)cfg->ws, B, L0, 1, cfg->flags);
+  const bool det = cfg->flags & RL_NET_DETERMINISTIC;
+  RlDet dk;   // deterministic mode: partial slabs of the kernel being enqueued (reduced at the end of its fork)
+  auto det_on = [&](float* slab, size_t cap) -> RlDet* {
+    if (!det) return nullptr;
+    dk = RlDet{slab, cap, 0, {}, 0};
+    return &dk;
+  };
   int rc;
   // input of block i (forward): output of the previous layer piece
   auto block_input = [&](int i) -> const float* {
@@ -238,7 +287,7 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
     rl_head_bwd_args ha = {};
     ha.B = B; ha.L = L0; ha.dout = dout; ha.x = w.ps_out[0]; ha.skip = w.x0; ha.w = P->head[0];
     ha.ds = w.gx0; ha.d_w = G->head[0]; ha.d_b = G->head[1];
-    if ((rc = ralenet_head_bwd(&ha, stream))) return rc;
+    if ((rc = rl_head_bwd(&ha, (cudaStream_t)stream, det_on(w.det_ends, w.det_ends_n)))) return rc;
   }
   const float* g = w.gx0;          // gradient w.r.t. the output of the piece about to be differentiated
   // Main chain: patch / feed-forward / attention data-gradient kernels, numbered n = 0, 1, ...; kernel n writes
@@ -275,6 +324,14 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
     last_side = slot;
     return RL_OK;
   };
+  // the same for a kernel whose parameter gradients went to the partial slabs in *d (deterministic mode): the fork
+  // also carries the reduction of every slab, after the GEMMs
+  auto fork_grads = [&](bool has, RlDet* d, auto launch) -> int {
+    return fork_wgrad(has || (d && d->nred > 0), [&](cudaStream_t q) -> int {
+      if (int r2 = launch(q)) return r2;
+      return d ? rl_launch_grad_reduce(d, q) : RL_OK;
+    });
+  };
   for (int i = RL_NBLOCKS - 1; i >= 0; --i) {
     const int s = kBlocks[i].stage, rwi = kBlocks[i].rw;
     const int C = 8 << s, L = L0 >> s, H = 2 << s;
@@ -293,8 +350,9 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
         before_main();
         pa.dx = rot(); pa.gsum = nullptr;
         pa.d_w = G->ps[j][0]; pa.d_ln_w = G->ps[j][1]; pa.d_ln_b = G->ps[j][2];
-        if ((rc = rl_patch_bwd_main(&pa, st_main))) return rc;
-        if ((rc = fork_wgrad(rl_patch_bwd_has_wgrad(&pa), [&](cudaStream_t q) { return rl_patch_bwd_wgrad(&pa, q); })))
+        RlDet* d = det_on(w.det_patch, w.det_patch_n);
+        if ((rc = rl_patch_bwd_main(&pa, st_main, d))) return rc;
+        if ((rc = fork_grads(rl_patch_bwd_has_wgrad(&pa), d, [&](cudaStream_t q) { return rl_patch_bwd_wgrad(&pa, q, d); })))
           return rc;
         ++n;
         g = pa.dx;
@@ -307,8 +365,9 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
         before_main();
         pa.dx = rot(); pa.gsum = w.gsum;
         pa.d_w = G->pm[layer][0]; pa.d_ln_w = G->pm[layer][1]; pa.d_ln_b = G->pm[layer][2];
-        if ((rc = rl_patch_bwd_main(&pa, st_main))) return rc;
-        if ((rc = fork_wgrad(rl_patch_bwd_has_wgrad(&pa), [&](cudaStream_t q) { return rl_patch_bwd_wgrad(&pa, q); })))
+        RlDet* d = det_on(w.det_patch, w.det_patch_n);
+        if ((rc = rl_patch_bwd_main(&pa, st_main, d))) return rc;
+        if ((rc = fork_grads(rl_patch_bwd_has_wgrad(&pa), d, [&](cudaStream_t q) { return rl_patch_bwd_wgrad(&pa, q, d); })))
           return rc;
         ++n;
         g = pa.dx;
@@ -324,8 +383,9 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
     fa.dx = rot(); fa.dh = w.dh[set]; fa.g2 = w.g2[set]; fa.u = w.uf[set];
     fa.d_ln_w = bg[RL_BLK_LN2W]; fa.d_ln_b = bg[RL_BLK_LN2B]; fa.d_w1 = bg[RL_BLK_W1]; fa.d_b1 = bg[RL_BLK_B1];
     fa.d_w2 = bg[RL_BLK_W2]; fa.d_b2 = bg[RL_BLK_B2]; fa.d_lew = bg[RL_BLK_LEW];
-    if ((rc = rl_ffn_bwd_main(&fa, st_main))) return rc;
-    if ((rc = fork_wgrad(rl_ffn_bwd_has_wgrad(&fa), [&](cudaStream_t q) { return rl_ffn_bwd_wgrad(&fa, q); })))
+    RlDet* dfa = det_on(w.det_ffn[set], w.det_ffn_n);
+    if ((rc = rl_ffn_bwd_main(&fa, st_main, dfa))) return rc;
+    if ((rc = fork_grads(rl_ffn_bwd_has_wgrad(&fa), dfa, [&](cudaStream_t q) { return rl_ffn_bwd_wgrad(&fa, q, dfa); })))
       return rc;
     ++n;
     g = fa.dx;
@@ -352,8 +412,9 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
     aa.d_wq = bg[RL_BLK_WQ]; aa.d_bq = bg[RL_BLK_BQ]; aa.d_wkv = bg[RL_BLK_WKV]; aa.d_bkv = bg[RL_BLK_BKV];
     aa.d_wp = bg[RL_BLK_WP]; aa.d_bp = bg[RL_BLK_BP];
     aa.d_table = has_rw ? G->table[rwi] : nullptr;
-    if ((rc = rl_attn_bwd_main(&aa, st_main))) return rc;
-    if ((rc = fork_wgrad(rl_attn_bwd_has_wgrad(&aa), [&](cudaStream_t q) { return rl_attn_bwd_wgrad(&aa, q); })))
+    RlDet* daa = det_on(w.det_attn[set], w.det_attn_n);
+    if ((rc = rl_attn_bwd_main(&aa, st_main, daa))) return rc;
+    if ((rc = fork_grads(rl_attn_bwd_has_wgrad(&aa), daa, [&](cudaStream_t q) { return rl_attn_bwd_wgrad(&aa, q, daa); })))
       return rc;
     ++n;
     g = dst;
@@ -375,7 +436,7 @@ extern "C" int ralenet_net_bwd_stem(const rl_net_cfg* cfg, const rl_net_ptrs* P,
   if (int rc = check_cfg(cfg, P)) return rc;
   RL_REQUIRE(G && x, RL_ERR_NULL, "net_bwd_stem: NULL argument");
   const int B = cfg->B, L0 = cfg->L0;
-  const Ws w = carve((float*)cfg->ws, B, L0, 1);
+  const Ws w = carve((float*)cfg->ws, B, L0, 1, cfg->flags);
   const float* g = w.gfirst;
   rl_stem_bwd_args sb = {};
   sb.B = B; sb.L = L0; sb.training = cfg->training;
@@ -384,5 +445,6 @@ extern "C" int ralenet_net_bwd_stem(const rl_net_cfg* cfg, const rl_net_ptrs* P,
   sb.sums = cfg->bn_stats + 32; sb.partials = w.partials; sb.dx = dx;
   sb.d_conv_w = G->stem[0]; sb.d_conv_b = G->stem[1]; sb.d_bn_w = G->stem[2]; sb.d_bn_b = G->stem[3];
   sb.eps = 1e-5f;
-  return ralenet_stem_bwd_apply(&sb, stream);
+  RlDet det = {w.det_ends, w.det_ends_n, 0, {}, 0};
+  return rl_stem_bwd_apply(&sb, (cudaStream_t)stream, (cfg->flags & RL_NET_DETERMINISTIC) ? &det : nullptr);
 }

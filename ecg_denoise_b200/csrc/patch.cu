@@ -64,7 +64,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) patch_fwd_kernel(const rl_patc
   });
 }
 
-template <int CN, int WIN>
+template <int CN, int WIN, bool DET>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) patch_bwd_kernel(const rl_patch_bwd_args a, float* __restrict__ gsum) {
   extern __shared__ __align__(16) float smem[];
   constexpr int LDA = ld_mk(CN);
@@ -111,7 +111,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) patch_bwd_kernel(const rl_patc
       [&](int r, int c) { return *reinterpret_cast<const float4*>(su + r * LDA + c); },
       [&](int r, int c, float4 dz, float4) { *reinterpret_cast<float4*>(dxw + src_index(mode, L, C, CN, r, c)) = dz; });
   __syncthreads();
-  ln_backward_finish<CN>(s_part, a.d_ln_w, a.d_ln_b);
+  ln_backward_finish<CN, DET>(s_part, grad_slot<DET>(a.d_ln_w, CN, blockIdx.x), grad_slot<DET>(a.d_ln_b, CN, blockIdx.x));
 }
 
 template <int CN>
@@ -128,18 +128,29 @@ int launch_fwd(const rl_patch_fwd_args* a, cudaStream_t st) {
   return rl_check_launch("patch_fwd_kernel", CN);
 }
 
-template <int CN>
-int launch_bwd(const rl_patch_bwd_args* a, float* gsum, cudaStream_t st) {
+template <int CN, bool DET>
+int launch_bwd_det(const rl_patch_bwd_args* a, float* gsum, cudaStream_t st) {
   const int rows = a->L * a->C / CN;
   const size_t smem = patch_smem<CN>(rows);
   if (a->L * a->C == 2048) {
-    if (int rc = rl_set_smem(patch_bwd_kernel<CN, 1>, smem)) return rc;
-    rl_launch_pdl(patch_bwd_kernel<CN, 1>, dim3(a->B), dim3(RL_NT), smem, st, *a, gsum);
+    if (int rc = rl_set_smem(patch_bwd_kernel<CN, 1, DET>, smem)) return rc;
+    rl_launch_pdl(patch_bwd_kernel<CN, 1, DET>, dim3(a->B), dim3(RL_NT), smem, st, *a, gsum);
   } else {
-    if (int rc = rl_set_smem(patch_bwd_kernel<CN, 2>, smem)) return rc;
-    rl_launch_pdl(patch_bwd_kernel<CN, 2>, dim3(a->B), dim3(RL_NT), smem, st, *a, gsum);
+    if (int rc = rl_set_smem(patch_bwd_kernel<CN, 2, DET>, smem)) return rc;
+    rl_launch_pdl(patch_bwd_kernel<CN, 2, DET>, dim3(a->B), dim3(RL_NT), smem, st, *a, gsum);
   }
   return rl_check_launch("patch_bwd_kernel", CN);
+}
+
+// det: LayerNorm partials one slot per window (CTA)
+template <int CN>
+int launch_bwd(const rl_patch_bwd_args* a, float* gsum, cudaStream_t st, RlDet* det) {
+  if (det == nullptr) return launch_bwd_det<CN, false>(a, gsum, st);
+  rl_patch_bwd_args d = *a;
+  d.d_ln_w = rl_det_take(det, a->d_ln_w, CN, a->B);
+  d.d_ln_b = rl_det_take(det, a->d_ln_b, CN, a->B);
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "patch_bwd: deterministic-mode workspace too small");
+  return launch_bwd_det<CN, true>(&d, gsum, st);
 }
 
 int check_shape(int B, int L, int C, int mode, int* cn) {
@@ -174,7 +185,7 @@ extern "C" int ralenet_patch_fwd(const rl_patch_fwd_args* a, void* stream) {
 
 // gsum: scratch [B, L*C] holding g + g2 when g2 is given (dx is used for it: see below)
 // the data-gradient kernel (also leaves g + g2 in gsum for the weight gradient)
-int rl_patch_bwd_main(const rl_patch_bwd_args* a, cudaStream_t st) {
+int rl_patch_bwd_main(const rl_patch_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(a, RL_ERR_NULL, "patch_bwd: args is NULL");
   int CN = 0;
   if (int rc = check_shape(a->B, a->L, a->C, a->mode, &CN)) return rc;
@@ -184,11 +195,11 @@ int rl_patch_bwd_main(const rl_patch_bwd_args* a, cudaStream_t st) {
   RL_REQUIRE(rl_al16(a->g, a->g2, a->gsum, a->x, a->w, a->ln_w, a->u, a->dx), RL_ERR_SHAPE,
              "patch_bwd: tensors must be 16-byte aligned");
   switch (CN) {
-    case 8: return launch_bwd<8>(a, a->gsum, st);
-    case 16: return launch_bwd<16>(a, a->gsum, st);
-    case 32: return launch_bwd<32>(a, a->gsum, st);
-    case 64: return launch_bwd<64>(a, a->gsum, st);
-    case 128: return launch_bwd<128>(a, a->gsum, st);
+    case 8: return launch_bwd<8>(a, a->gsum, st, det);
+    case 16: return launch_bwd<16>(a, a->gsum, st, det);
+    case 32: return launch_bwd<32>(a, a->gsum, st, det);
+    case 64: return launch_bwd<64>(a, a->gsum, st, det);
+    case 128: return launch_bwd<128>(a, a->gsum, st, det);
   }
   return RL_ERR_SHAPE;
 }
@@ -196,11 +207,11 @@ int rl_patch_bwd_main(const rl_patch_bwd_args* a, cudaStream_t st) {
 bool rl_patch_bwd_has_wgrad(const rl_patch_bwd_args* a) { return a->d_w != nullptr; }
 
 // dW = (g + g2)^T u over all tokens; may run on another stream once the main kernel is done
-int rl_patch_bwd_wgrad(const rl_patch_bwd_args* a, cudaStream_t st) {
+int rl_patch_bwd_wgrad(const rl_patch_bwd_args* a, cudaStream_t st, RlDet* det) {
   const int CN = (a->mode == 0) ? 2 * a->C : a->C / 2;
   const int M = a->B * (a->L * a->C / CN);
   const RlWgradDesc d[1] = {{a->g2 ? a->gsum : a->g, CN, a->u, CN, CN, CN, a->d_w, nullptr}};
-  return rl_launch_wgrad_group(d, 1, M, st);
+  return rl_launch_wgrad_group(d, 1, M, st, det);
 }
 
 extern "C" int ralenet_patch_bwd(const rl_patch_bwd_args* a, void* stream) {

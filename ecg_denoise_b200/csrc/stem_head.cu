@@ -197,6 +197,7 @@ __global__ void __launch_bounds__(RL_NT) stem_bwd_stats_kernel(const rl_stem_bwd
   }
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(RL_NT) stem_bwd_apply_kernel(const rl_stem_bwd_args a) {
   pdl_wait();      // programmatic dependent launch: the previous kernel on the stream has completed
   pdl_trigger();   // let the next kernel get scheduled while this one runs
@@ -263,7 +264,9 @@ __global__ void __launch_bounds__(RL_NT) stem_bwd_apply_kernel(const rl_stem_bwd
       acc += __shfl_xor_sync(0xffffffffu, acc, 1);
       acc += __shfl_xor_sync(0xffffffffu, acc, 2);
       acc += __shfl_xor_sync(0xffffffffu, acc, 4);
-      if (seg == 0 && j < 56) atomicAdd(j < 48 ? a.d_conv_w + j : a.d_conv_b + j - 48, acc);
+      if (seg == 0 && j < 56)        // DET: d_conv_w / d_conv_b are partial slabs [B][48] / [B][8]
+        grad_add<DET>(j < 48 ? grad_slot<DET>(a.d_conv_w, 48, blockIdx.x) + j
+                             : grad_slot<DET>(a.d_conv_b, 8, blockIdx.x) + j - 48, acc);
     }
   }
   if (a.dx) {   // dx[i][t] = sum_{o,k} dc[o][t-k+1] w[o][i][k]
@@ -313,6 +316,7 @@ __global__ void __launch_bounds__(RL_NT) head_fwd_kernel(const rl_head_fwd_args 
   }
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(RL_NT) head_bwd_kernel(const rl_head_bwd_args a) {
   pdl_wait();      // programmatic dependent launch: the previous kernel on the stream has completed
   pdl_trigger();   // let the next kernel get scheduled while this one runs
@@ -368,12 +372,15 @@ __global__ void __launch_bounds__(RL_NT) head_bwd_kernel(const rl_head_bwd_args 
       acc += __shfl_xor_sync(0xffffffffu, acc, 1);
       acc += __shfl_xor_sync(0xffffffffu, acc, 2);
       acc += __shfl_xor_sync(0xffffffffu, acc, 4);
-      if (seg == 0 && j < 50) atomicAdd(j < 48 ? a.d_w + j : a.d_b + j - 48, acc);
+      if (seg == 0 && j < 50)        // DET: d_w / d_b are partial slabs [B][48] / [B][2]
+        grad_add<DET>(j < 48 ? grad_slot<DET>(a.d_w, 48, blockIdx.x) + j : grad_slot<DET>(a.d_b, 2, blockIdx.x) + j - 48,
+                      acc);
     }
   }
 }
 
 // ---------------------------------------------------------------------------------------------
+template <bool DET>
 __global__ void __launch_bounds__(RL_NT) mse_kernel(const rl_mse_args a) {
   pdl_wait();      // programmatic dependent launch: the previous kernel on the stream has completed
   pdl_trigger();   // let the next kernel get scheduled while this one runs
@@ -395,7 +402,8 @@ __global__ void __launch_bounds__(RL_NT) mse_kernel(const rl_mse_args a) {
   sw = block_sum(sw, s_red);
   st = block_sum(st, s_red);
   if (tid == 0) {
-    atomicAdd(a.loss, sw * a.inv_count);
+    if (DET) a.partials[blockIdx.x] = sw * a.inv_count;      // summed in window order by grad_reduce_kernel
+    else atomicAdd(a.loss, sw * a.inv_count);
     if (a.rmse) a.rmse[blockIdx.x] = sqrtf(se / per);
     if (a.snr) a.snr[blockIdx.x] = 10.f * log10f(st / se);
   }
@@ -577,15 +585,28 @@ extern "C" int ralenet_stem_bwd_stats(const rl_stem_bwd_args* a, void* stream) {
   return rl_check_launch("reduce16_kernel");
 }
 
-extern "C" int ralenet_stem_bwd_apply(const rl_stem_bwd_args* a, void* stream) {
+int rl_stem_bwd_apply(const rl_stem_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(a, RL_ERR_NULL, "stem_bwd_apply: args is NULL");
   if (int rc = check_BL("stem_bwd_apply", a->B, a->L)) return rc;
   RL_REQUIRE(a->g && a->x && a->conv_w && a->conv_b && a->bn_w && a->sums, RL_ERR_NULL, "stem_bwd_apply: NULL tensor");
   RL_REQUIRE(a->training ? (a->stats != nullptr) : (a->running_var && a->running_mean), RL_ERR_NULL,
              "stem_bwd_apply: needs stats (training) or running stats (eval)");
   RL_REQUIRE(!a->d_conv_w == !a->d_conv_b, RL_ERR_NULL, "stem_bwd_apply: d_conv_w/d_conv_b both or neither");
-  rl_launch_pdl(stem_bwd_apply_kernel, dim3(a->B), dim3(RL_NT), 0, (cudaStream_t)stream, *a);
-  return rl_check_launch("stem_bwd_apply_kernel");
+  if (det == nullptr) {
+    rl_launch_pdl(stem_bwd_apply_kernel<false>, dim3(a->B), dim3(RL_NT), 0, st, *a);
+    return rl_check_launch("stem_bwd_apply_kernel");
+  }
+  rl_stem_bwd_args d = *a;                     // one partial slot per window (CTA)
+  d.d_conv_w = rl_det_take(det, a->d_conv_w, 48, a->B);
+  d.d_conv_b = rl_det_take(det, a->d_conv_b, 8, a->B);
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "stem_bwd_apply: deterministic-mode workspace too small");
+  rl_launch_pdl(stem_bwd_apply_kernel<true>, dim3(a->B), dim3(RL_NT), 0, st, d);
+  if (int rc = rl_check_launch("stem_bwd_apply_kernel")) return rc;
+  return rl_launch_grad_reduce(det, st);
+}
+
+extern "C" int ralenet_stem_bwd_apply(const rl_stem_bwd_args* a, void* stream) {
+  return rl_stem_bwd_apply(a, (cudaStream_t)stream);
 }
 
 extern "C" int ralenet_head_fwd(const rl_head_fwd_args* a, void* stream) {
@@ -596,21 +617,40 @@ extern "C" int ralenet_head_fwd(const rl_head_fwd_args* a, void* stream) {
   return rl_check_launch("head_fwd_kernel");
 }
 
-extern "C" int ralenet_head_bwd(const rl_head_bwd_args* a, void* stream) {
+int rl_head_bwd(const rl_head_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(a, RL_ERR_NULL, "head_bwd: args is NULL");
   if (int rc = check_BL("head_bwd", a->B, a->L)) return rc;
   RL_REQUIRE(a->dout && a->x && a->w && a->ds, RL_ERR_NULL, "head_bwd: NULL tensor");
   RL_REQUIRE(!a->d_w == !a->d_b, RL_ERR_NULL, "head_bwd: d_w/d_b both or neither");
-  rl_launch_pdl(head_bwd_kernel, dim3(a->B), dim3(RL_NT), 0, (cudaStream_t)stream, *a);
-  return rl_check_launch("head_bwd_kernel");
+  if (det == nullptr) {
+    rl_launch_pdl(head_bwd_kernel<false>, dim3(a->B), dim3(RL_NT), 0, st, *a);
+    return rl_check_launch("head_bwd_kernel");
+  }
+  rl_head_bwd_args d = *a;                     // one partial slot per window (CTA)
+  d.d_w = rl_det_take(det, a->d_w, 48, a->B);
+  d.d_b = rl_det_take(det, a->d_b, 2, a->B);
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "head_bwd: deterministic-mode workspace too small");
+  rl_launch_pdl(head_bwd_kernel<true>, dim3(a->B), dim3(RL_NT), 0, st, d);
+  if (int rc = rl_check_launch("head_bwd_kernel")) return rc;
+  return rl_launch_grad_reduce(det, st);
 }
+
+extern "C" int ralenet_head_bwd(const rl_head_bwd_args* a, void* stream) { return rl_head_bwd(a, (cudaStream_t)stream); }
 
 extern "C" int ralenet_mse(const rl_mse_args* a, void* stream) {
   RL_REQUIRE(a, RL_ERR_NULL, "mse: args is NULL");
   RL_REQUIRE(a->B > 0 && a->per > 0, RL_ERR_SHAPE, "mse: B=%d per=%d", a->B, a->per);
   RL_REQUIRE(a->pred && a->target && a->loss, RL_ERR_NULL, "mse: NULL tensor");
-  rl_launch_pdl(mse_kernel, dim3(a->B), dim3(RL_NT), 0, (cudaStream_t)stream, *a);
-  return rl_check_launch("mse_kernel");
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (a->partials == nullptr) {
+    rl_launch_pdl(mse_kernel<false>, dim3(a->B), dim3(RL_NT), 0, st, *a);
+    return rl_check_launch("mse_kernel");
+  }
+  rl_launch_pdl(mse_kernel<true>, dim3(a->B), dim3(RL_NT), 0, st, *a);
+  if (int rc = rl_check_launch("mse_kernel")) return rc;
+  RlDet det = {a->partials, (size_t)((a->B + 3) & ~3), 0, {}, 0};     // the per-window sums, added in window order
+  rl_det_take(&det, a->loss, 1, a->B);
+  return rl_launch_grad_reduce(&det, st);
 }
 
 // tensor-core implicit-GEMM path for the k = 13 layers of newrale (conv_mma.cu)

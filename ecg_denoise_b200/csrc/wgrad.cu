@@ -9,7 +9,7 @@ namespace {
 
 constexpr int MS = 32;   // tokens staged per inner step
 
-template <int TN, int TK>
+template <int TN, int TK, bool DET>
 __global__ void __launch_bounds__(RL_NT) wgrad_kernel(const float* __restrict__ dY, int ldy,
                                                       const float* __restrict__ X, int ldx, int M, int N, int K,
                                                       float* __restrict__ dW, float* __restrict__ db, int MC) {
@@ -58,42 +58,51 @@ __global__ void __launch_bounds__(RL_NT) wgrad_kernel(const float* __restrict__ 
     }
     __syncthreads();
   }
+  dW = grad_slot<DET>(dW, (size_t)N * K, blockIdx.y);       // DET: slot = token slice
   if (active) {
 #pragma unroll
     for (int i = 0; i < RM; ++i)
 #pragma unroll
       for (int j = 0; j < RN; ++j)
-        atomicAdd(dW + (size_t)(n_base + tm * RM + i) * K + k_base + tn + j * NTN, acc[i][j]);
+        grad_add<DET>(dW + (size_t)(n_base + tm * RM + i) * K + k_base + tn + j * NTN, acc[i][j]);
   }
-  if (do_bias && tid < TN) atomicAdd(db + n_base + tid, bacc);
+  if (do_bias && tid < TN) grad_add<DET>(grad_slot<DET>(db, N, blockIdx.y) + n_base + tid, bacc);
 }
 
 template <int TN, int TK>
 int launch(const float* dY, int ldy, const float* X, int ldx, int M, int N, int K, float* dW, float* db,
-           cudaStream_t st) {
+           cudaStream_t st, RlDet* det) {
   const int tiles = (N / TN) * (K / TK);
   // aim for ~4 CTAs per SM overall, but never slices shorter than 128 tokens
   int splits = (592 + tiles - 1) / tiles;
   const int max_splits = (M + 127) / 128;
   if (splits > max_splits) splits = max_splits;
+  if (det && splits > RL_DET_MAX_SPLIT) splits = RL_DET_MAX_SPLIT;
   if (splits < 1) splits = 1;
   int MC = (M + splits - 1) / splits;
   MC = ((MC + MS - 1) / MS) * MS;
   splits = (M + MC - 1) / MC;
   dim3 grid(tiles, splits);
-  rl_launch_pdl(wgrad_kernel<TN, TK>, dim3(grid), dim3(RL_NT), 0, st, dY, ldy, X, ldx, M, N, K, dW, db, MC);
+  if (det == nullptr) {
+    rl_launch_pdl(wgrad_kernel<TN, TK, false>, dim3(grid), dim3(RL_NT), 0, st, dY, ldy, X, ldx, M, N, K, dW, db, MC);
+    return rl_check_launch("wgrad_kernel", N, K);
+  }
+  dW = rl_det_take(det, dW, (size_t)N * K, splits);     // one partial slot per token slice
+  db = rl_det_take(det, db, N, splits);
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "wgrad: deterministic-mode workspace too small");
+  rl_launch_pdl(wgrad_kernel<TN, TK, true>, dim3(grid), dim3(RL_NT), 0, st, dY, ldy, X, ldx, M, N, K, dW, db, MC);
   return rl_check_launch("wgrad_kernel", N, K);
 }
 
 template <int TN>
 int dispatch_k(int TK, const float* dY, int ldy, const float* X, int ldx, int M, int N, int K, float* dW, float* db,
-               cudaStream_t st) {
+               cudaStream_t st, RlDet* det) {
   switch (TK) {
-    case 4: return launch<TN, 4>(dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 8: return launch<TN, 8>(dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 16: return launch<TN, 16>(dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 32: return launch<TN, 32>(dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 64: return launch<TN, 64>(dY, ldy, X, ldx, M, N, K, dW, db, st);
+    case 4: return launch<TN, 4>(dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 8: return launch<TN, 8>(dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 16: return launch<TN, 16>(dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 32: return launch<TN, 32>(dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 64: return launch<TN, 64>(dY, ldy, X, ldx, M, N, K, dW, db, st, det);
   }
   rl_set_error("wgrad: unsupported K tile %d", TK);
   return RL_ERR_SHAPE;
@@ -125,7 +134,7 @@ struct WgGroup {
 
 constexpr int WG_MS = 64;   // tokens per pipeline stage
 
-template <int T>
+template <int T, bool DET>
 __global__ void __launch_bounds__(RL_NT) wgrad_group_kernel(const WgGroup grp) {
   pdl_wait();      // programmatic dependent launch: the previous kernel on the stream has completed
   pdl_trigger();   // let the next kernel get scheduled while this one runs
@@ -185,26 +194,38 @@ __global__ void __launch_bounds__(RL_NT) wgrad_group_kernel(const WgGroup grp) {
     }
     __syncthreads();
   }
-  float* dW = P.dW;
   const int K = P.K;
-  acc.epilogue([&](int n, int k, float v) { atomicAdd(dW + (size_t)(n_base + n) * K + k_base + k, v); });
-  if (do_bias && tid < T) atomicAdd(P.db + n_base + tid, bacc);
+  float* dW = grad_slot<DET>(P.dW, (size_t)P.N * K, blockIdx.y);     // DET: slot = token slice
+  acc.epilogue([&](int n, int k, float v) { grad_add<DET>(dW + (size_t)(n_base + n) * K + k_base + k, v); });
+  if (do_bias && tid < T) grad_add<DET>(grad_slot<DET>(P.db, P.N, blockIdx.y) + n_base + tid, bacc);
 }
 
 template <int T>
-int launch_group(WgGroup& g, int total_tiles, cudaStream_t st) {
+int launch_group(WgGroup& g, int total_tiles, cudaStream_t st, RlDet* det) {
   int splits = (444 + total_tiles - 1) / total_tiles;            // ~3 CTAs per SM overall
   const int max_splits = (g.M + 2 * WG_MS - 1) / (2 * WG_MS);    // at least 2 pipeline stages per CTA
   if (splits > max_splits) splits = max_splits;
+  if (det && splits > RL_DET_MAX_SPLIT) splits = RL_DET_MAX_SPLIT;
   if (splits < 1) splits = 1;
   int MC = (g.M + splits - 1) / splits;
   MC = ((MC + WG_MS - 1) / WG_MS) * WG_MS;
   splits = (g.M + MC - 1) / MC;
   g.MC = MC;
   const size_t smem = sizeof(float) * 4 * WG_MS * (T + 8);
-  if (int rc = rl_set_smem(wgrad_group_kernel<T>, smem)) return rc;
   dim3 grid(total_tiles, splits);
-  rl_launch_pdl(wgrad_group_kernel<T>, dim3(grid), dim3(RL_NT), smem, st, g);
+  if (det == nullptr) {
+    if (int rc = rl_set_smem(wgrad_group_kernel<T, false>, smem)) return rc;
+    rl_launch_pdl(wgrad_group_kernel<T, false>, dim3(grid), dim3(RL_NT), smem, st, g);
+    return rl_check_launch("wgrad_group_kernel", T, total_tiles);
+  }
+  for (int i = 0; i < g.nprob; ++i) {      // one partial slot per token slice
+    g.p[i].dW = rl_det_take(det, g.p[i].dW, (size_t)g.p[i].N * g.p[i].K, splits);
+    g.p[i].db = rl_det_take(det, g.p[i].db, g.p[i].N, splits);
+  }
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "wgrad: deterministic-mode workspace too small");
+  for (int i = g.nprob; i < 4; ++i) g.p[i] = g.p[0];
+  if (int rc = rl_set_smem(wgrad_group_kernel<T, true>, smem)) return rc;
+  rl_launch_pdl(wgrad_group_kernel<T, true>, dim3(grid), dim3(RL_NT), smem, st, g);
   return rl_check_launch("wgrad_group_kernel", T, total_tiles);
 }
 
@@ -212,17 +233,18 @@ int launch_group(WgGroup& g, int total_tiles, cudaStream_t st) {
 
 // up to 4 problems sharing M; dims must all be multiples of 32 for the tensor-core path, otherwise the
 // problems are launched one by one on the FFMA kernel.
-int rl_launch_wgrad_group_umma(const RlWgradDesc* d, int n, int M, cudaStream_t st);   // wgrad_umma.cu
+int rl_launch_wgrad_group_umma(const RlWgradDesc* d, int n, int M, cudaStream_t st, RlDet* det);   // wgrad_umma.cu
 
-int rl_launch_wgrad_group_reg(const RlWgradDesc* d, int n, int M, cudaStream_t st);    // wgrad_reg.cu
+int rl_launch_wgrad_group_reg(const RlWgradDesc* d, int n, int M, cudaStream_t st, RlDet* det);    // wgrad_reg.cu
 
-int rl_launch_wgrad_group(const RlWgradDesc* d, int n, int M, cudaStream_t st) {
+// det: deterministic mode, the GEMMs write partial slabs [token slice][N][K] recorded in *det
+int rl_launch_wgrad_group(const RlWgradDesc* d, int n, int M, cudaStream_t st, RlDet* det) {
   {
-    const int rc = rl_launch_wgrad_group_reg(d, n, M, st);     // register-tile kernel; 1: group not handled there
+    const int rc = rl_launch_wgrad_group_reg(d, n, M, st, det);     // register-tile kernel; 1: group not handled there
     if (rc <= 0) return rc;
   }
   {
-    const int rc = rl_launch_wgrad_group_umma(d, n, M, st);    // tcgen05 kernels; 1: group not handled there
+    const int rc = rl_launch_wgrad_group_umma(d, n, M, st, det);    // tcgen05 kernels; 1: group not handled there
     if (rc <= 0) return rc;
   }
   int cnt = 0, mind = 1 << 30;
@@ -237,7 +259,7 @@ int rl_launch_wgrad_group(const RlWgradDesc* d, int n, int M, cudaStream_t st) {
   if (cnt == 0) return RL_OK;
   if (!aligned || cnt > 4) {
     for (int i = 0; i < n; ++i)
-      if (int rc = rl_launch_wgrad(d[i].dY, d[i].ldy, d[i].X, d[i].ldx, M, d[i].N, d[i].K, d[i].dW, d[i].db, st))
+      if (int rc = rl_launch_wgrad(d[i].dY, d[i].ldy, d[i].X, d[i].ldx, M, d[i].N, d[i].K, d[i].dW, d[i].db, st, det))
         return rc;
     return RL_OK;
   }
@@ -256,20 +278,20 @@ int rl_launch_wgrad_group(const RlWgradDesc* d, int n, int M, cudaStream_t st) {
     tiles += (d[i].N / T) * (d[i].K / T);
   }
   for (int i = g.nprob; i < 4; ++i) g.p[i] = g.p[0];
-  return T == 64 ? launch_group<64>(g, tiles, st) : launch_group<32>(g, tiles, st);
+  return T == 64 ? launch_group<64>(g, tiles, st, det) : launch_group<32>(g, tiles, st, det);
 }
 
 int rl_launch_wgrad(const float* dY, int ldy, const float* X, int ldx, int M, int N, int K, float* dW, float* db,
-                    cudaStream_t st) {
+                    cudaStream_t st, RlDet* det) {
   if (dW == nullptr) return RL_OK;
   const int TN = pick_tile(N), TK = pick_tile(K);
   RL_REQUIRE(TN && TK && M > 0, RL_ERR_SHAPE, "wgrad: unsupported shape M=%d N=%d K=%d", M, N, K);
   switch (TN) {
-    case 4: return dispatch_k<4>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 8: return dispatch_k<8>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 16: return dispatch_k<16>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 32: return dispatch_k<32>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st);
-    case 64: return dispatch_k<64>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st);
+    case 4: return dispatch_k<4>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 8: return dispatch_k<8>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 16: return dispatch_k<16>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 32: return dispatch_k<32>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st, det);
+    case 64: return dispatch_k<64>(TK, dY, ldy, X, ldx, M, N, K, dW, db, st, det);
   }
   return RL_ERR_SHAPE;
 }

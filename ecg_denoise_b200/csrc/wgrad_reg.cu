@@ -43,6 +43,7 @@ __device__ __forceinline__ void red_add_v4(float* p, float4 v) {
                : "memory");
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(RL_NT, 2) wgrad_reg_kernel(const RgGroup grp) {
   pdl_wait();      // programmatic dependent launch: the previous kernel on the stream has completed
   pdl_trigger();
@@ -154,7 +155,10 @@ __global__ void __launch_bounds__(RL_NT, 2) wgrad_reg_kernel(const RgGroup grp) 
       s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
     }
     const int nn = (tl / P.tiles_k) * WT + row, kk = (tl % P.tiles_k) * WT + c4;
-    red_add_v4(P.dW + (size_t)nn * P.K + kk, s);
+    if constexpr (DET)      // slot = token slice blockIdx.y of the partial slab
+      *reinterpret_cast<float4*>(grad_slot<DET>(P.dW, (size_t)P.N * P.K, blockIdx.y) + (size_t)nn * P.K + kk) = s;
+    else
+      red_add_v4(P.dW + (size_t)nn * P.K + kk, s);
   }
   if (P.db != nullptr)
     for (int it = tid; it < tpc * WT; it += RL_NT) {
@@ -163,7 +167,7 @@ __global__ void __launch_bounds__(RL_NT, 2) wgrad_reg_kernel(const RgGroup grp) 
       if (tl >= P.ntiles || tl % P.tiles_k != 0) continue;
       float s = 0.f;
       for (int ts = 0; ts < nts; ++ts) s += s_bias[ts * tpc + wt][row];
-      atomicAdd(P.db + (tl / P.tiles_k) * WT + row, s);
+      grad_add<DET>(grad_slot<DET>(P.db, P.N, blockIdx.y) + (tl / P.tiles_k) * WT + row, s);
     }
 }
 
@@ -185,7 +189,7 @@ extern "C" int ralenet_set_wgrad_reg(int on) {
 }
 
 // returns 1 when the group is not handled here (caller falls through to wgrad_umma.cu / wgrad.cu)
-int rl_launch_wgrad_group_reg(const RlWgradDesc* d, int n, int M, cudaStream_t st) {
+int rl_launch_wgrad_group_reg(const RlWgradDesc* d, int n, int M, cudaStream_t st, RlDet* det) {
   if (!wgrad_reg_on() || M < 64) return 1;
   RgGroup grp;
   grp.nprob = 0;
@@ -222,10 +226,22 @@ int rl_launch_wgrad_group_reg(const RlWgradDesc* d, int n, int M, cudaStream_t s
   int splits = (2 * 2 * 148 + ctas - 1) / ctas;
   const int max_splits = max(1, M / (64 * nts));
   splits = max(1, min(splits, max_splits));
+  if (det) splits = min(splits, RL_DET_MAX_SPLIT);
   int MC = (M + splits - 1) / splits;
   MC = (MC + 8 * nts - 1) / (8 * nts) * (8 * nts);
   splits = (M + MC - 1) / MC;
   grp.MC = MC;
-  rl_launch_pdl(wgrad_reg_kernel, dim3(ctas, splits), dim3(RL_NT), 0, st, grp);
+  if (det == nullptr) {
+    rl_launch_pdl(wgrad_reg_kernel<false>, dim3(ctas, splits), dim3(RL_NT), 0, st, grp);
+    return rl_check_launch("wgrad_reg_kernel", max_tiles, ctas);
+  }
+  for (int i = 0; i < grp.nprob; ++i) {     // one partial slot per token slice
+    RgProblem& p = grp.p[i];
+    p.dW = rl_det_take(det, p.dW, (size_t)p.N * p.K, splits);
+    p.db = rl_det_take(det, p.db, p.N, splits);
+  }
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "wgrad: deterministic-mode workspace too small");
+  for (int i = grp.nprob; i < 4; ++i) grp.p[i] = grp.p[0];
+  rl_launch_pdl(wgrad_reg_kernel<true>, dim3(ctas, splits), dim3(RL_NT), 0, st, grp);
   return rl_check_launch("wgrad_reg_kernel", max_tiles, ctas);
 }

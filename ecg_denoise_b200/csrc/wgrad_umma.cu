@@ -112,7 +112,7 @@ struct WuSmem {
   static constexpr size_t BYTES = sizeof(float) * (2 * STAGE + TN + TK) + 64;
 };
 
-template <int TK>
+template <int TK, bool DET>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) wgrad_umma_kernel(const WuGroup grp) {
   constexpr int TCOLS = (TK < 32) ? 32 : TK;                  // TMEM columns (power of two >= 32)
   static_assert((RL_NT / 32) % (TN / 32) == 0 && (RL_NT / 32) % (TK / 32) == 0, "one row per thread in TokStage");
@@ -194,8 +194,18 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) wgrad_umma_kernel(const WuGrou
     step(j, sa[0], sb[0]);
     if (j + 1 < nchunk) step(j + 1, sa[1], sb[1]);
   }
-  if (want_ba && sa[0].active()) atomicAdd(&s_ba[sa[0].my_row()], bsum_a);
-  if (want_bb && sb[0].active()) atomicAdd(&s_bb[sb[0].my_row()], bsum_b);
+  if constexpr (DET) {            // the warps holding the same rows add their sums in warp order
+    for (int w = 0; w < RL_NT / 32; ++w) {
+      if (warp == w) {
+        if (want_ba && sa[0].active()) s_ba[sa[0].my_row()] += bsum_a;
+        if (want_bb && sb[0].active()) s_bb[sb[0].my_row()] += bsum_b;
+      }
+      __syncthreads();
+    }
+  } else {
+    if (want_ba && sa[0].active()) atomicAdd(&s_ba[sa[0].my_row()], bsum_a);
+    if (want_bb && sb[0].active()) atomicAdd(&s_bb[sb[0].my_row()], bsum_b);
+  }
   if (nchunk > 0) {
     ring.wait_last();
     umma::tc_fence_after();
@@ -203,7 +213,9 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) wgrad_umma_kernel(const WuGrou
     // are dealt round-robin to the four warp groups w / 4
     const int quad = warp & 3, cgp = warp >> 2;
     const int row = quad * 32 + lane;
-    float* orow = P.out + (size_t)(r_base + row) * P.so_r + (size_t)c_base * P.so_c;
+    // DET: out / bias_a / bias_b are partial slabs [token slice][rows x cols], slot = blockIdx.y
+    float* orow = grad_slot<DET>(P.out, (size_t)P.rows * P.tiles_c * TK, blockIdx.y) + (size_t)(r_base + row) * P.so_r +
+                  (size_t)c_base * P.so_c;
     const int so_c = P.so_c;
 #pragma unroll
     for (int c16 = cgp; c16 < TK / 16; c16 += 4) {
@@ -214,41 +226,60 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) wgrad_umma_kernel(const WuGrou
           // a thread owns 16 consecutive columns of its row: four 16-byte vector reductions (a quarter of the L2
           // transactions of scalar ones, which would touch 32 rows = 32 sectors per warp instruction)
 #pragma unroll
-          for (int i = 0; i < 16; i += 4)
-            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(orow + c16 * 16 + i), "f"(t0[i]),
-                         "f"(t0[i + 1]), "f"(t0[i + 2]), "f"(t0[i + 3])
-                         : "memory");
+          for (int i = 0; i < 16; i += 4) {
+            if constexpr (DET)
+              *reinterpret_cast<float4*>(orow + c16 * 16 + i) = make_float4(t0[i], t0[i + 1], t0[i + 2], t0[i + 3]);
+            else
+              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(orow + c16 * 16 + i), "f"(t0[i]),
+                           "f"(t0[i + 1]), "f"(t0[i + 2]), "f"(t0[i + 3])
+                           : "memory");
+          }
         } else {
           // transposed output: the lanes (rows of the tile) are contiguous in memory, one line per warp instruction
 #pragma unroll
-          for (int i = 0; i < 16; ++i) atomicAdd(orow + (size_t)(c16 * 16 + i) * so_c, t0[i]);
+          for (int i = 0; i < 16; ++i) grad_add<DET>(orow + (size_t)(c16 * 16 + i) * so_c, t0[i]);
         }
       }
     }
   }
   umma::tc_fence_before();
   __syncthreads();
-  if (want_ba && tid < rows_valid) atomicAdd(P.bias_a + r_base + tid, s_ba[tid]);
-  if (want_bb && tid < TK) atomicAdd(P.bias_b + c_base + tid, s_bb[tid]);
+  if (want_ba && tid < rows_valid) grad_add<DET>(grad_slot<DET>(P.bias_a, P.rows, blockIdx.y) + r_base + tid, s_ba[tid]);
+  if (want_bb && tid < TK) grad_add<DET>(grad_slot<DET>(P.bias_b, P.tiles_c * TK, blockIdx.y) + c_base + tid, s_bb[tid]);
   if (warp == 0) umma::tmem_dealloc<TCOLS>(tb);
 }
 
 template <int TK>
-int launch(WuGroup& g, int total_tiles, cudaStream_t st) {
+int launch(WuGroup& g, int total_tiles, cudaStream_t st, RlDet* det) {
   // one wave of CTAs (148 SMs), each with at least four chunks of tokens.  Measured on the training step (B = 256):
   // 112 / 148 / 222 / 296 CTAs -> 2.266 / 2.248 / 2.290 / 2.265 ms, 64 -> 2.355, 32 -> 2.425 (the in-order side stream
   // becomes the critical path); the SM time of these kernels (CTAs x duration) is the same at every split.
   int splits = (148 + total_tiles - 1) / total_tiles;
   const int max_splits = (g.M + 4 * KC - 1) / (4 * KC);
   if (splits > max_splits) splits = max_splits;
+  if (det && splits > RL_DET_MAX_SPLIT) splits = RL_DET_MAX_SPLIT;
   if (splits < 1) splits = 1;
   int MC = (g.M + splits - 1) / splits;
   MC = ((MC + KC - 1) / KC) * KC;
   splits = (g.M + MC - 1) / MC;
   g.MC = MC;
   const size_t smem = WuSmem<TK>::BYTES;
-  if (int rc = rl_set_smem(wgrad_umma_kernel<TK>, smem)) return rc;
-  rl_launch_pdl(wgrad_umma_kernel<TK>, dim3(total_tiles, splits), dim3(RL_NT), smem, st, g);
+  if (det == nullptr) {
+    if (int rc = rl_set_smem(wgrad_umma_kernel<TK, false>, smem)) return rc;
+    rl_launch_pdl(wgrad_umma_kernel<TK, false>, dim3(total_tiles, splits), dim3(RL_NT), smem, st, g);
+    return rl_check_launch("wgrad_umma_kernel", TK, total_tiles);
+  }
+  for (int i = 0; i < g.nprob; ++i) {      // one partial slot per token slice
+    WuProblem& p = g.p[i];
+    const size_t cols = (size_t)p.tiles_c * TK;
+    p.out = rl_det_take(det, p.out, (size_t)p.rows * cols, splits);
+    p.bias_a = rl_det_take(det, p.bias_a, p.rows, splits);
+    p.bias_b = rl_det_take(det, p.bias_b, cols, splits);
+  }
+  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "wgrad: deterministic-mode workspace too small");
+  for (int i = g.nprob; i < 4; ++i) g.p[i] = g.p[0];
+  if (int rc = rl_set_smem(wgrad_umma_kernel<TK, true>, smem)) return rc;
+  rl_launch_pdl(wgrad_umma_kernel<TK, true>, dim3(total_tiles, splits), dim3(RL_NT), smem, st, g);
   return rl_check_launch("wgrad_umma_kernel", TK, total_tiles);
 }
 
@@ -271,7 +302,7 @@ extern "C" int ralenet_set_wgrad_umma(int on) {
 }
 
 // returns 1 if the group is not handled here (caller falls through to wgrad.cu)
-int rl_launch_wgrad_group_umma(const RlWgradDesc* d, int n, int M, cudaStream_t st) {
+int rl_launch_wgrad_group_umma(const RlWgradDesc* d, int n, int M, cudaStream_t st, RlDet* det) {
   if (!wgrad_umma_on() || M < 4 * KC) return 1;
   WuGroup g;
   g.nprob = 0;
@@ -307,9 +338,9 @@ int rl_launch_wgrad_group_umma(const RlWgradDesc* d, int n, int M, cudaStream_t 
   if (g.nprob == 0) return RL_OK;
   for (int i = g.nprob; i < 4; ++i) g.p[i] = g.p[0];
   switch (TK) {
-    case 32: return launch<32>(g, tiles, st);
-    case 64: return launch<64>(g, tiles, st);
-    case 128: return launch<128>(g, tiles, st);
+    case 32: return launch<32>(g, tiles, st, det);
+    case 64: return launch<64>(g, tiles, st, det);
+    case 128: return launch<128>(g, tiles, st, det);
   }
   return 1;
 }

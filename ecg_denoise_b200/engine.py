@@ -228,14 +228,14 @@ class NetPlan:
             p.grad = view
         return fresh
 
-    def cfg(self, B: int, L0: int, training: bool, save: bool, ws: torch.Tensor):
+    def cfg(self, B: int, L0: int, training: bool, save: bool, ws: torch.Tensor, flags: int = 0):
         net = self.net
         bn = net.conv1[2]
         if self.pe_L0 != L0 or self.pe is None or self.pe[0].device != self.flat.device:
             self.pe = [pos_table(L0 >> s, 8 << s, self.flat.device) for s in range(5)]
             self.pe_L0 = L0
         c = STRUCTS["rl_net_cfg"]()
-        c.B, c.L0, c.le_mode, c.training, c.save = B, L0, self.le_mode, int(training), int(save)
+        c.B, c.L0, c.le_mode, c.training, c.save, c.flags = B, L0, self.le_mode, int(training), int(save), flags
         for s in range(5):
             c.pe[s] = self.pe[s].data_ptr()
         c.running_mean, c.running_var = bn.running_mean.data_ptr(), bn.running_var.data_ptr()
@@ -267,8 +267,10 @@ def _capture_stream(batch: int):
     return None
 
 
-def workspace_bytes(B: int, L0: int, save: bool) -> int:
-    return int(_lib.load().ralenet_net_workspace_bytes(B, L0, int(save)))
+def workspace_bytes(B: int, L0: int, save: bool, flags: int = 0) -> int:
+    """bytes of the whole-network workspace; flags = RL_NET_DETERMINISTIC adds the partial slabs of the
+    deterministic backward."""
+    return int(_lib.load().ralenet_net_workspace_bytes_ex(B, L0, int(save), flags))
 
 
 def _call(name, *args):
@@ -310,13 +312,13 @@ def _check_input(x):
     return x
 
 
-def _forward_impl(plan: NetPlan, x, save: bool):
+def _forward_impl(plan: NetPlan, x, save: bool, flags: int = 0):
     B, _, L0 = x.shape
     plan.ensure(x.device)
     plan.refresh_requires_grad()
     training = plan.net.training
-    lease = _lease_ws(plan, workspace_bytes(B, L0, save), x.device)
-    cfg = plan.cfg(B, L0, training, save, lease.buf)
+    lease = _lease_ws(plan, workspace_bytes(B, L0, save, flags), x.device)
+    cfg = plan.cfg(B, L0, training, save, lease.buf, flags)
     out = torch.empty(B, 2, L0, device=x.device, dtype=torch.float32)
     st = ctypes.c_void_p(_stream())
     if training:
@@ -349,10 +351,13 @@ class RalenetFn(torch.autograd.Function):
         x = _check_input(x)
         B, _, L0 = x.shape
         save = bool(ctx.needs_input_grad[0] or ctx.needs_input_grad[1])
-        out, lease, training = _forward_impl(plan, x, save)
+        # torch.use_deterministic_algorithms(True) at forward time selects the deterministic backward; the
+        # workspace is sized for it here and the backward follows this choice
+        flags = _lib.RL_NET_DETERMINISTIC if save and torch.are_deterministic_algorithms_enabled() else 0
+        out, lease, training = _forward_impl(plan, x, save, flags)
         plan.last_ws_bytes = lease.buf.numel()
         if save:
-            ctx.plan, ctx.ws, ctx.shape, ctx.training = plan, lease, (B, L0), training
+            ctx.plan, ctx.ws, ctx.shape, ctx.training, ctx.flags = plan, lease, (B, L0), training, flags
             # BN stats of THIS forward are needed by its backward; keep a private copy
             ctx.bn_stats = plan.bn_stats.clone() if training else None
             ctx.save_for_backward(x)
@@ -364,13 +369,15 @@ class RalenetFn(torch.autograd.Function):
         (x,) = ctx.saved_tensors
         B, L0 = ctx.shape
         dout = _chk(dout, "grad_output")
+        if not ctx.flags:
+            _lib.deterministic_guard("ralenet backward of a forward run without torch.use_deterministic_algorithms(True)")
         plan.ensure(x.device)
         plan.attach_grads()
         if ctx.bn_stats is not None:
             plan.bn_stats[:17].copy_(ctx.bn_stats[:17])
         # the saved activations are only read by the backward kernels (their scratch is a separate part of the
         # workspace), so the node can be differentiated again under retain_graph=True: the lease lives as long as ctx
-        cfg = plan.cfg(B, L0, ctx.training, True, ctx.ws.buf)
+        cfg = plan.cfg(B, L0, ctx.training, True, ctx.ws.buf, ctx.flags)
         st = ctypes.c_void_p(_stream())
         _call("ralenet_net_bwd", ctypes.byref(cfg), ctypes.byref(plan.P), ctypes.byref(plan.G),
               ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(dout.data_ptr()), st)
@@ -455,11 +462,15 @@ class FusedTrainer(_HostPipeline):
     Under torch.distributed the batch is sharded across ranks: BatchNorm statistics are all-reduced
     (SyncBN-equivalent, so the result equals the single-process step on the global batch) and the flat
     gradient buffer is all-reduced once (sum) in front of Adam.
+
+    deterministic: True = bit-reproducible steps on one GPU (gradients, BatchNorm sums, loss, Adam trajectory; the
+    backward writes partial slabs that are reduced in a fixed order, RL_NET_DETERMINISTIC); None = follow
+    torch.are_deterministic_algorithms_enabled() at construction.  Not available with more than one rank.
     """
 
     def __init__(self, net: nn.Module, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8,
                  process_group=None, use_graph: bool = False, graph_collectives: Optional[bool] = None,
-                 loss_weight: Optional[torch.Tensor] = None):
+                 loss_weight: Optional[torch.Tensor] = None, deterministic: Optional[bool] = None):
         from . import ops
         self.ops = ops
         self.net = net
@@ -472,6 +483,17 @@ class FusedTrainer(_HostPipeline):
         self.world = 1
         if process_group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()):
             self.world = torch.distributed.get_world_size(process_group)
+        if self.world > 1:
+            if deterministic:
+                raise _lib.RalenetError("FusedTrainer(deterministic=True) is single-GPU only: the order of the "
+                                        "multi-rank gradient exchange is not fixed")
+            if deterministic is None:
+                _lib.deterministic_guard("FusedTrainer with more than one rank")
+            deterministic = False
+        elif deterministic is None:
+            deterministic = torch.are_deterministic_algorithms_enabled()
+        self.deterministic = bool(deterministic)
+        self.net_flags = _lib.RL_NET_DETERMINISTIC if self.deterministic else 0
         self.use_graph = use_graph
         # capture the NCCL all-reduces inside the step's CUDA graph (default; RALENET_GRAPH_NCCL=0 keeps them outside)
         self.graph_collectives = (os.environ.get("RALENET_GRAPH_NCCL", "1") != "0") if graph_collectives is None \
@@ -532,7 +554,7 @@ class FusedTrainer(_HostPipeline):
         xp = ctypes.c_void_p(x.data_ptr())
 
         def cfg():
-            return plan.cfg(B, L0, True, True, ws)
+            return plan.cfg(B, L0, True, True, ws, self.net_flags)
 
         def st():
             return ctypes.c_void_p(_stream())
@@ -548,7 +570,7 @@ class FusedTrainer(_HostPipeline):
             c = cfg()
             _call("ralenet_net_fwd", ctypes.byref(c), ctypes.byref(plan.P), xp, ctypes.c_void_p(out.data_ptr()), st())
             loss, dout, rmse, snr = ops.mse_loss_metrics(out, target, True, 1.0, out.numel() * self.world,
-                                                         weight=self.loss_weight)
+                                                         weight=self.loss_weight, partials=self._loss_partials)
             _call("ralenet_net_bwd", ctypes.byref(c), ctypes.byref(plan.P), ctypes.byref(plan.G), xp,
                   ctypes.c_void_p(dout.data_ptr()), st())
             self._res = (loss, rmse, snr, out)
@@ -606,7 +628,8 @@ class FusedTrainer(_HostPipeline):
         B, _, L0 = shape
         probe = torch.empty(0, device=device)
         self._setup(probe)
-        self._ws = torch.empty(workspace_bytes(B, L0, True), device=device, dtype=torch.uint8)
+        self._ws = torch.empty(workspace_bytes(B, L0, True, self.net_flags), device=device, dtype=torch.uint8)
+        self._loss_partials = torch.empty(B, device=device, dtype=torch.float32) if self.deterministic else None
         self._out = torch.empty(B, 2, L0, device=device, dtype=torch.float32)
         self._static = (torch.empty(shape, device=device, dtype=torch.float32),
                         torch.empty(shape, device=device, dtype=torch.float32))
@@ -817,6 +840,7 @@ class FineTuneTrainer(_HostPipeline):
         return self._res
 
     def _run(self):
+        _lib.deterministic_guard("FineTuneTrainer (lead-mixing convolution weight gradients)")
         if not self.use_graph:
             return self._step_impl()
         if self.graph is None:

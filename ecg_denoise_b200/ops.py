@@ -96,6 +96,7 @@ class AttnBlockFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        _lib.deterministic_guard("AttnBlockFn backward (parameter gradients accumulated with atomics)")
         x, ln_w, ln_b, wq, bq, wkv, bkv, wp, bp, table, q, k, v, o, lse = ctx.saved_tensors
         H, W, c0, flags = ctx.meta
         B, L, C = x.shape
@@ -143,6 +144,7 @@ class FFNBlockFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        _lib.deterministic_guard("FFNBlockFn backward (parameter gradients accumulated with atomics)")
         x, ln_w, ln_b, w1, b1, w2, b2, lew, h = ctx.saved_tensors
         le_mode, flags = ctx.meta
         B, L, C = x.shape
@@ -187,6 +189,7 @@ class PatchFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        _lib.deterministic_guard("PatchFn backward (parameter gradients accumulated with atomics)")
         x, ln_w, w, u = ctx.saved_tensors
         B, L, C = x.shape
         g = _chk(g, "grad")
@@ -230,6 +233,7 @@ class StemFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        _lib.deterministic_guard("StemFn backward (parameter gradients accumulated with atomics)")
         x, conv_w, conv_b, bn_w, running_mean, running_var, stats = ctx.saved_tensors
         training, eps, reduce_fn = ctx.meta
         B, _, L = x.shape
@@ -266,6 +270,7 @@ class HeadFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dout):
+        _lib.deterministic_guard("HeadFn backward (parameter gradients accumulated with atomics)")
         x, skip, w = ctx.saved_tensors
         B, L, _ = x.shape
         dout = _chk(dout, "grad")
@@ -295,6 +300,7 @@ class Conv1dFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dy):
+        _lib.deterministic_guard("Conv1dFn backward (parameter gradients accumulated with atomics)")
         x, w, b = ctx.saved_tensors
         act, slope = ctx.meta
         B, Ci, L = x.shape
@@ -331,6 +337,7 @@ class EcaFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        _lib.deterministic_guard("EcaFn backward (parameter gradients accumulated with atomics)")
         x, w, s = ctx.saved_tensors
         B, L, C = x.shape
         g = _chk(g, "grad")
@@ -381,6 +388,7 @@ class LinearFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dy):
+        _lib.deterministic_guard("LinearFn backward (parameter gradients accumulated with atomics)")
         x, w = ctx.saved_tensors
         dy = _chk(dy, "grad")
         K, N = x.shape[-1], w.shape[0]
@@ -429,6 +437,7 @@ class PartialConvFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dy):
+        _lib.deterministic_guard("PartialConvFn backward (parameter gradients accumulated with atomics)")
         x, w = ctx.saved_tensors
         dy = _chk(dy, "grad")
         B, C, L = x.shape
@@ -444,11 +453,16 @@ class PartialConvFn(torch.autograd.Function):
 
 
 def mse_loss_metrics(pred: torch.Tensor, target: torch.Tensor, want_grad: bool = True, gscale: float = 1.0,
-                     global_numel: Optional[int] = None, weight: Optional[torch.Tensor] = None):
+                     global_numel: Optional[int] = None, weight: Optional[torch.Tensor] = None,
+                     partials: Optional[torch.Tensor] = None):
     """Fused F.mse_loss (denoise_train.py:53) + its gradient + per-window RMSE / SNR
-    (local_utils/evaluate.py:27-29, 49-51).  Returns (loss[1], dout or None, rmse[B], snr[B])."""
+    (local_utils/evaluate.py:27-29, 49-51).  Returns (loss[1], dout or None, rmse[B], snr[B]).
+    partials: optional float32 [B] scratch; with it the per-window sums are added to the loss in window order
+    (bit-reproducible) instead of with atomics.  Under torch.use_deterministic_algorithms(True) one is allocated."""
     pred, target = _chk(pred, "pred"), _chk(target, "target")
     B = pred.shape[0]
+    if partials is None and torch.are_deterministic_algorithms_enabled():
+        partials = torch.empty(B, device=pred.device, dtype=torch.float32)
     per = pred.numel() // B
     loss = torch.zeros(1, device=pred.device, dtype=torch.float32)
     dout = torch.empty_like(pred) if want_grad else None
@@ -456,7 +470,7 @@ def mse_loss_metrics(pred: torch.Tensor, target: torch.Tensor, want_grad: bool =
     snr = torch.empty(B, device=pred.device, dtype=torch.float32)
     n = pred.numel() if global_numel is None else global_numel
     a = _fill("rl_mse_args", B=B, per=per, pred=pred, target=target, weight=_p(weight), dout=_p(dout), loss=loss,
-              rmse=rmse, snr=snr, inv_count=1.0 / n, gscale=gscale)
+              rmse=rmse, snr=snr, inv_count=1.0 / n, gscale=gscale, partials=_p(partials))
     _lib.call("ralenet_mse", a, _stream())
     return loss, dout, rmse, snr
 

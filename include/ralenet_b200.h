@@ -16,8 +16,10 @@
  *   - the library never allocates, frees or synchronises: every buffer (incl. workspaces) is owned
  *     by the caller; `stream` is a cudaStream_t passed as void*.  Entry points are re-entrant.
  *   - return value: 0 = ok, <0 = RL_ERR_* ; ralenet_last_error() gives a thread-local message.
- *   - gradients of parameters are ACCUMULATED (+=, atomically) into the given buffers, which the
- *     caller zero-fills when it wants plain gradients.  Data gradients are overwritten.
+ *   - gradients of parameters are ACCUMULATED (+=) into the given buffers, which the caller zero-fills when it
+ *     wants plain gradients.  Data gradients are overwritten.  By default the per-CTA partial sums are added with
+ *     fp32 atomics, so their low bits depend on scheduling; the whole-network backward with RL_NET_DETERMINISTIC
+ *     (rl_net_cfg.flags) stores them into partial slabs and adds them in a fixed order instead (bit-reproducible).
  *   - head_dim is 4 everywhere (C / H == 4), softmax scale = 4^-0.5 (model/transformer.py:277-278).
  */
 #ifndef RALENET_B200_H
@@ -29,7 +31,7 @@
 extern "C" {
 #endif
 
-#define RL_ABI_VERSION 3
+#define RL_ABI_VERSION 4
 
 enum {
   RL_OK = 0,
@@ -264,6 +266,8 @@ typedef struct {
   float* loss;                 /* [1] (+=)                                                      */
   float* rmse; float* snr;     /* [B] each or NULL                                              */
   float inv_count, gscale;
+  float* partials;             /* [B] scratch or NULL: per-window loss sums are stored here and   */
+                               /* added to loss[0] in window order (deterministic); NULL: atomics */
 } rl_mse_args;
 int ralenet_mse(const rl_mse_args* a, void* stream);
 
@@ -327,14 +331,23 @@ typedef struct {
   int32_t le_mode;             /* RL_LE_*                                                        */
   int32_t training;            /* BatchNorm batch statistics + running-stat update               */
   int32_t save;                /* keep activations for ralenet_net_bwd                           */
-  int32_t _pad;
+  int32_t flags;               /* RL_NET_* (0: default)                                          */
   const float* pe[5];          /* P[:L_s] per stage, [L_s, C_s]                                  */
   float* running_mean; float* running_var; int64_t* num_batches_tracked;
   float* bn_stats;             /* [64]: [0:17] forward stats, [32:48] backward sums              */
-  void* ws; uint64_t ws_bytes; /* workspace of >= ralenet_net_workspace_bytes(B, L0, save)       */
+  void* ws; uint64_t ws_bytes; /* workspace of >= ralenet_net_workspace_bytes_ex(B, L0, save, flags) */
 } rl_net_cfg;
 
-uint64_t ralenet_net_workspace_bytes(int32_t B, int32_t L0, int32_t save);
+/* RL_NET_DETERMINISTIC: the backward pass (ralenet_net_bwd / ralenet_net_bwd_stem) gives bit-identical parameter
+ * gradients, BatchNorm sums and dx from run to run for a fixed build, batch shape and kernel-selection switches,
+ * whatever the scheduling of CTAs and streams: every cross-CTA accumulation into a parameter gradient is a plain store
+ * into its own slot of a partial slab in the workspace, and a reduction kernel adds the slots in slot order with one
+ * read-modify-write per gradient element.  The forward pass is deterministic in either mode. */
+enum { RL_NET_DETERMINISTIC = 1 };
+
+uint64_t ralenet_net_workspace_bytes(int32_t B, int32_t L0, int32_t save);      /* == _ex(B, L0, save, 0) */
+/* the deterministic mode needs the partial slabs on top (a function of B and L0 only) */
+uint64_t ralenet_net_workspace_bytes_ex(int32_t B, int32_t L0, int32_t save, int32_t flags);
 /* forward: phase 1 (training only) computes BN partial stats into cfg->bn_stats[0:17];
  * the host may all-reduce them; phase 2 runs the rest.  Eval mode: call phase 2 only. */
 int ralenet_net_fwd_stats(const rl_net_cfg* cfg, const rl_net_ptrs* P, const float* x, void* stream);
