@@ -34,8 +34,6 @@ namespace cg = cooperative_groups;
 
 RL_TRACE_DEFINE(attn_umma)
 
-int rl_umma_tma_on();            // ffn_umma.cu: ralenet_set_umma_tma / RALENET_UMMA_TMA
-
 namespace {
 
 constexpr int TM = 128;          // tokens per tile (UMMA M)
@@ -58,66 +56,16 @@ struct ASmem {
   static constexpr size_t BYTES = sizeof(float) * (R0 + R1 + 128 + CONSTS) + 64;
 };
 
-// Staging of one K chunk of the [q | k | v] weight rows of head slice r into a K-major tile pair:
-//   tile row n <- Wq[32 r + n] (n < 32), Wk[32 r + n - 32] (n < 64), Wv[32 r + n - 64]   (Wk, Wv = halves of to_kv)
-// 24 warp-wide groups of 8 rows x 4 sixteen-byte chunks, as umma::KStage.
-struct QkvStage {
-  static constexpr int NCH = KC / 4, ITEMS = (NQ / 8) * (NCH / 4), NWARP = RL_NT / 32;
-  static constexpr int PER = (ITEMS + NWARP - 1) / NWARP;
-  float4 v[PER];
-
-  __device__ __forceinline__ void load(const float* __restrict__ wq, const float* __restrict__ wkv, int r, int C,
-                                       int k0) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int rsub = lane & 7, qsub = lane >> 3;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) {
-      const int grp = wid + i * NWARP;
-      v[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (grp < ITEMS) {
-        const int rgrp = grp % (NQ / 8), qgrp = grp / (NQ / 8);
-        const int n = rgrp * 8 + rsub, q = qgrp * 4 + qsub;
-        const int seg = n / CS, nn = n % CS;
-        const float* row = (seg == 0) ? wq + (size_t)(CS * r + nn) * C : wkv + (size_t)((seg - 1) * C + CS * r + nn) * C;
-        v[i] = __ldg(reinterpret_cast<const float4*>(row + k0) + q);
-      }
-    }
-  }
-  __device__ __forceinline__ void store(float* hi, float* lo) const {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int rsub = lane & 7, qsub = lane >> 3;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) {
-      const int grp = wid + i * NWARP;
-      if (grp < ITEMS) {
-        const int rgrp = grp % (NQ / 8), qgrp = grp / (NQ / 8);
-        const int o = rsub * 4 + (qgrp * 4 + qsub) * 32 + rgrp * (NCH * 32);
-        *reinterpret_cast<float4*>(hi + o) = v[i];
-        *reinterpret_cast<float4*>(lo + o) =
-            umma::lo4(v[i]);
-      }
-    }
-  }
-};
-
-// TMA = true: the weight operands arrive through cp.async.bulk.tensor (tma.cuh): per 32-wide K chunk three 32-row boxes
-// (the q, k and v rows of this CTA's head slice, from to_q and the two halves of to_kv) into one 96-row SWIZZLE_128B
-// tile, and one C-row box for the K-slice of the output projection.  TMA = false: the round-1 register staging (A/B).
-template <int C, bool TMA>
+// The weight operands arrive through cp.async.bulk.tensor (tma.cuh): per 32-wide K chunk three 32-row boxes (the q, k
+// and v rows of this CTA's head slice, from to_q and the two halves of to_kv) into one 96-row SWIZZLE_128B tile, and one
+// C-row box for the K-slice of the output projection.
+template <int C>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_attn_fwd_args a,
                                                                        const __grid_constant__ CUtensorMap tmq,
                                                                        const __grid_constant__ CUtensorMap tmkv,
                                                                        const __grid_constant__ CUtensorMap tmp) {
   constexpr int L = 2048 / C, H = C / RL_HD, NSL = C / CS, NWT = TM / L, HS = CS / RL_HD, QT = L / 16;
   constexpr int NCHK = C / KC;
-  // the weights are not written by the preceding kernels of the step: pull the whole q|k|v slice of this CTA into
-  // registers before waiting on the programmatic dependency, so its L2 latency hides behind the previous kernel
-  QkvStage wr[TMA ? 1 : NCHK];
-  if constexpr (!TMA) {
-    const int rp = (int)(blockIdx.x % NSL);
-#pragma unroll
-    for (int j = 0; j < NCHK; ++j) wr[j].load(a.wq, a.wkv, rp, C, j * KC);
-  }
   extern __shared__ __align__(1024) float smem[];
   float* r0 = smem;
   float* r1 = smem + ASmem<C>::R0;
@@ -142,14 +90,12 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
     umma::mbar_init(bars + 3, 1);
     umma::mbar_init(bars + 4, 1);
     umma::fence_mbar_init();
-    if constexpr (TMA) {
-      umma::fence_async_smem();
-      tma::prefetch_desc(&tmq);
-      tma::prefetch_desc(&tmkv);
-      tma::prefetch_desc(&tmp);
-      tma_issue_qkv(0);                  // weights are immutable inside the step: the ring fills while the previous
-      tma_issue_qkv(1);                  // kernel drains (NCHK >= 2)
-    }
+    umma::fence_async_smem();
+    tma::prefetch_desc(&tmq);
+    tma::prefetch_desc(&tmkv);
+    tma::prefetch_desc(&tmp);
+    tma_issue_qkv(0);                    // weights are immutable inside the step: the ring fills while the previous
+    tma_issue_qkv(1);                    // kernel drains (NCHK >= 2)
   }
   // ... and so do the constants of phase 1 (positional tile, LayerNorm affine) and the R-wave table: staged in
   // shared memory here, phase 1 then waits for ONE round of global loads (x) instead of three
@@ -265,36 +211,26 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
     for (int j = 0; j < NCHK; ++j) {
       float* bh = sB + ring.buf() * 2 * NQ * KC;
       float* bl = bh + NQ * KC;
-      if constexpr (TMA) {
-        umma::mbar_wait(bars + 2 + (j & 1), (uint32_t)((j >> 1) & 1));
-        tma::derive_lo<RL_NT>(bh, bl, NQ * KC);
-      } else {
-        ring.wait_free();
-        wr[j].store(bh, bl);
-      }
+      umma::mbar_wait(bars + 2 + (j & 1), (uint32_t)((j >> 1) & 1));
+      tma::derive_lo<RL_NT>(bh, bl, NQ * KC);
       umma::fence_async_smem();
       __syncthreads();
       if (tid == 0) {
         umma::tc_fence_after();
-        if constexpr (TMA) tma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
-        else umma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
+        tma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
         umma::commit(bars + ring.buf());
-        if constexpr (TMA) {
-          if (j + 2 < NCHK) {            // refill this buffer once its MMAs have drained
-            ++ring.chunk;
-            ring.wait_last();
-            --ring.chunk;
-            tma_issue_qkv(j + 2);
-          }
+        if (j + 2 < NCHK) {              // refill this buffer once its MMAs have drained
+          ++ring.chunk;
+          ring.wait_last();
+          --ring.chunk;
+          tma_issue_qkv(j + 2);
         }
       }
       ++ring.chunk;
     }
   }
-  // the Wp slice of this CTA goes to registers now; its latency hides behind the epilogue and the attention core
-  umma::KStage<C, CS, RL_NT> wpr;
-  if constexpr (!TMA) wpr.load(a.wp + CS * r, C, C);
-  // ... and so do the bias values of epilogue 1 (warp group w / 4 = 0, 1, 2 takes q, k, v)
+  // the bias values of epilogue 1 go to registers now; their latency hides behind the MMAs (warp group w / 4 = 0, 1, 2
+  // takes q, k, v)
   float4 bias4[CS / 4];
   {
     const int seg = warp >> 2;
@@ -311,13 +247,11 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
   ring.wait_last();
   umma::tc_fence_after();
   RL_TS(attn_umma, 5);
-  if constexpr (TMA) {
-    // the ring is dead (its last MMAs have completed): the K-slice Wp[:, 32 r : 32 r + 32] lands over it while
-    // epilogue 1 and the attention core run
-    if (tid == 0) {
-      tma::expect_tx(bars + 4, C * CS * 4);
-      tma::load_2d(sW_hi, &tmp, CS * r, 0, bars + 4);
-    }
+  // the ring is dead (its last MMAs have completed): the K-slice Wp[:, 32 r : 32 r + 32] lands over it while
+  // epilogue 1 and the attention core run
+  if (tid == 0) {
+    tma::expect_tx(bars + 4, C * CS * 4);
+    tma::load_2d(sW_hi, &tmp, CS * r, 0, bars + 4);
   }
 
   // 3a. epilogue 1: + bias, q / k / v slices -> shared memory [TM][LDS] (over the dead u tile) and, for the
@@ -393,19 +327,14 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
       *reinterpret_cast<float4*>(sO_hi + o) = o4;
       *reinterpret_cast<float4*>(sO_lo + o) = umma::lo4(o4);
     }
-    if constexpr (TMA) {
-      umma::mbar_wait(bars + 4, 0u);
-      tma::derive_lo<RL_NT>(sW_hi, sW_lo, C * CS);
-    } else {
-      wpr.store(sW_hi, sW_lo);
-    }
+    umma::mbar_wait(bars + 4, 0u);
+    tma::derive_lo<RL_NT>(sW_hi, sW_lo, C * CS);
     umma::fence_async_smem();
     __syncthreads();
     if (tid == 0) {
       constexpr uint32_t idesc = umma::idesc_tf32(TM, C);
       umma::tc_fence_after();
-      if constexpr (TMA) tma::mma_chunk_3x<CS>(tb + NQ, sO_hi, sO_lo, CS, 0, sW_hi, sW_lo, idesc, 0u);
-      else umma::mma_chunk_3x<CS>(tb + NQ, sO_hi, sO_lo, CS, 0, sW_hi, sW_lo, idesc, 0u);
+      tma::mma_chunk_3x<CS>(tb + NQ, sO_hi, sO_lo, CS, 0, sW_hi, sW_lo, idesc, 0u);
       umma::commit(bars + ring.buf());
     }
     ++ring.chunk;
@@ -475,17 +404,15 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
   RL_TS(attn_umma, 12);
 }
 
-template <int C, bool TMA>
+template <int C>
 int launch(const rl_attn_fwd_args& a, cudaStream_t st) {
   constexpr int NSL = C / CS;
   const int tiles = (a.B * a.L + TM - 1) / TM;
   CUtensorMap tmq = {}, tmkv = {}, tmp = {};
-  if (TMA) {
-    if (int rc = rl_tmap_weight(a.wq, C, C, C, CS, &tmq)) return rc;          // to_q  [C][C]:  32-row boxes
-    if (int rc = rl_tmap_weight(a.wkv, 2 * C, C, C, CS, &tmkv)) return rc;    // to_kv [2C][C]: 32-row boxes
-    if (int rc = rl_tmap_weight(a.wp, C, C, C, C, &tmp)) return rc;           // proj  [C][C]:  all C rows, 32 columns
-  }
-  auto kernel = attn_fwd_umma_kernel<C, TMA>;
+  if (int rc = rl_tmap_weight(a.wq, C, C, C, CS, &tmq)) return rc;            // to_q  [C][C]:  32-row boxes
+  if (int rc = rl_tmap_weight(a.wkv, 2 * C, C, C, CS, &tmkv)) return rc;      // to_kv [2C][C]: 32-row boxes
+  if (int rc = rl_tmap_weight(a.wp, C, C, C, C, &tmp)) return rc;             // proj  [C][C]:  all C rows, 32 columns
+  auto kernel = attn_fwd_umma_kernel<C>;
   if (int rc = rl_set_smem(kernel, ASmem<C>::BYTES)) return rc;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(tiles * NSL);
@@ -543,8 +470,6 @@ int rl_attn_fwd_umma(const rl_attn_fwd_args* a, cudaStream_t st) {
     const int ctas = (a->B * a->L + TM - 1) / TM * (a->C / CS);
     if (ctas > n_sm) return 1;
   }
-  const bool tma_ok = rl_umma_tma_on() && ((uintptr_t)a->wq % 16 == 0) && ((uintptr_t)a->wkv % 16 == 0) &&
-                      ((uintptr_t)a->wp % 16 == 0);
-  if (a->C == 128) return tma_ok ? launch<128, true>(*a, st) : launch<128, false>(*a, st);
-  return tma_ok ? launch<64, true>(*a, st) : launch<64, false>(*a, st);
+  if (a->C == 128) return launch<128>(*a, st);
+  return launch<64>(*a, st);
 }

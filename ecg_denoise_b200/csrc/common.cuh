@@ -227,35 +227,6 @@ __device__ __forceinline__ void micro_gemm(float (&acc)[RM][RN], const float* __
   }
 }
 
-// stage W^T chunk: dst[k*ldd + n] = W[(n0+n)*ldw + k0 + k]   for n < NC, k < KC   (coalesced along k)
-__device__ __forceinline__ void stage_wT(float* dst, int ldd, const float* __restrict__ W, int ldw, int n0, int NC,
-                                         int k0, int KC) {
-  for (int i = threadIdx.x; i < NC * KC; i += RL_NT) {
-    const int k = i % KC, n = i / KC;
-    dst[k * ldd + n] = __ldg(W + (size_t)(n0 + n) * ldw + k0 + k);
-  }
-}
-// stage W chunk as is: dst[r*ldd + c] = W[(r0+r)*ldw + c0 + c]   for r < R, c < Cc   (coalesced along c)
-__device__ __forceinline__ void stage_w(float* dst, int ldd, const float* __restrict__ W, int ldw, int r0, int R,
-                                        int c0, int Cc) {
-  for (int i = threadIdx.x; i < R * Cc; i += RL_NT) {
-    const int c = i % Cc, r = i / Cc;
-    dst[r * ldd + c] = __ldg(W + (size_t)(r0 + r) * ldw + c0 + c);
-  }
-}
-
-// copy a contiguous [n] float block global <-> shared with float4 (n % 4 == 0, 16B aligned)
-__device__ __forceinline__ void copy_g2s(float* dst, const float* __restrict__ src, int n) {
-  const float4* s4 = reinterpret_cast<const float4*>(src);
-  float4* d4 = reinterpret_cast<float4*>(dst);
-  for (int i = threadIdx.x; i < n / 4; i += RL_NT) d4[i] = __ldg(s4 + i);
-}
-__device__ __forceinline__ void copy_s2g(float* __restrict__ dst, const float* src, int n) {
-  const float4* s4 = reinterpret_cast<const float4*>(src);
-  float4* d4 = reinterpret_cast<float4*>(dst);
-  for (int i = threadIdx.x; i < n / 4; i += RL_NT) d4[i] = s4[i];
-}
-
 // ---------------------------------------------------------------------------------------------
 // Parameter-gradient output of a backward kernel.  Default: fp32 atomics into the gradient, so the low bits depend on
 // the order in which CTAs arrive.  Deterministic mode (DET, RL_NET_DETERMINISTIC): the gradient pointer handed to the
@@ -418,51 +389,6 @@ __device__ __forceinline__ void ln_backward_finish(const float* s_part, float* _
     grad_add<DET>((i < C) ? d_ln_w + i : d_ln_b + i - C, s);
   }
 }
-
-// ---------------------------------------------------------------------------------------------
-constexpr int SW_FLOATS = 4608;   // weight staging area (18 KB)
-
-// CTA-wide GEMM accumulator: out[M x N] spread over RL_NT threads, RM x RN micro tile per thread at
-// rows m0+i, cols n0 + j*nst.  Requires (M/RM)*(N/RN) <= RL_NT.
-template <int RM, int RN>
-struct TileAcc {
-  float acc[RM][RN];
-  int m0, n0, nst;
-  bool active;
-  __device__ __forceinline__ void init(int M, int N) {
-    const int ntn = N / RN;
-    const int t = threadIdx.x;
-    active = t < (M / RM) * ntn;
-    m0 = (t / ntn) * RM;
-    n0 = t % ntn;
-    nst = ntn;
-#pragma unroll
-    for (int i = 0; i < RM; ++i)
-#pragma unroll
-      for (int j = 0; j < RN; ++j) acc[i][j] = 0.f;
-  }
-  __device__ __forceinline__ void mac(const float* A, int sam, int sak, const float* B, int sbk, int K) {
-    if (active) micro_gemm<RM, RN>(acc, A, sam, sak, B, sbk, m0, n0, nst, K);
-  }
-  template <class F>
-  __device__ __forceinline__ void epilogue(F f) {
-    if (active) {
-#pragma unroll
-      for (int i = 0; i < RM; ++i)
-#pragma unroll
-        for (int j = 0; j < RN; ++j) f(m0 + i, n0 + j * nst, acc[i][j]);
-    }
-  }
-};
-
-__device__ __forceinline__ int pow2_floor(int v) {
-  int p = 1;
-  while (p * 2 <= v) p *= 2;
-  return p;
-}
-
-template <int C>
-__host__ __device__ constexpr int lda_of() { return C + 1; }   // odd row stride: conflict-free A operand
 
 // ---------------------------------------------------------------------------------------------
 // Tensor-core CTA GEMM on shared-memory operands: legacy mma.sync m16n8k8 TF32 with the 3xTF32 split
@@ -703,16 +629,6 @@ __device__ __forceinline__ void copy_rows_s2g(float* __restrict__ dst, const flo
     reinterpret_cast<float4*>(dst + r * cols)[c4] = *reinterpret_cast<const float4*>(src + r * lds + 4 * c4);
   }
 }
-// stage a weight block: dst[r*ldd + c] = W[(r0+r)*ldw + c0 + c], r < R, c < Cc (Cc, c0, ldw, ldd % 4 == 0), float4
-__device__ __forceinline__ void stage_w4(float* dst, int ldd, const float* __restrict__ W, int ldw, int r0, int R,
-                                         int c0, int Cc) {
-  const int c4n = Cc >> 2;
-  for (int i = threadIdx.x; i < R * c4n; i += RL_NT) {
-    const int r = i / c4n, c4 = i % c4n;
-    *reinterpret_cast<float4*>(dst + r * ldd + 4 * c4) =
-        __ldg(reinterpret_cast<const float4*>(W + (size_t)(r0 + r) * ldw + c0) + c4);
-  }
-}
 
 // ---------------------------------------------------------------------------------------------
 // Weight streaming for the fused block kernels: the weight matrix stays in global memory (L2-resident, 4.3 MB
@@ -809,47 +725,7 @@ struct WStream {
 // ---------------------------------------------------------------------------------------------
 // In-CTA weight gradient for the narrow stages (C <= 16), where a separate GEMM launch costs more than the math:
 //   dW[n*K + k] += sum_{t<L} A[t*lda + n] * B[t*ldb + k]      db[n] += sum_t A[t*lda + n]
-// one partial per CTA (window), finished with fp32 red.global.  All RL_NT threads must call.
-template <int N, int K, int L>
-__device__ __forceinline__ void cta_wgrad(const float* A, int lda, const float* B, int ldb, float* __restrict__ dW,
-                                          float* __restrict__ db) {
-  constexpr int OUT = N * K;
-  const int tid = threadIdx.x;
-  if (dW != nullptr) {
-    if (OUT >= RL_NT) {
-      static_assert(OUT < RL_NT || OUT % RL_NT == 0, "cta_wgrad: outputs must tile the CTA");
-      constexpr int R = (OUT >= RL_NT) ? OUT / RL_NT : 1;
-      float acc[R];
-#pragma unroll
-      for (int r = 0; r < R; ++r) acc[r] = 0.f;
-#pragma unroll 4
-      for (int t = 0; t < L; ++t) {
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-          const int o = tid + r * RL_NT;
-          acc[r] = fmaf(A[t * lda + o / K], B[t * ldb + o % K], acc[r]);
-        }
-      }
-#pragma unroll
-      for (int r = 0; r < R; ++r) atomicAdd(dW + tid + r * RL_NT, acc[r]);
-    } else {
-      constexpr int G = (OUT < RL_NT) ? RL_NT / OUT : 1;          // token groups
-      const int o = tid % OUT, grp = tid / OUT;
-      float acc = 0.f;
-      if (grp < G)
-        for (int t = grp; t < L; t += G) acc = fmaf(A[t * lda + o / K], B[t * ldb + o % K], acc);
-      if (grp < G) atomicAdd(dW + o, acc);
-    }
-  }
-  if (db != nullptr && tid < N) {
-    float s = 0.f;
-#pragma unroll 4
-    for (int t = 0; t < L; ++t) s += A[t * lda + tid];
-    atomicAdd(db + tid, s);
-  }
-}
-
-// Tensor-core form of the same in-CTA weight gradient, in two phases around ONE CTA barrier:
+// on the tensor cores, in two phases around ONE CTA barrier:
 //   partial(): every warp owns one (m16n8 tile of dW, token range) item -- rows = output features (padded to 16),
 //     columns = input features, the L tokens split KS ways so that all 16 warps work (round 2 gave each tile to one warp
 //     for all L tokens: at C = 16 two warps ran the MMAs while fourteen sat at the next barrier, 15 % of the samples of

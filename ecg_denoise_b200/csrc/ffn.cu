@@ -11,11 +11,9 @@
 #define RL_MINB 2
 #include "common.cuh"
 
-// cluster kernels for the wide stages (ffn_cluster.cu); return 1 when the shape/mode is not handled there
-int rl_ffn_fwd_umma(const rl_ffn_fwd_args* a, cudaStream_t st);      // tcgen05 kernels (ffn_umma.cu)
+// tcgen05 kernels for the wide stages (ffn_umma.cu); return 1 when the shape/mode is not handled there
+int rl_ffn_fwd_umma(const rl_ffn_fwd_args* a, cudaStream_t st);
 int rl_ffn_bwd_umma(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det);
-int rl_ffn_fwd_cluster(const rl_ffn_fwd_args* a, cudaStream_t st);
-int rl_ffn_bwd_cluster(const rl_ffn_bwd_args* a, cudaStream_t st);
 
 #include "ffn_body.cuh"
 
@@ -341,12 +339,8 @@ extern "C" int ralenet_ffn_fwd(const rl_ffn_fwd_args* a, void* stream) {
   RL_REQUIRE(rl_al16(a->x, a->y, a->w1, a->w2, a->ln_w, a->ln_b, a->h, a->extra), RL_ERR_SHAPE,
              "ffn_fwd: tensors must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
-  {
-    int rc = rl_ffn_fwd_umma(a, st);
-    if (rc <= 0) return rc;
-    rc = rl_ffn_fwd_cluster(a, st);
-    if (rc <= 0) return rc;
-  }
+  const int rc = rl_ffn_fwd_umma(a, st);
+  if (rc != 1) return rc;
   switch (a->C) {
     case 8: return launch_fwd<8>(a, st);
     case 16: return launch_fwd<16>(a, st);
@@ -367,18 +361,16 @@ int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(!a->d_ln_w == !a->d_ln_b, RL_ERR_NULL, "ffn_bwd: d_ln_w/d_ln_b must be both set or both NULL");
   RL_REQUIRE(rl_al16(a->g, a->x, a->w1, a->w2, a->ln_w, a->ln_b, a->h, a->dx, a->dh, a->g2, a->u), RL_ERR_SHAPE,
              "ffn_bwd: tensors must be 16-byte aligned");
-  int rc = rl_ffn_bwd_umma(a, st, det);
-  if (rc < 0) return rc;
-  if (rc == 1 && det == nullptr) rc = rl_ffn_bwd_cluster(a, st);   // (never reached: the tcgen05 kernels take its shapes)
-  if (rc < 0) return rc;
-  if (rc == 1) switch (a->C) {
-    case 8: rc = launch_bwd<8>(a, st, det); break;
-    case 16: rc = launch_bwd<16>(a, st, det); break;
-    case 32: rc = launch_bwd<32>(a, st, det); break;
-    case 64: rc = launch_bwd<64>(a, st, det); break;
-    case 128: rc = launch_bwd<128>(a, st, det); break;
+  const int rc = rl_ffn_bwd_umma(a, st, det);
+  if (rc != 1) return rc;
+  switch (a->C) {
+    case 8: return launch_bwd<8>(a, st, det);
+    case 16: return launch_bwd<16>(a, st, det);
+    case 32: return launch_bwd<32>(a, st, det);
+    case 64: return launch_bwd<64>(a, st, det);
+    case 128: return launch_bwd<128>(a, st, det);
   }
-  return rc;
+  return RL_ERR_SHAPE;
 }
 
 bool rl_ffn_bwd_has_wgrad(const rl_ffn_bwd_args* a) { return a->C > RL_FW_MAXC && (a->d_w1 || a->d_w2); }

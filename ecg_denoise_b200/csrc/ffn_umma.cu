@@ -40,23 +40,15 @@ struct FwdSmem {
 
 using umma::Ring;
 
-// TMA = true: the weight chunks of fc1 and fc2 arrive through cp.async.bulk.tensor (tma.cuh) in one 2-stage ring that
-// runs across both GEMMs (chunks 0 .. C/32 - 1 from W1, then TS/32 chunks from W2); one thread issues, the CTA only
-// derives the tf32 remainder tile.  TMA = false: the round-1 path (registers -> st.shared), kept for A/B.
-template <int C, bool TMA>
+// The weight chunks of fc1 and fc2 arrive through cp.async.bulk.tensor (tma.cuh) in one 2-stage ring that runs across
+// both GEMMs (chunks 0 .. C/32 - 1 from W1, then TS/32 chunks from W2); one thread issues, the CTA only derives the tf32
+// remainder tile.
+template <int C>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_ffn_fwd_args a,
                                                                       const __grid_constant__ CUtensorMap tm1,
                                                                       const __grid_constant__ CUtensorMap tm2) {
   constexpr int L = 2048 / C, HC = 4 * C, NSL = HC / TS;
-  constexpr int NCH1 = C / KC, NCH2 = TS / KC;
-  // the weights are not written by the preceding kernels of the step: pull the whole fc1 slice of this CTA into
-  // registers before waiting on the programmatic dependency, so its L2 latency hides behind the previous kernel
-  umma::KStage<TS, KC, RL_NT> w1r[TMA ? 1 : C / KC];
-  if constexpr (!TMA) {
-    const float* w1s = a.w1 + (size_t)(blockIdx.x % NSL) * TS * C;
-#pragma unroll
-    for (int j = 0; j < C / KC; ++j) w1r[j].load(w1s + j * KC, C, TS);
-  }
+  constexpr int NCH1 = C / KC;
   extern __shared__ __align__(1024) float smem[];
   float* sA_hi = smem;
   float* sA_lo = sA_hi + FwdSmem<C>::A_FLOATS;
@@ -97,13 +89,11 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
     umma::mbar_init(bars + 2, 1);
     umma::mbar_init(bars + 3, 1);
     umma::fence_mbar_init();
-    if constexpr (TMA) {
-      umma::fence_async_smem();
-      tma::prefetch_desc(&tm1);
-      tma::prefetch_desc(&tm2);
-      tma_issue(0);                      // weights are immutable inside the step: both ring buffers fill while the
-      tma_issue(1);                      // previous kernel drains
-    }
+    umma::fence_async_smem();
+    tma::prefetch_desc(&tm1);
+    tma::prefetch_desc(&tm2);
+    tma_issue(0);                        // weights are immutable inside the step: both ring buffers fill while the
+    tma_issue(1);                        // previous kernel drains
   }
   // ... and so does the LayerNorm affine: staged in shared memory here, phase 1 then waits for one round of global
   // loads (x) instead of one more round per 16-byte chunk
@@ -191,35 +181,22 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
     for (int j = 0; j < C / KC; ++j) {
       float* bh = sB + ring.buf() * 2 * FwdSmem<C>::B_FLOATS;
       float* bl = bh + FwdSmem<C>::B_FLOATS;
-      if constexpr (TMA) {
-        tma_consume(j, TS);
-      } else {
-        ring.wait_free();
-        w1r[j].store(bh, bl);
-      }
+      tma_consume(j, TS);
       umma::fence_async_smem();
       __syncthreads();
       if (tid == 0) {
         umma::tc_fence_after();
-        if constexpr (TMA) tma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
-        else umma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
+        tma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
         umma::commit(bars + ring.buf());
-        if constexpr (TMA) {             // refill this buffer with chunk j + 2 as soon as its MMAs have drained
-          ++ring.chunk;
-          ring.wait_last();
-          --ring.chunk;
-          tma_issue(j + 2);              // (NCH2 >= 2: chunk j + 2 always exists here)
-        }
+        // refill this buffer with chunk j + 2 as soon as its MMAs have drained (TS / KC >= 2: chunk j + 2 always
+        // exists here)
+        ++ring.chunk;
+        ring.wait_last();
+        --ring.chunk;
+        tma_issue(j + 2);
       }
       ++ring.chunk;
     }
-  }
-  // the fc2 slice of this CTA goes to registers now; its latency hides behind the epilogue below
-  umma::KStage<C, KC, RL_NT> w2r[TMA ? 1 : TS / KC];
-  if constexpr (!TMA) {
-    const float* w2s = a.w2 + (size_t)r * TS;
-#pragma unroll
-    for (int j = 0; j < TS / KC; ++j) w2r[j].load(w2s + j * KC, HC, C);
   }
   RL_TS(umma, 4);
   ring.wait_last();
@@ -292,26 +269,18 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
     for (int j = 0; j < TS / KC; ++j) {
       float* bh = sB + ring.buf() * 2 * FwdSmem<C>::B_FLOATS;
       float* bl = bh + FwdSmem<C>::B_FLOATS;
-      if constexpr (TMA) {
-        tma_consume(NCH1 + j, C);
-      } else {
-        ring.wait_free();
-        w2r[j].store(bh, bl);
-      }
+      tma_consume(NCH1 + j, C);
       umma::fence_async_smem();
       __syncthreads();
       if (tid == 0) {
         umma::tc_fence_after();
-        if constexpr (TMA) tma::mma_chunk_3x<KC>(tb + TS, sA_hi, sA_lo, TS, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
-        else umma::mma_chunk_3x<KC>(tb + TS, sA_hi, sA_lo, TS, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
+        tma::mma_chunk_3x<KC>(tb + TS, sA_hi, sA_lo, TS, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
         umma::commit(bars + ring.buf());
-        if constexpr (TMA) {
-          if (j + 2 < TS / KC) {
-            ++ring.chunk;
-            ring.wait_last();
-            --ring.chunk;
-            tma_issue(NCH1 + j + 2);
-          }
+        if (j + 2 < TS / KC) {
+          ++ring.chunk;
+          ring.wait_last();
+          --ring.chunk;
+          tma_issue(NCH1 + j + 2);
         }
       }
       ++ring.chunk;
@@ -731,31 +700,13 @@ int launch_cluster(void (*kernel)(const Args), size_t smem, int grid, int cl, co
 
 }  // namespace
 
-// returns 1 if the shape/mode is not handled here (caller falls through to the kernels in ffn_cluster.cu / ffn.cu)
-static int g_ffn_tma = -1;
-static int ffn_tma_on() {
-  if (g_ffn_tma < 0) {
-    const char* e = getenv("RALENET_UMMA_TMA");
-    g_ffn_tma = (e && e[0] == '0') ? 0 : 1;
-  }
-  return g_ffn_tma;
-}
-int rl_umma_tma_on() { return ffn_tma_on(); }
-extern "C" int ralenet_set_umma_tma(int on) {
-  const int prev = ffn_tma_on();
-  g_ffn_tma = on ? 1 : 0;
-  return prev;
-}
-
-template <int C, bool TMA>
+template <int C>
 static int launch_fwd(const rl_ffn_fwd_args* a, int tiles, cudaStream_t st) {
   constexpr int NSL = 4 * C / TS;
   CUtensorMap tm1 = {}, tm2 = {};
-  if (TMA) {
-    if (int rc = rl_tmap_weight(a->w1, 4 * C, C, C, TS, &tm1)) return rc;         // fc1 [4C][C]: 128-row slices
-    if (int rc = rl_tmap_weight(a->w2, C, 4 * C, 4 * C, C, &tm2)) return rc;      // fc2 [C][4C]: all C rows
-  }
-  auto kernel = ffn_fwd_umma_kernel<C, TMA>;
+  if (int rc = rl_tmap_weight(a->w1, 4 * C, C, C, TS, &tm1)) return rc;           // fc1 [4C][C]: 128-row slices
+  if (int rc = rl_tmap_weight(a->w2, C, 4 * C, 4 * C, C, &tm2)) return rc;        // fc2 [C][4C]: all C rows
+  auto kernel = ffn_fwd_umma_kernel<C>;
   const size_t smem = FwdSmem<C>::BYTES + 64;
   if (int rc = rl_set_smem(kernel, smem)) return rc;
   cudaLaunchConfig_t cfg = {};
@@ -777,12 +728,12 @@ static int launch_fwd(const rl_ffn_fwd_args* a, int tiles, cudaStream_t st) {
   return rl_check_launch("ffn_fwd_umma", C);
 }
 
+// returns 1 if the shape/mode is not handled here (caller falls through to the per-window kernels in ffn.cu)
 int rl_ffn_fwd_umma(const rl_ffn_fwd_args* a, cudaStream_t st) {
   if (a->L * a->C != 2048 || a->le_mode == RL_LE_DEPTHWISE) return 1;
   const int tiles = (a->B * a->L + TM - 1) / TM;
-  const bool tma_ok = ffn_tma_on() && ((uintptr_t)a->w1 % 16 == 0) && ((uintptr_t)a->w2 % 16 == 0);
-  if (a->C == 128) return tma_ok ? launch_fwd<128, true>(a, tiles, st) : launch_fwd<128, false>(a, tiles, st);
-  if (a->C == 64) return tma_ok ? launch_fwd<64, true>(a, tiles, st) : launch_fwd<64, false>(a, tiles, st);
+  if (a->C == 128) return launch_fwd<128>(a, tiles, st);
+  if (a->C == 64) return launch_fwd<64>(a, tiles, st);
   return 1;
 }
 

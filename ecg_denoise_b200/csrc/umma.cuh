@@ -18,12 +18,6 @@ namespace umma {
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-// float offset of element (r, k) in a K-major tile whose rows hold KT contraction elements:
-// K-adjacent core matrices are contiguous (LBO = 128 B), 8-row groups follow each other (SBO = KT/4 * 128 B)
-__host__ __device__ constexpr int koff(int r, int k, int KT) {
-  return (r % 8) * 4 + (k % 4) + (k / 4) * 32 + (r / 8) * (KT / 4) * 32;
-}
-
 __device__ __forceinline__ uint64_t make_desc(uint32_t byte_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;
   d |= (uint64_t)((byte_addr >> 4) & 0x3fff);
@@ -158,52 +152,12 @@ __device__ __forceinline__ float4 lo4(float4 v) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// Staging of a ROWS x KC operand block from a k-contiguous global matrix into a K-major tile pair
-// (hi = x, lo = x - trunc(x)):   element (r, k) <- src[r * ld + k]   (r < rows_valid, else 0).
-// src 16-byte aligned, ld % 4 == 0.  A warp covers 8 rows x 4 sixteen-byte chunks = 512 contiguous bytes of the
-// tile (conflict-free stores) and 8 x 64 contiguous bytes of global memory (full 32-byte sectors).
-// Split in two halves so that the global loads can be issued long before the tile buffer is free:
-// load() pulls the block into registers, store() splits and writes it.  NT = threads of the CTA.
-template <int ROWS, int KC, int NT>
-struct KStage {
-  static constexpr int NCH = KC / 4, RG = ROWS / 8, QG = NCH / 4;
-  static constexpr int ITEMS = RG * QG;                      // warp-wide groups of 8 rows x 4 chunks
-  static constexpr int PER = (ITEMS + NT / 32 - 1) / (NT / 32);
-  static_assert(ROWS % 8 == 0 && NCH % 4 == 0, "KStage: tile shape");
-  float4 v[PER];
-
-  __device__ __forceinline__ void load(const float* __restrict__ src, int ld, int rows_valid) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int rsub = lane & 7, qsub = lane >> 3;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) {
-      const int grp = wid + i * (NT / 32);
-      const int rgrp = grp % RG, qgrp = grp / RG;
-      const int r = rgrp * 8 + rsub, q = qgrp * 4 + qsub;
-      v[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (grp < ITEMS && r < rows_valid) v[i] = __ldg(reinterpret_cast<const float4*>(src + (size_t)r * ld) + q);
-    }
-  }
-  __device__ __forceinline__ void store(float* hi, float* lo) const {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int rsub = lane & 7, qsub = lane >> 3;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) {
-      const int grp = wid + i * (NT / 32);
-      if (grp < ITEMS) {
-        const int rgrp = grp % RG, qgrp = grp / RG;
-        const int o = rsub * 4 + (qgrp * 4 + qsub) * 32 + rgrp * (NCH * 32);
-        *reinterpret_cast<float4*>(hi + o) = v[i];
-        *reinterpret_cast<float4*>(lo + o) = lo4(v[i]);
-      }
-    }
-  }
-};
-
-// Transposing variant for operands whose contraction index is the ROW of the global matrix (dgrad: B = W^T):
-//   element (n, k) <- src[k * ld + n],  n < ROWS (multiple of 32), k < KC.
-// A warp reads 32 consecutive n of four consecutive k rows (4 x 128 contiguous bytes) and each lane writes one
-// 16-byte chunk (its n, four k) of the K-major tile.
+// Staging of a ROWS x KC operand block whose contraction index is the ROW of the global matrix (dgrad: B = W^T) into a
+// K-major tile pair (hi = x, lo = x - trunc(x)):   element (n, k) <- src[k * ld + n],  n < ROWS (multiple of 32),
+// k < KC.  A warp reads 32 consecutive n of four consecutive k rows (4 x 128 contiguous bytes) and each lane writes one
+// 16-byte chunk (its n, four k) of the K-major tile.  Split in two halves so that the global loads can be issued long
+// before the tile buffer is free: load() pulls the block into registers, store() splits and writes it.  NT = threads of
+// the CTA.
 template <int ROWS, int KC, int NT>
 struct TStage {
   static constexpr int NB = ROWS / 32, NQ = KC / 4, ITEMS = NB * NQ;

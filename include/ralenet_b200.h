@@ -118,10 +118,6 @@ int ralenet_set_wgrad_umma(int on);
  * 32 x 32 tiles (the HBM-bound ones: C = 32 stages and the 32-wide patch layers), 2 = every eligible group.
  * Same function; A/B switch, initial value from RALENET_WGRAD_REG.  Returns the previous setting. */
 int ralenet_set_wgrad_reg(int on);
-/* Weight staging of the tcgen05 forward kernels (feed-forward and attention tile kernels, C = 64, 128): 1 (default) = TMA (cp.async.bulk.tensor into
- * the SWIZZLE_128B layout, tma.cuh), 0 = the round-1 path (ld.global -> registers -> st.shared).  Same function; A/B
- * switch, initial value from RALENET_UMMA_TMA.  Returns the previous setting. */
-int ralenet_set_umma_tma(int on);
 
 /* ------------------------------------------------------------------------------------------
  * Feed-forward half:  y = x + fc2(GELU(leconv(GELU(fc1(LN2(x))))))  (+ extra)
