@@ -42,7 +42,7 @@ void rl_prof_pre(cudaStream_t st) {
   }
 }
 
-int rl_check_launch(const char* what, int t0, int t1) {
+int rl_check_launch(const char* what, int t0, int t1, const char* suffix) {
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
     rl_set_error("%s: %s", what, cudaGetErrorString(e));
@@ -51,9 +51,9 @@ int rl_check_launch(const char* what, int t0, int t1) {
   ++g_launches;
   if (g_prof.on && g_prof.n < kMaxProf) {
     const int i = g_prof.n++;
-    if (t1 >= 0) snprintf(g_prof.label[i], sizeof(g_prof.label[i]), "%s<%d,%d>", what, t0, t1);
-    else if (t0 >= 0) snprintf(g_prof.label[i], sizeof(g_prof.label[i]), "%s<%d>", what, t0);
-    else snprintf(g_prof.label[i], sizeof(g_prof.label[i]), "%s", what);
+    if (t1 >= 0) snprintf(g_prof.label[i], sizeof(g_prof.label[i]), "%s<%d,%d>%s", what, t0, t1, suffix);
+    else if (t0 >= 0) snprintf(g_prof.label[i], sizeof(g_prof.label[i]), "%s<%d>%s", what, t0, suffix);
+    else snprintf(g_prof.label[i], sizeof(g_prof.label[i]), "%s%s", what, suffix);
     cudaEventRecord(g_prof.ev[i + 1], g_prof.stream);
   }
   return RL_OK;

@@ -45,7 +45,8 @@ size_t attn_fwd_smem(int L) {
 }
 
 // ---------------------------------------------------------------------------------------------
-template <int C, int WIN, int NWC>
+// TF32: single-pass projection GEMMs (RL_F_TF32, see MmaTile::mac); the attention core is the same in both forms
+template <int C, int WIN, int NWC, bool TF32>
 __device__ __forceinline__ void attn_fwd_body(const rl_attn_fwd_args& a, float* smem) {
   constexpr int L = 2048 * WIN / C, H = C / RL_HD, M = NWC * L;      // M token rows (NWC whole windows) per CTA
   constexpr int LDC = ld_mk(C);
@@ -92,7 +93,7 @@ __device__ __forceinline__ void attn_fwd_body(const rl_attn_fwd_args& a, float* 
   {
     MmaTile<M, 3 * C> acc;
     acc.init();
-    WS::Qkv::template run<true>(acc, su, LDC, sw, a.wq, C, a.wkv, C);
+    WS::Qkv::template run<true, TF32>(acc, su, LDC, sw, a.wq, C, a.wkv, C);
     WS::Proj::prefetch(sw, a.wp, C, nullptr, C);              // lands while the attention core runs
     const float* bq = a.bq;
     const float* bkv = a.bkv;
@@ -136,7 +137,7 @@ __device__ __forceinline__ void attn_fwd_body(const rl_attn_fwd_args& a, float* 
     // MMAs (ncu r2_v24: 8 % of the samples of block_fwd<16> sat on these loads when they followed the GEMM)
     float rv[MmaTile<M, C>::RT][MmaTile<M, C>::CT][4] = {};
     if (a.flags & RL_F_RESIDUAL) acc.gather(xw, C, rv);
-    WS::Proj::template run<true>(acc, sq, LDC, sw, a.wp, C, nullptr, C);
+    WS::Proj::template run<true, TF32>(acc, sq, LDC, sw, a.wp, C, nullptr, C);
     RL_TS(attn, 7);
     const float* bp = a.bp;
     float* yw = a.y + woff;
@@ -152,10 +153,10 @@ __device__ __forceinline__ void attn_fwd_body(const rl_attn_fwd_args& a, float* 
   RL_TS(attn, 8);
 }
 
-template <int C, int WIN, int NWC>
+template <int C, int WIN, int NWC, bool TF32>
 __global__ void __launch_bounds__(RL_NT, (NWC >= 4) ? 1 : RL_MINB) attn_fwd_kernel(const rl_attn_fwd_args a) {
   extern __shared__ __align__(16) float smem[];
-  attn_fwd_body<C, WIN, NWC>(a, smem);
+  attn_fwd_body<C, WIN, NWC, TF32>(a, smem);
 }
 
 // One launch per TransformerBlock for the narrow stages (C <= 32, one window per CTA): attention half, then the
@@ -163,12 +164,12 @@ __global__ void __launch_bounds__(RL_NT, (NWC >= 4) ? 1 : RL_MINB) attn_fwd_kern
 // backward needs it anyway) and read back by the same CTA through L2-coherent loads after a CTA barrier; the second
 // half's first weight chunk is requested before that barrier.  Saves a launch boundary (drain + fill + dependency
 // wait) per block: 10 of the 36 block-half launches of a forward pass.
-template <int C>
+template <int C, bool TF32>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) block_fwd_kernel(const rl_attn_fwd_args a, const rl_ffn_fwd_args f) {
   extern __shared__ __align__(16) float smem[];
-  attn_fwd_body<C, 1, 1>(a, smem);
+  attn_fwd_body<C, 1, 1, TF32>(a, smem);
   __syncthreads();                       // every thread's part of x1 is in global memory; the attention tiles are dead
-  ffn_fwd_body<C, 1, true>(f, smem);
+  ffn_fwd_body<C, 1, true, TF32>(f, smem);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -404,23 +405,23 @@ rl_attn_fwd_args attn_fwd_slice(const rl_attn_fwd_args& a, int w0, int n) {
 }
 
 // launches floor(B / NWC) CTAs of NWC windows each; returns the number of windows covered through *done
-template <int C, int NWC>
+template <int C, int NWC, bool TF32>
 int launch_fwd_groups(const rl_attn_fwd_args* a, cudaStream_t st, int* done) {
   const size_t smem = attn_fwd_smem<C, NWC>(a->L);
-  if (int rc = rl_set_smem(attn_fwd_kernel<C, 1, NWC>, smem)) return rc;
-  rl_launch_pdl(attn_fwd_kernel<C, 1, NWC>, dim3(a->B / NWC), dim3(RL_NT), smem, st, *a);
+  if (int rc = rl_set_smem(attn_fwd_kernel<C, 1, NWC, TF32>, smem)) return rc;
+  rl_launch_pdl(attn_fwd_kernel<C, 1, NWC, TF32>, dim3(a->B / NWC), dim3(RL_NT), smem, st, *a);
   *done = (a->B / NWC) * NWC;
-  return rl_check_launch("attn_fwd_kernel", C, NWC);
+  return rl_check_launch("attn_fwd_kernel", C, NWC, rl_tf32_tag(TF32));
 }
 
-template <int C>
+template <int C, bool TF32>
 int launch_fwd(const rl_attn_fwd_args* a, cudaStream_t st) {
   const int win = a->L * C / 2048;
   if (win != 1) {
     const size_t smem = attn_fwd_smem<C, 1>(a->L);
-    if (int rc = rl_set_smem(attn_fwd_kernel<C, 2, 1>, smem)) return rc;
-    rl_launch_pdl(attn_fwd_kernel<C, 2, 1>, dim3(a->B), dim3(RL_NT), smem, st, *a);
-    return rl_check_launch("attn_fwd_kernel", C);
+    if (int rc = rl_set_smem(attn_fwd_kernel<C, 2, 1, TF32>, smem)) return rc;
+    rl_launch_pdl(attn_fwd_kernel<C, 2, 1, TF32>, dim3(a->B), dim3(RL_NT), smem, st, *a);
+    return rl_check_launch("attn_fwd_kernel", C, -1, rl_tf32_tag(TF32));
   }
   if (C >= 64) {
     const int rc = rl_attn_fwd_umma(a, st);                      // 1: shape / batch not handled there
@@ -428,12 +429,16 @@ int launch_fwd(const rl_attn_fwd_args* a, cudaStream_t st) {
   }
   int done = 0;
   if (C >= 64 && a->B >= RL_NWC_MIN_B) {
-    if (int rc = launch_fwd_groups<C, (C >= 64) ? 2 : 1>(a, st, &done)) return rc;
+    if (int rc = launch_fwd_groups<C, (C >= 64) ? 2 : 1, TF32>(a, st, &done)) return rc;
   }
   if (done == a->B) return RL_OK;
   const rl_attn_fwd_args rest = attn_fwd_slice(*a, done, a->B - done);     // the odd windows, one per CTA
   int d1 = 0;
-  return launch_fwd_groups<C, 1>(&rest, st, &d1);
+  return launch_fwd_groups<C, 1, TF32>(&rest, st, &d1);
+}
+template <int C>
+int launch_fwd(const rl_attn_fwd_args* a, cudaStream_t st) {
+  return (a->flags & RL_F_TF32) ? launch_fwd<C, true>(a, st) : launch_fwd<C, false>(a, st);
 }
 
 template <int C, int WIN, bool DET>
@@ -473,13 +478,17 @@ int check_shape(int B, int L, int C, int H, int W, int c0) {
   return RL_OK;
 }
 
-template <int C>
+template <int C, bool TF32>
 int launch_block_fwd(const rl_attn_fwd_args* a, const rl_ffn_fwd_args* f, cudaStream_t st) {
   const size_t s1 = attn_fwd_smem<C, 1>(a->L), s2 = ffn_fwd_smem<C>(a->L);
   const size_t smem = s1 > s2 ? s1 : s2;
-  if (int rc = rl_set_smem(block_fwd_kernel<C>, smem)) return rc;
-  rl_launch_pdl(block_fwd_kernel<C>, dim3(a->B), dim3(RL_NT), smem, st, *a, *f);
-  return rl_check_launch("block_fwd_kernel", C);
+  if (int rc = rl_set_smem(block_fwd_kernel<C, TF32>, smem)) return rc;
+  rl_launch_pdl(block_fwd_kernel<C, TF32>, dim3(a->B), dim3(RL_NT), smem, st, *a, *f);
+  return rl_check_launch("block_fwd_kernel", C, -1, rl_tf32_tag(TF32));
+}
+template <int C>
+int launch_block_fwd(const rl_attn_fwd_args* a, const rl_ffn_fwd_args* f, cudaStream_t st) {
+  return (a->flags & RL_F_TF32) ? launch_block_fwd<C, true>(a, f, st) : launch_block_fwd<C, false>(a, f, st);
 }
 
 int g_block_fuse = -1;
@@ -504,6 +513,7 @@ extern "C" int ralenet_set_block_fuse(int on) {
 // two halves one after the other.
 extern "C" int ralenet_block_fwd(const rl_attn_fwd_args* a, const rl_ffn_fwd_args* f, void* stream) {
   RL_REQUIRE(a && f, RL_ERR_NULL, "block_fwd: args is NULL");
+  RL_REQUIRE(((a->flags ^ f->flags) & RL_F_TF32) == 0, RL_ERR_SHAPE, "block_fwd: the halves differ in RL_F_TF32");
   const int want = RL_F_PRENORM | RL_F_RESIDUAL;
   const bool fuse = block_fuse_on() && a->C <= 32 && a->L * a->C == 2048 && f->x == a->y && f->B == a->B &&
                     f->L == a->L && f->C == a->C && (a->flags & want) == want && (f->flags & want) == want &&
@@ -517,6 +527,8 @@ extern "C" int ralenet_block_fwd(const rl_attn_fwd_args* a, const rl_ffn_fwd_arg
              "block_fwd: NULL attention tensor");
   RL_REQUIRE(a->W == 0 || a->table, RL_ERR_NULL, "block_fwd: W>0 needs table");
   RL_REQUIRE(!a->q || (a->k && a->v && a->o && a->lse), RL_ERR_NULL, "block_fwd: partial save set");
+  RL_REQUIRE(!(a->flags & RL_F_TF32) || !(a->q || a->k || a->v || a->o || a->lse || f->h), RL_ERR_SHAPE,
+             "block_fwd: RL_F_TF32 is inference only (saved-tensor pointers must be NULL)");
   RL_REQUIRE(f->y && f->w1 && f->w2 && f->ln_w && f->ln_b, RL_ERR_NULL, "block_fwd: NULL feed-forward tensor");
   RL_REQUIRE(f->le_mode == RL_LE_NONE || f->lew, RL_ERR_NULL, "block_fwd: local-enhancement weights missing");
   RL_REQUIRE(rl_al16(a->x, a->y, a->pe, a->ln_w, a->ln_b, a->wq, a->wkv, a->wp, a->q, a->k, a->v, a->o, f->y, f->w1, f->w2,
@@ -538,6 +550,8 @@ extern "C" int ralenet_attn_fwd(const rl_attn_fwd_args* a, void* stream) {
   RL_REQUIRE(!(a->flags & RL_F_PRENORM) || (a->pe && a->ln_w && a->ln_b), RL_ERR_NULL, "attn_fwd: prenorm needs pe/ln");
   RL_REQUIRE(a->W == 0 || a->table, RL_ERR_NULL, "attn_fwd: W>0 needs table");
   RL_REQUIRE(!a->q || (a->k && a->v && a->o && a->lse), RL_ERR_NULL, "attn_fwd: partial save set");
+  RL_REQUIRE(!(a->flags & RL_F_TF32) || !(a->q || a->k || a->v || a->o || a->lse), RL_ERR_SHAPE,
+             "attn_fwd: RL_F_TF32 is inference only (q/k/v/o/lse must be NULL)");
   RL_REQUIRE(rl_al16(a->x, a->y, a->pe, a->ln_w, a->ln_b, a->wq, a->wkv, a->wp, a->q, a->k, a->v, a->o), RL_ERR_SHAPE,
              "attn_fwd: tensors must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
@@ -554,6 +568,7 @@ extern "C" int ralenet_attn_fwd(const rl_attn_fwd_args* a, void* stream) {
 // the data-gradient kernel (also writes the dqkv / u scratch of the weight gradients)
 int rl_attn_bwd_main(const rl_attn_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(a, RL_ERR_NULL, "attn_bwd: args is NULL");
+  RL_REQUIRE(!(a->flags & RL_F_TF32), RL_ERR_SHAPE, "attn_bwd: RL_F_TF32 is a forward-only (inference) flag");
   if (int rc = check_shape(a->B, a->L, a->C, a->H, a->W, a->c0)) return rc;
   RL_REQUIRE(a->g && a->x && a->wq && a->wkv && a->wp && a->q && a->k && a->v && a->o && a->lse && a->dx && a->dqkv &&
                  a->u,

@@ -58,8 +58,9 @@ struct ASmem {
 
 // The weight operands arrive through cp.async.bulk.tensor (tma.cuh): per 32-wide K chunk three 32-row boxes (the q, k
 // and v rows of this CTA's head slice, from to_q and the two halves of to_kv) into one 96-row SWIZZLE_128B tile, and one
-// C-row box for the K-slice of the output projection.
-template <int C>
+// C-row box for the K-slice of the output projection.  TF32 (RL_F_TF32): single-pass projection MMAs on operand tiles
+// rounded to tf32 (no remainder tiles); the attention core is the same in both forms.
+template <int C, bool TF32>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_attn_fwd_args a,
                                                                        const __grid_constant__ CUtensorMap tmq,
                                                                        const __grid_constant__ CUtensorMap tmkv,
@@ -193,8 +194,12 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
       }
       if (!ok) u = make_float4(0.f, 0.f, 0.f, 0.f);
       const int o = rsub * 4 + qc * 32 + warp * (C / 4) * 32;
-      *reinterpret_cast<float4*>(sA_hi + o) = u;
-      *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(u);
+      if constexpr (TF32) {
+        *reinterpret_cast<float4*>(sA_hi + o) = umma::rna4(u);
+      } else {
+        *reinterpret_cast<float4*>(sA_hi + o) = u;
+        *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(u);
+      }
     }
   }
   umma::tc_fence_before();
@@ -212,12 +217,12 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
       float* bh = sB + ring.buf() * 2 * NQ * KC;
       float* bl = bh + NQ * KC;
       umma::mbar_wait(bars + 2 + (j & 1), (uint32_t)((j >> 1) & 1));
-      tma::derive_lo<RL_NT>(bh, bl, NQ * KC);
+      tma::derive_lo<RL_NT, TF32>(bh, bl, NQ * KC);
       umma::fence_async_smem();
       __syncthreads();
       if (tid == 0) {
         umma::tc_fence_after();
-        tma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
+        tma::mma_chunk_3x<KC, TF32>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
         umma::commit(bars + ring.buf());
         if (j + 2 < NCHK) {              // refill this buffer once its MMAs have drained
           ++ring.chunk;
@@ -324,17 +329,21 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
       const float4 o4 = *reinterpret_cast<const float4*>(sq + row * LDS + 4 * qc);
       if (a.o && row < nvalid) *reinterpret_cast<float4*>(a.o + (tok0 + row) * C + CS * r + 4 * qc) = o4;
       const int o = rsub * 4 + qc * 32 + warp * (CS / 4) * 32;
-      *reinterpret_cast<float4*>(sO_hi + o) = o4;
-      *reinterpret_cast<float4*>(sO_lo + o) = umma::lo4(o4);
+      if constexpr (TF32) {
+        *reinterpret_cast<float4*>(sO_hi + o) = umma::rna4(o4);
+      } else {
+        *reinterpret_cast<float4*>(sO_hi + o) = o4;
+        *reinterpret_cast<float4*>(sO_lo + o) = umma::lo4(o4);
+      }
     }
     umma::mbar_wait(bars + 4, 0u);
-    tma::derive_lo<RL_NT>(sW_hi, sW_lo, C * CS);
+    tma::derive_lo<RL_NT, TF32>(sW_hi, sW_lo, C * CS);
     umma::fence_async_smem();
     __syncthreads();
     if (tid == 0) {
       constexpr uint32_t idesc = umma::idesc_tf32(TM, C);
       umma::tc_fence_after();
-      tma::mma_chunk_3x<CS>(tb + NQ, sO_hi, sO_lo, CS, 0, sW_hi, sW_lo, idesc, 0u);
+      tma::mma_chunk_3x<CS, TF32>(tb + NQ, sO_hi, sO_lo, CS, 0, sW_hi, sW_lo, idesc, 0u);
       umma::commit(bars + ring.buf());
     }
     ++ring.chunk;
@@ -404,7 +413,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
   RL_TS(attn_umma, 12);
 }
 
-template <int C>
+template <int C, bool TF32>
 int launch(const rl_attn_fwd_args& a, cudaStream_t st) {
   constexpr int NSL = C / CS;
   const int tiles = (a.B * a.L + TM - 1) / TM;
@@ -412,7 +421,7 @@ int launch(const rl_attn_fwd_args& a, cudaStream_t st) {
   if (int rc = rl_tmap_weight(a.wq, C, C, C, CS, &tmq)) return rc;            // to_q  [C][C]:  32-row boxes
   if (int rc = rl_tmap_weight(a.wkv, 2 * C, C, C, CS, &tmkv)) return rc;      // to_kv [2C][C]: 32-row boxes
   if (int rc = rl_tmap_weight(a.wp, C, C, C, C, &tmp)) return rc;             // proj  [C][C]:  all C rows, 32 columns
-  auto kernel = attn_fwd_umma_kernel<C>;
+  auto kernel = attn_fwd_umma_kernel<C, TF32>;
   if (int rc = rl_set_smem(kernel, ASmem<C>::BYTES)) return rc;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(tiles * NSL);
@@ -430,7 +439,7 @@ int launch(const rl_attn_fwd_args& a, cudaStream_t st) {
   cfg.numAttrs = 2;
   rl_prof_pre(st);
   cudaLaunchKernelEx(&cfg, kernel, a, tmq, tmkv, tmp);
-  return rl_check_launch("attn_fwd_umma", C);
+  return rl_check_launch("attn_fwd_umma", C, -1, rl_tf32_tag(TF32));
 }
 
 }  // namespace
@@ -470,6 +479,7 @@ int rl_attn_fwd_umma(const rl_attn_fwd_args* a, cudaStream_t st) {
     const int ctas = (a->B * a->L + TM - 1) / TM * (a->C / CS);
     if (ctas > n_sm) return 1;
   }
-  if (a->C == 128) return launch<128>(*a, st);
-  return launch<64>(*a, st);
+  const bool tf32 = a->flags & RL_F_TF32;
+  if (a->C == 128) return tf32 ? launch<128, true>(*a, st) : launch<128, false>(*a, st);
+  return tf32 ? launch<64, true>(*a, st) : launch<64, false>(*a, st);
 }

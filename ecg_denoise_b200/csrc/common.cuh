@@ -34,7 +34,9 @@
 
 void rl_set_error(const char* fmt, ...);
 void rl_count_launch();
-int rl_check_launch(const char* what, int tag0 = -1, int tag1 = -1);
+// profiler label "what<tag0,tag1>suffix" (suffix ":tf32" marks the single-pass TF32 forward kernels)
+int rl_check_launch(const char* what, int tag0 = -1, int tag1 = -1, const char* suffix = "");
+constexpr const char* rl_tf32_tag(bool tf32) { return tf32 ? ":tf32" : ""; }
 void rl_prof_pre(cudaStream_t st);     // profiling: event right before the next launch on the profiled stream
 
 #define RL_REQUIRE(cond, code, ...)            \
@@ -408,6 +410,13 @@ __device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], 
       : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
 }
+// single-pass TF32 operand (RL_F_TF32): x rounded to nearest (ties away) to a 10-bit mantissa.  Rounding, not the
+// truncation of split_tf32, so that the errors of a long contraction (fc2: 4C = 512 terms) do not all lean one way.
+__device__ __forceinline__ uint32_t rna_tf32(float x) {
+  uint32_t r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+  return r;
+}
 // x = hi + lo exactly; hi has a 10-bit mantissa (truncated), lo is fed as is (the MMA ignores its low 13 bits)
 __device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
   hi = __float_as_uint(x) & 0xffffe000u;
@@ -473,7 +482,8 @@ struct MmaTile {
   }
 
   // acc += A[:, 0:K] * B[0:K, :]   (K % 8 == 0; A and B point at k = 0 of the chunk)
-  template <int AL, int BL>
+  // TF32: one MMA per fragment pair on rounded operands (inference precision RL_F_TF32) instead of the 3-pass split
+  template <int AL, int BL, bool TF32 = false>
   __device__ __forceinline__ void mac(const float* __restrict__ A, int lda, const float* __restrict__ B, int ldb,
                                       int K) {
     const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
@@ -491,8 +501,12 @@ struct MmaTile {
           const float* p = A + (k0 + t) * lda + m;
           a0 = p[0]; a1 = p[8]; a2 = p[4 * lda]; a3 = p[4 * lda + 8];
         }
-        split_tf32x2(a0, a1, ahi[r][0], ahi[r][1], alo[r][0], alo[r][1]);
-        split_tf32x2(a2, a3, ahi[r][2], ahi[r][3], alo[r][2], alo[r][3]);
+        if constexpr (TF32) {
+          ahi[r][0] = rna_tf32(a0); ahi[r][1] = rna_tf32(a1); ahi[r][2] = rna_tf32(a2); ahi[r][3] = rna_tf32(a3);
+        } else {
+          split_tf32x2(a0, a1, ahi[r][0], ahi[r][1], alo[r][0], alo[r][1]);
+          split_tf32x2(a2, a3, ahi[r][2], ahi[r][3], alo[r][2], alo[r][3]);
+        }
       }
 #pragma unroll
       for (int c = 0; c < CT; ++c) {
@@ -506,11 +520,17 @@ struct MmaTile {
           b0 = p[0]; b1 = p[4 * ldb];
         }
         uint32_t bhi[2], blo[2];
-        split_tf32x2(b0, b1, bhi[0], bhi[1], blo[0], blo[1]);
+        if constexpr (TF32) {
+          bhi[0] = rna_tf32(b0); bhi[1] = rna_tf32(b1);
+        } else {
+          split_tf32x2(b0, b1, bhi[0], bhi[1], blo[0], blo[1]);
+        }
 #pragma unroll
         for (int r = 0; r < RT; ++r) {
-          mma_tf32(acc[r][c], alo[r], bhi);
-          mma_tf32(acc[r][c], ahi[r], blo);
+          if constexpr (!TF32) {
+            mma_tf32(acc[r][c], alo[r], bhi);
+            mma_tf32(acc[r][c], ahi[r], blo);
+          }
           mma_tf32(acc[r][c], ahi[r], bhi);
         }
       }
@@ -696,8 +716,8 @@ struct WStream {
 
   // acc += A[:, 0:K] * W      (A in smem, A_MK with stride lda; sw holds FLOATS floats).  When the K range is the
   // concatenation of several A arrays (a_seg columns each, a_seg % KC == 0) the next one starts a_seg_stride floats
-  // after the previous.  Ends with a barrier: afterwards sw (and A) may be overwritten.
-  template <bool PREFETCHED = false, class Acc>
+  // after the previous.  Ends with a barrier: afterwards sw (and A) may be overwritten.  TF32: see MmaTile::mac.
+  template <bool PREFETCHED = false, bool TF32 = false, class Acc>
   __device__ static __forceinline__ void run(Acc& acc, const float* A, int lda, float* sw,
                                              const float* __restrict__ W0, int split,
                                              const float* __restrict__ W1, int ldw, int a_seg = K,
@@ -716,7 +736,8 @@ struct WStream {
           cp_async_commit();                          // empty group keeps the wait count static
       }
       const int k0 = c * KC;
-      acc.template mac<A_MK, BL>(A + (k0 / a_seg) * a_seg_stride + (k0 % a_seg), lda, sw + (c % NSE) * STAGE, LD, KC);
+      acc.template mac<A_MK, BL, TF32>(A + (k0 / a_seg) * a_seg_stride + (k0 % a_seg), lda, sw + (c % NSE) * STAGE, LD,
+                                       KC);
     }
     __syncthreads();
   }

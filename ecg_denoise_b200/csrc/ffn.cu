@@ -19,10 +19,10 @@ int rl_ffn_bwd_umma(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det);
 
 namespace {
 
-template <int C, int WIN>
+template <int C, int WIN, bool TF32>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_kernel(const rl_ffn_fwd_args a) {
   extern __shared__ __align__(16) float smem[];
-  ffn_fwd_body<C, WIN, false>(a, smem);
+  ffn_fwd_body<C, WIN, false, TF32>(a, smem);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -273,17 +273,21 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_kernel(const rl_ffn_bw
   }
 }
 
-template <int C>
+template <int C, bool TF32>
 int launch_fwd(const rl_ffn_fwd_args* a, cudaStream_t st) {
   const size_t smem = ffn_fwd_smem<C>(a->L);
   if (a->L * C == 2048) {
-    if (int rc = rl_set_smem(ffn_fwd_kernel<C, 1>, smem)) return rc;
-    rl_launch_pdl(ffn_fwd_kernel<C, 1>, dim3(a->B), dim3(RL_NT), smem, st, *a);
+    if (int rc = rl_set_smem(ffn_fwd_kernel<C, 1, TF32>, smem)) return rc;
+    rl_launch_pdl(ffn_fwd_kernel<C, 1, TF32>, dim3(a->B), dim3(RL_NT), smem, st, *a);
   } else {
-    if (int rc = rl_set_smem(ffn_fwd_kernel<C, 2>, smem)) return rc;
-    rl_launch_pdl(ffn_fwd_kernel<C, 2>, dim3(a->B), dim3(RL_NT), smem, st, *a);
+    if (int rc = rl_set_smem(ffn_fwd_kernel<C, 2, TF32>, smem)) return rc;
+    rl_launch_pdl(ffn_fwd_kernel<C, 2, TF32>, dim3(a->B), dim3(RL_NT), smem, st, *a);
   }
-  return rl_check_launch("ffn_fwd_kernel", C);
+  return rl_check_launch("ffn_fwd_kernel", C, -1, rl_tf32_tag(TF32));
+}
+template <int C>
+int launch_fwd(const rl_ffn_fwd_args* a, cudaStream_t st) {
+  return (a->flags & RL_F_TF32) ? launch_fwd<C, true>(a, st) : launch_fwd<C, false>(a, st);
 }
 
 template <int C, int WIN, bool DW, bool DET>
@@ -336,6 +340,7 @@ extern "C" int ralenet_ffn_fwd(const rl_ffn_fwd_args* a, void* stream) {
   RL_REQUIRE(a->x && a->y && a->w1 && a->w2, RL_ERR_NULL, "ffn_fwd: NULL tensor");
   RL_REQUIRE(!(a->flags & RL_F_PRENORM) || (a->ln_w && a->ln_b), RL_ERR_NULL, "ffn_fwd: prenorm needs ln");
   RL_REQUIRE(a->le_mode == RL_LE_NONE || a->lew, RL_ERR_NULL, "ffn_fwd: le_mode needs lew");
+  RL_REQUIRE(!(a->flags & RL_F_TF32) || !a->h, RL_ERR_SHAPE, "ffn_fwd: RL_F_TF32 is inference only (h must be NULL)");
   RL_REQUIRE(rl_al16(a->x, a->y, a->w1, a->w2, a->ln_w, a->ln_b, a->h, a->extra), RL_ERR_SHAPE,
              "ffn_fwd: tensors must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
@@ -353,6 +358,7 @@ extern "C" int ralenet_ffn_fwd(const rl_ffn_fwd_args* a, void* stream) {
 
 int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   RL_REQUIRE(a, RL_ERR_NULL, "ffn_bwd: args is NULL");
+  RL_REQUIRE(!(a->flags & RL_F_TF32), RL_ERR_SHAPE, "ffn_bwd: RL_F_TF32 is a forward-only (inference) flag");
   if (int rc = check_shape(a->B, a->L, a->C, a->le_mode)) return rc;
   RL_REQUIRE(a->g && a->x && a->w1 && a->w2 && a->h && a->dx && a->dh && a->g2 && a->u, RL_ERR_NULL,
              "ffn_bwd: NULL tensor");

@@ -14,8 +14,8 @@ size_t ffn_fwd_smem(int L) {
 
 // CHAIN = true: second half of a fused block kernel (attn.cu::block_fwd_kernel): the input a.x was written by this
 // very CTA a moment ago (the attention half's output), so there is no programmatic-dependency wait and the input is
-// read with L2-coherent loads.
-template <int C, int WIN, bool CHAIN>
+// read with L2-coherent loads.  TF32: single-pass GEMMs (RL_F_TF32, see MmaTile::mac).
+template <int C, int WIN, bool CHAIN, bool TF32>
 __device__ __forceinline__ void ffn_fwd_body(const rl_ffn_fwd_args& a, float* smem) {
   constexpr int L = 2048 * WIN / C;
   constexpr int LDC = ld_mk(C);
@@ -54,7 +54,7 @@ __device__ __forceinline__ void ffn_fwd_body(const rl_ffn_fwd_args& a, float* sm
   {
     MmaTile<L, HC> acc;
     acc.init();
-    WStream<HC, C, B_NK>::template run<true>(acc, su, LDC, sw, a.w1, HC, nullptr, C);
+    WStream<HC, C, B_NK>::template run<true, TF32>(acc, su, LDC, sw, a.w1, HC, nullptr, C);
     WStream<C, HC, B_NK>::prefetch(sw, a.w2, C, nullptr, HC);      // lands behind the GELU / local-enhancement phase
     const float* b1 = a.b1;
     float* hs = a.h ? a.h + (size_t)blockIdx.x * L * HC : nullptr;
@@ -111,7 +111,7 @@ __device__ __forceinline__ void ffn_fwd_body(const rl_ffn_fwd_args& a, float* sm
     // before the fc2 GEMM so that the round trip passes behind the MMAs
     float rv[MmaTile<L, C>::RT][MmaTile<L, C>::CT][4] = {}, ev[MmaTile<L, C>::RT][MmaTile<L, C>::CT][4] = {};
     if (resid) acc.template gather<CHAIN>(xw, C, rv);
-    WStream<C, HC, B_NK>::template run<true>(acc, sh, LDH, sw, a.w2, C, nullptr, HC);
+    WStream<C, HC, B_NK>::template run<true, TF32>(acc, sh, LDH, sw, a.w2, C, nullptr, HC);
     const float* b2 = a.b2;
     const float* ex = a.extra ? a.extra + woff : nullptr;
     float* yw = a.y + woff;

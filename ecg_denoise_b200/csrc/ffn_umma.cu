@@ -42,8 +42,9 @@ using umma::Ring;
 
 // The weight chunks of fc1 and fc2 arrive through cp.async.bulk.tensor (tma.cuh) in one 2-stage ring that runs across
 // both GEMMs (chunks 0 .. C/32 - 1 from W1, then TS/32 chunks from W2); one thread issues, the CTA only derives the tf32
-// remainder tile.
-template <int C>
+// remainder tile.  TF32 (RL_F_TF32): single-pass MMAs; the CTA rounds the operand tiles to tf32 instead of splitting them
+// (the remainder halves of the shared-memory plan stay unused).
+template <int C, bool TF32>
 __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_ffn_fwd_args a,
                                                                       const __grid_constant__ CUtensorMap tm1,
                                                                       const __grid_constant__ CUtensorMap tm2) {
@@ -72,15 +73,16 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
       tma::load_2d(dst, &tm2, r_early * TS + (jj - NCH1) * KC, 0, bars + 2 + b);
     }
   };
-  // all threads: wait for chunk jj, derive its remainder tile (same swizzled layout, element-wise)
+  // all threads: wait for chunk jj, derive its remainder tile (same swizzled layout, element-wise; TF32: round in place)
   auto tma_consume = [&](int jj, int rows) {
     const int b = jj & 1;
     umma::mbar_wait(bars + 2 + b, (uint32_t)((jj >> 1) & 1));
-    const float4* hi4 = reinterpret_cast<const float4*>(sB + b * 2 * FwdSmem<C>::B_FLOATS);
+    float4* hi4 = reinterpret_cast<float4*>(sB + b * 2 * FwdSmem<C>::B_FLOATS);
     float4* lo4 = reinterpret_cast<float4*>(sB + b * 2 * FwdSmem<C>::B_FLOATS + FwdSmem<C>::B_FLOATS);
     for (int i = threadIdx.x; i < rows * KC / 4; i += RL_NT) {
       const float4 v = hi4[i];
-      lo4[i] = umma::lo4(v);
+      if constexpr (TF32) hi4[i] = umma::rna4(v);
+      else lo4[i] = umma::lo4(v);
     }
   };
   if (threadIdx.x == 0) {
@@ -163,8 +165,12 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
         if (!ok) u = make_float4(0.f, 0.f, 0.f, 0.f);
       }
       const int o = rsub * 4 + qc * 32 + warp * (C / 4) * 32;
-      *reinterpret_cast<float4*>(sA_hi + o) = u;
-      *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(u);
+      if constexpr (TF32) {
+        *reinterpret_cast<float4*>(sA_hi + o) = umma::rna4(u);
+      } else {
+        *reinterpret_cast<float4*>(sA_hi + o) = u;
+        *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(u);
+      }
     }
   }
   umma::tc_fence_before();
@@ -186,7 +192,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
       __syncthreads();
       if (tid == 0) {
         umma::tc_fence_after();
-        tma::mma_chunk_3x<KC>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
+        tma::mma_chunk_3x<KC, TF32>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
         umma::commit(bars + ring.buf());
         // refill this buffer with chunk j + 2 as soon as its MMAs have drained (TS / KC >= 2: chunk j + 2 always
         // exists here)
@@ -254,8 +260,12 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
     for (int i = 0; i < 8; ++i) {
       const int o = obase + (col0 / 4 + i) * 32;
       const float4 g = make_float4(hv[4 * i], hv[4 * i + 1], hv[4 * i + 2], hv[4 * i + 3]);
-      *reinterpret_cast<float4*>(sA_hi + o) = g;
-      *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(g);
+      if constexpr (TF32) {
+        *reinterpret_cast<float4*>(sA_hi + o) = umma::rna4(g);
+      } else {
+        *reinterpret_cast<float4*>(sA_hi + o) = g;
+        *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(g);
+      }
     }
   }
   umma::tc_fence_before();     // the tcgen05.ld reads of the fc1 accumulator precede the barrier below
@@ -274,7 +284,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
       __syncthreads();
       if (tid == 0) {
         umma::tc_fence_after();
-        tma::mma_chunk_3x<KC>(tb + TS, sA_hi, sA_lo, TS, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
+        tma::mma_chunk_3x<KC, TF32>(tb + TS, sA_hi, sA_lo, TS, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
         umma::commit(bars + ring.buf());
         if (j + 2 < TS / KC) {
           ++ring.chunk;
@@ -700,13 +710,13 @@ int launch_cluster(void (*kernel)(const Args), size_t smem, int grid, int cl, co
 
 }  // namespace
 
-template <int C>
+template <int C, bool TF32>
 static int launch_fwd(const rl_ffn_fwd_args* a, int tiles, cudaStream_t st) {
   constexpr int NSL = 4 * C / TS;
   CUtensorMap tm1 = {}, tm2 = {};
   if (int rc = rl_tmap_weight(a->w1, 4 * C, C, C, TS, &tm1)) return rc;           // fc1 [4C][C]: 128-row slices
   if (int rc = rl_tmap_weight(a->w2, C, 4 * C, 4 * C, C, &tm2)) return rc;        // fc2 [C][4C]: all C rows
-  auto kernel = ffn_fwd_umma_kernel<C>;
+  auto kernel = ffn_fwd_umma_kernel<C, TF32>;
   const size_t smem = FwdSmem<C>::BYTES + 64;
   if (int rc = rl_set_smem(kernel, smem)) return rc;
   cudaLaunchConfig_t cfg = {};
@@ -725,15 +735,16 @@ static int launch_fwd(const rl_ffn_fwd_args* a, int tiles, cudaStream_t st) {
   cfg.numAttrs = 2;
   rl_prof_pre(st);
   cudaLaunchKernelEx(&cfg, kernel, *a, tm1, tm2);
-  return rl_check_launch("ffn_fwd_umma", C);
+  return rl_check_launch("ffn_fwd_umma", C, -1, rl_tf32_tag(TF32));
 }
 
 // returns 1 if the shape/mode is not handled here (caller falls through to the per-window kernels in ffn.cu)
 int rl_ffn_fwd_umma(const rl_ffn_fwd_args* a, cudaStream_t st) {
   if (a->L * a->C != 2048 || a->le_mode == RL_LE_DEPTHWISE) return 1;
   const int tiles = (a->B * a->L + TM - 1) / TM;
-  if (a->C == 128) return launch_fwd<128>(a, tiles, st);
-  if (a->C == 64) return launch_fwd<64>(a, tiles, st);
+  const bool tf32 = a->flags & RL_F_TF32;
+  if (a->C == 128) return tf32 ? launch_fwd<128, true>(a, tiles, st) : launch_fwd<128, false>(a, tiles, st);
+  if (a->C == 64) return tf32 ? launch_fwd<64, true>(a, tiles, st) : launch_fwd<64, false>(a, tiles, st);
   return 1;
 }
 

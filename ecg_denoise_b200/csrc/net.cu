@@ -115,7 +115,8 @@ int check_cfg(const rl_net_cfg* cfg, const rl_net_ptrs* P) {
              cfg->L0);
   RL_REQUIRE(!(P->table[0] && cfg->L0 != 256), RL_ERR_SHAPE,
              "net: the R-wave bias tables are defined for 256-sample windows only (model/transformer.py:568-579)");
-  RL_REQUIRE((cfg->flags & ~RL_NET_DETERMINISTIC) == 0, RL_ERR_SHAPE, "net: unknown flags 0x%x", cfg->flags);
+  RL_REQUIRE((cfg->flags & ~(RL_NET_DETERMINISTIC | RL_NET_TF32)) == 0, RL_ERR_SHAPE, "net: unknown flags 0x%x",
+             cfg->flags);
   RL_REQUIRE(cfg->ws && cfg->ws_bytes >= ralenet_net_workspace_bytes_ex(cfg->B, cfg->L0, cfg->save, cfg->flags),
              RL_ERR_NULL, "net: workspace missing or too small (%llu bytes given)", (unsigned long long)cfg->ws_bytes);
   RL_REQUIRE(cfg->running_mean && cfg->running_var && cfg->bn_stats, RL_ERR_NULL, "net: BN buffers missing");
@@ -186,7 +187,10 @@ extern "C" int ralenet_net_fwd_stats(const rl_net_cfg* cfg, const rl_net_ptrs* P
 extern "C" int ralenet_net_fwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, const float* x, float* out, void* stream) {
   if (int rc = check_cfg(cfg, P)) return rc;
   RL_REQUIRE(x && out, RL_ERR_NULL, "net_fwd: x/out is NULL");
+  RL_REQUIRE(!(cfg->flags & RL_NET_TF32) || !cfg->save, RL_ERR_SHAPE,
+             "net_fwd: RL_NET_TF32 is an inference precision (save must be 0: no backward may use a TF32 forward)");
   const int B = cfg->B, L0 = cfg->L0, save = cfg->save;
+  const int32_t blk_flags = RL_F_PRENORM | RL_F_RESIDUAL | ((cfg->flags & RL_NET_TF32) ? RL_F_TF32 : 0);
   const Ws w = carve((float*)cfg->ws, B, L0, save, cfg->flags);
   int rc;
   {
@@ -206,7 +210,7 @@ extern "C" int ralenet_net_fwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
     const bool has_rw = rwi >= 0 && P->table[rwi] != nullptr;
     aa.W = has_rw ? kRwWindow[rwi] : 0;
     aa.c0 = has_rw ? (L - aa.W) / 2 : 0;
-    aa.flags = RL_F_PRENORM | RL_F_RESIDUAL;
+    aa.flags = blk_flags;
     aa.x = cur; aa.pe = cfg->pe[s];
     aa.ln_w = bp[RL_BLK_LN1W]; aa.ln_b = bp[RL_BLK_LN1B];
     aa.wq = bp[RL_BLK_WQ]; aa.bq = bp[RL_BLK_BQ]; aa.wkv = bp[RL_BLK_WKV]; aa.bkv = bp[RL_BLK_BKV];
@@ -219,7 +223,7 @@ extern "C" int ralenet_net_fwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
       aa.y = next_buf();
     }
     rl_ffn_fwd_args fa = {};
-    fa.B = B; fa.L = L; fa.C = C; fa.le_mode = cfg->le_mode; fa.flags = RL_F_PRENORM | RL_F_RESIDUAL;
+    fa.B = B; fa.L = L; fa.C = C; fa.le_mode = cfg->le_mode; fa.flags = blk_flags;
     fa.x = aa.y;
     fa.extra = (i == 9) ? w.pm_out[3] : nullptr;                    // x_mid += x4 (transformer.py:646)
     fa.ln_w = bp[RL_BLK_LN2W]; fa.ln_b = bp[RL_BLK_LN2B];
@@ -264,6 +268,7 @@ extern "C" int ralenet_net_bwd(const rl_net_cfg* cfg, const rl_net_ptrs* P, cons
   if (int rc = check_cfg(cfg, P)) return rc;
   RL_REQUIRE(G && x && dout, RL_ERR_NULL, "net_bwd: NULL argument");
   RL_REQUIRE(cfg->save, RL_ERR_SHAPE, "net_bwd: forward was run without save");
+  RL_REQUIRE(!(cfg->flags & RL_NET_TF32), RL_ERR_SHAPE, "net_bwd: RL_NET_TF32 is an inference precision");
   const int B = cfg->B, L0 = cfg->L0;
   const Ws w = carve((float*)cfg->ws, B, L0, 1, cfg->flags);
   const bool det = cfg->flags & RL_NET_DETERMINISTIC;

@@ -52,7 +52,9 @@ namespace tma {
 // D[tmem] (+)= A[:, k0:k0+KCW] * B^T with the 3-pass tf32 split; A: un-swizzled K-major tile pair (umma.cuh) with KT_A
 // contraction elements per row, B: one KCW <= 32 wide chunk in the K-major SWIZZLE_128B layout written by TMA and its
 // remainder tile in the same layout.  Issued by ONE thread.
-template <int KCW>
+// TF32 (inference precision RL_F_TF32): ONE pass, hi x hi, on operands rounded to tf32 (umma::rna4, derive_lo<NT, true>);
+// the remainder tiles are neither written nor read.
+template <int KCW, bool TF32 = false>
 __device__ __forceinline__ void mma_chunk_3x(uint32_t tmem_d, const float* a_hi, const float* a_lo, int KT_A, int k0,
                                              const float* b_hi, const float* b_lo, uint32_t idesc, uint32_t accum) {
   static_assert(KCW % 8 == 0 && KCW <= 32, "one SWIZZLE_128B atom holds 32 contraction floats");
@@ -63,20 +65,26 @@ __device__ __forceinline__ void mma_chunk_3x(uint32_t tmem_d, const float* a_hi,
   for (int ks = 0; ks < KCW / 8; ++ks) {
     const uint64_t dah = umma::make_desc(ah + ks * 256u, 128u, sbo_a), dal = umma::make_desc(al + ks * 256u, 128u, sbo_a);
     const uint64_t dbh = desc_sw128(bh + ks * 32u), dbl = desc_sw128(bl + ks * 32u);
-    umma::mma_tf32(tmem_d, dal, dbh, idesc, accum);
-    umma::mma_tf32(tmem_d, dah, dbl, idesc, 1u);
-    umma::mma_tf32(tmem_d, dah, dbh, idesc, 1u);
+    if constexpr (TF32) {
+      umma::mma_tf32(tmem_d, dah, dbh, idesc, accum);
+    } else {
+      umma::mma_tf32(tmem_d, dal, dbh, idesc, accum);
+      umma::mma_tf32(tmem_d, dah, dbl, idesc, 1u);
+      umma::mma_tf32(tmem_d, dah, dbh, idesc, 1u);
+    }
     accum = 1u;
   }
 }
-// element-wise remainder tile of a landed chunk (any layout): lo = hi - trunc_tf32(hi); all NT threads of the CTA
-template <int NT>
-__device__ __forceinline__ void derive_lo(const float* hi, float* lo, int floats) {
-  const float4* h4 = reinterpret_cast<const float4*>(hi);
+// element-wise remainder tile of a landed chunk (any layout): lo = hi - trunc_tf32(hi); all NT threads of the CTA.
+// TF32: the chunk is rounded to tf32 in place instead (same pass, same synchronisation point; lo is not touched).
+template <int NT, bool TF32 = false>
+__device__ __forceinline__ void derive_lo(float* hi, float* lo, int floats) {
+  float4* h4 = reinterpret_cast<float4*>(hi);
   float4* l4 = reinterpret_cast<float4*>(lo);
   for (int i = threadIdx.x; i < floats / 4; i += NT) {
     const float4 v = h4[i];
-    l4[i] = umma::lo4(v);
+    if constexpr (TF32) h4[i] = umma::rna4(v);
+    else l4[i] = umma::lo4(v);
   }
 }
 }  // namespace tma

@@ -136,6 +136,15 @@ __device__ __forceinline__ uint32_t tmem_addr(uint32_t base, int col) {
 }
 
 __device__ __forceinline__ float trunc_tf32(float x) { return __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
+// single-pass operand (RL_F_TF32): four values rounded to nearest (ties away) to tf32, stored in the fp32 container
+__device__ __forceinline__ float4 rna4(float4 v) {
+  uint32_t r0, r1, r2, r3;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r0) : "f"(v.x));
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r1) : "f"(v.y));
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r2) : "f"(v.z));
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r3) : "f"(v.w));
+  return make_float4(__uint_as_float(r0), __uint_as_float(r1), __uint_as_float(r2), __uint_as_float(r3));
+}
 // tf32 remainder of four values, v - trunc_tf32(v), with two packed subtractions (Blackwell `sub.f32x2`, SASS FADD2)
 __device__ __forceinline__ float4 lo4(float4 v) {
   const float t0 = trunc_tf32(v.x), t1 = trunc_tf32(v.y), t2 = trunc_tf32(v.z), t3 = trunc_tf32(v.w);

@@ -330,11 +330,23 @@ def _forward_impl(plan: NetPlan, x, save: bool, flags: int = 0):
     return out, lease, training
 
 
+# inference precisions of a forward without an autograd node (_RalenetBase.inference_precision) -> rl_net_cfg.flags
+INFERENCE_PRECISIONS = {"fp32": 0, "tf32": CONSTS["RL_NET_TF32"]}
+
+
+def check_precision(value) -> str:
+    if not isinstance(value, str) or value not in INFERENCE_PRECISIONS:
+        raise ValueError(f"inference precision must be one of {sorted(INFERENCE_PRECISIONS)}, got {value!r}")
+    return value
+
+
 def forward_no_grad(plan: NetPlan, x):
     """ralenet.forward without an autograd node (torch.no_grad() / nothing requires grad): nothing is saved, the
-    workspace is the 7-tensors-per-window ping/pong form (`save = 0` of net.cu::carve)."""
+    workspace is the 7-tensors-per-window ping/pong form (`save = 0` of net.cu::carve).  Runs in the module's
+    inference_precision ("tf32": RL_NET_TF32, single-pass TF32 block GEMMs)."""
     x = _check_input(x)
-    out, lease, _ = _forward_impl(plan, x, save=False)
+    flags = INFERENCE_PRECISIONS[check_precision(plan.net.inference_precision)]
+    out, lease, _ = _forward_impl(plan, x, save=False, flags=flags)
     plan.last_ws_bytes = lease.buf.numel()
     return out
 

@@ -13,6 +13,7 @@ from typing import Optional
 import torch
 
 from . import _lib
+from .engine import check_precision
 from .ops import _chk, _stream
 
 
@@ -57,13 +58,22 @@ def windows_to_records(win: torch.Tensor, x: torch.Tensor, stats: Optional[torch
 
 @torch.no_grad()
 def denoise_records(model, records: torch.Tensor, window: int = 256, stride: int = 256, batch: int = 8192,
-                    znorm: bool = True, stitch: bool = True):
+                    znorm: bool = True, stitch: bool = True, precision: Optional[str] = None):
     """Denoise (R, 2, T) records with an RA-LENet `model` in eval mode.  Returns the stitched records
     (R, 2, T), or the denoised windows (R*nper, 2, window) when stitch=False.  Data-parallel use: give each rank
-    its own slice of the records -- no communication is needed."""
+    its own slice of the records -- no communication is needed.
+    precision: None keeps the inference_precision of every RA-LENet module inside `model`; "fp32" or "tf32" sets it
+    on all of them (e.g. the core of a 12-lead `newrale`) for this call and restores it afterwards."""
+    from .model._blocks import _RalenetBase
+    cores = []
+    if precision is not None:
+        check_precision(precision)
+        cores = [(m, m.inference_precision) for m in model.modules() if isinstance(m, _RalenetBase)]
     was_training = model.training
     model.eval()
     try:
+        for m, _ in cores:
+            m.inference_precision = precision
         win, stats = records_to_windows(records, window, stride, znorm)
         out = torch.empty_like(win)
         for i in range(0, win.shape[0], batch):
@@ -71,3 +81,5 @@ def denoise_records(model, records: torch.Tensor, window: int = 256, stride: int
         return windows_to_records(out, records, stats, stride) if stitch else out
     finally:
         model.train(was_training)
+        for m, p in cores:
+            m.inference_precision = p

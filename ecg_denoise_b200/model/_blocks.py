@@ -17,7 +17,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .. import _lib, ops
-from ..engine import NetPlan, RalenetFn, forward_no_grad
+from ..engine import NetPlan, RalenetFn, check_precision, forward_no_grad
 
 
 def _unsupported(what: str):
@@ -385,6 +385,21 @@ class _RalenetBase(nn.Module):
     def __setstate__(self, state):
         super().__setstate__(state)
         self._init_plan()
+
+    @property
+    def inference_precision(self) -> str:
+        """Precision of the forwards that build no autograd node (under torch.no_grad(), or when neither the input nor
+        any parameter requires grad): "fp32" (default) or "tf32".  "tf32" runs the projection and feed-forward GEMMs of
+        the 18 blocks as ONE tf32 tensor-core pass on operands rounded to nearest, instead of the 3-pass split that keeps
+        them fp32-grade (RL_NET_TF32, include/ralenet_b200.h); the attention core, LayerNorm, GELU, patch layers, stem
+        and head are unchanged.  Outputs stay within 1e-2 * (|ref| + rms(ref)) of the fp64 reference.  A forward that is
+        recorded for a backward always runs fp32.  torch.backends.cuda.matmul.allow_tf32 has no effect here.  Not part
+        of state_dict(); copy.deepcopy and pickling keep it.  Any other value raises ValueError."""
+        return self.__dict__.get("_inference_precision", "fp32")
+
+    @inference_precision.setter
+    def inference_precision(self, value: str) -> None:
+        self.__dict__["_inference_precision"] = check_precision(value)
 
     def forward(self, x):
         if not x.is_cuda:

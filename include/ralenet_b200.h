@@ -47,8 +47,12 @@ enum { RL_LE_NONE = 0, RL_LE_PARTIAL = 1, RL_LE_DEPTHWISE = 2 };
 /* flags of the attention / feed-forward halves */
 enum {
   RL_F_PRENORM = 1,   /* apply (x*sqrt(C) + PE, LayerNorm) resp. LayerNorm in front (TransformerBlock) */
-  RL_F_RESIDUAL = 2   /* add the block input to the result (TransformerBlock)                          */
+  RL_F_RESIDUAL = 2,  /* add the block input to the result (TransformerBlock)                          */
+  RL_F_TF32 = 4       /* forward only: single-pass TF32 projection / feed-forward GEMMs (RL_NET_TF32)  */
 };
+/* RL_F_TF32 is an inference precision: ralenet_attn_fwd / ralenet_ffn_fwd / ralenet_block_fwd reject it together with
+ * saved-tensor pointers (q, k, v, o, lse, h) with RL_ERR_SHAPE, ralenet_block_fwd rejects halves whose RL_F_TF32 bits
+ * differ, and ralenet_attn_bwd / ralenet_ffn_bwd reject the bit. */
 
 int ralenet_abi_version(void);
 const char* ralenet_last_error(void);
@@ -339,7 +343,16 @@ typedef struct {
  * whatever the scheduling of CTAs and streams: every cross-CTA accumulation into a parameter gradient is a plain store
  * into its own slot of a partial slab in the workspace, and a reduction kernel adds the slots in slot order with one
  * read-modify-write per gradient element.  The forward pass is deterministic in either mode. */
-enum { RL_NET_DETERMINISTIC = 1 };
+/* RL_NET_TF32: inference precision of ralenet_net_fwd with save == 0 (RL_ERR_SHAPE with save != 0: no backward may
+ * consume such a forward).  The q|k|v, output-projection, fc1 and fc2 GEMMs of every block run ONE tf32 tensor-core pass
+ * on operands rounded to nearest (ties away) to a 10-bit mantissa, instead of the 3-pass split that keeps the default
+ * fp32-grade.  The attention core (softmax logits), LayerNorm, GELU, positional encoding, R-wave bias, patch layers,
+ * stem and head are computed exactly as in the default mode.  Precision contract: the output is held to the reduced-
+ * precision gate |out - ref| <= 1e-2 * (|ref| + rms(ref)) against the fp64 reference, and per-window SNR / RMSE within
+ * 0.01 dB of the default mode.  Deterministic (bit-identical from run to run) like the default forward; combining it
+ * with RL_NET_DETERMINISTIC is legal (that bit has no effect on a forward without save).  The workspace size does not
+ * depend on it. */
+enum { RL_NET_DETERMINISTIC = 1, RL_NET_TF32 = 2 };
 
 uint64_t ralenet_net_workspace_bytes(int32_t B, int32_t L0, int32_t save);      /* == _ex(B, L0, save, 0) */
 /* the deterministic mode needs the partial slabs on top (a function of B and L0 only) */
