@@ -80,6 +80,14 @@ __device__ __forceinline__ void prefetch_l2_block(const void* p, int bytes) {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
+// SplitMix64 finaliser: the counter-based hash behind the device-side batch sources (synth.cu, records.cu)
+__device__ __forceinline__ uint64_t mix64(uint64_t z) {
+  z += 0x9e3779b97f4a7c15ull;
+  z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+  z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+  return z ^ (z >> 31);
+}
+
 template <typename K>
 static inline int rl_set_smem(K kernel, size_t bytes) {
   cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);

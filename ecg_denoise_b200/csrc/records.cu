@@ -5,6 +5,8 @@
 // stitches them back.  Here: per-(record, lead) statistics, a fused z-norm + window gather, and a
 // deterministic overlap-add stitch (gather form, no atomics) that also undoes the normalisation.
 // All three are HBM-bound streaming kernels.
+// For training (SURVEY.md 8f-3), record_sample_kernel draws the same z-normalised windows from a record bank in a
+// keyed per-epoch order and pairs each with a window of a noise bank and an SNR level; ralenet_snr_mix does the mix.
 #include "common.cuh"
 
 namespace {
@@ -92,6 +94,69 @@ __global__ void __launch_bounds__(RL_NT) window_scatter_kernel(const float* __re
   }
 }
 
+// ---- training-window sampler: the reference's data recipe (cut, np_norm, noise at a target SNR) drawn on the device
+constexpr int FEISTEL_ROUNDS = 4;
+
+// keyed bijection of [0, n): a balanced Feistel network on the smallest even bit width 2h >= 2 with 2^(2h) >= n,
+// walked until the value falls back into [0, n) (the walk ends because x itself lies on a cycle that enters [0, n))
+__device__ __forceinline__ uint64_t feistel_perm(uint64_t x, uint64_t n, uint64_t key) {
+  int h = 1;
+  while ((1ull << (2 * h)) < n) ++h;
+  const uint64_t m = (1ull << h) - 1;
+  do {
+    uint64_t l = x >> h, r = x & m;
+#pragma unroll
+    for (int k = 0; k < FEISTEL_ROUNDS; ++k) {
+      const uint64_t t = l ^ (mix64(r ^ mix64(key + k)) & m);
+      l = r;
+      r = t;
+    }
+    x = (l << h) | r;
+  } while (x >= n);
+  return x;
+}
+
+// one CTA per window; the plan (which record window, which noise window, which SNR level) is computed by every thread
+__global__ void __launch_bounds__(RL_NT) record_sample_kernel(rl_sample_args a, int nper, uint64_t n, uint64_t spe) {
+  pdl_wait();                                     // *counter may be the Adam step counter the previous kernel bumped
+  pdl_trigger();
+  const int i = blockIdx.x, tid = threadIdx.x, W = a.W;
+  const uint64_t ctr = a.counter ? (uint64_t)(uint32_t)(*a.counter) : 0ull;
+  const uint64_t slot = (uint64_t)a.rank * a.B + i;                        // slot within the world batch
+  const uint64_t g = (ctr % spe) * (uint64_t)a.world * a.B + slot;         // position in this epoch's order
+  const uint64_t item = feistel_perm(g, n, mix64(a.seed ^ mix64(2 * (ctr / spe))));
+  const int64_t rec = (int64_t)(item / nper), off = (int64_t)(item % nper) * a.stride;
+  const uint64_t hw = mix64(mix64(a.seed ^ mix64(2 * ctr + 1)) ^ slot);
+  const int64_t nrec = (int64_t)(mix64(hw + 1) % (uint64_t)a.N);
+  const int64_t noff = (int64_t)(mix64(hw + 2) % (uint64_t)(a.Tn - W + 1));
+  const int lvl = (int)(mix64(hw + 3) % (uint64_t)a.n_snr);
+  if (tid == 0) {
+    a.snr_out[i] = __ldg(a.snr_levels + lvl);
+    if (a.meta) {
+      a.meta[4 * i] = (int32_t)rec;
+      a.meta[4 * i + 1] = (int32_t)off;
+      a.meta[4 * i + 2] = (int32_t)nrec;
+      a.meta[4 * i + 3] = (int32_t)noff;
+    }
+  }
+  for (int l = 0; l < a.leads; ++l) {
+    const size_t rc = (size_t)rec * a.leads + l;
+    const float* xs = a.records + rc * a.T + off;
+    const float* ns = a.noise + ((size_t)nrec * a.noise_leads + l % a.noise_leads) * a.Tn + noff;
+    float mean = 0.f, rstd = 1.f;
+    if (a.stats) { mean = __ldg(a.stats + 2 * rc); rstd = __ldg(a.stats + 2 * rc + 1); }
+    float* cw = a.clean_out + ((size_t)i * a.leads + l) * W;
+    float* nw = a.noise_out + ((size_t)i * a.leads + l) * W;
+    for (int t = tid; t < W; t += RL_NT) {
+      float v = __ldg(xs + t);
+      const float nz = __ldg(ns + t);
+      if (a.stats) v = (v - mean) * rstd;          // the arithmetic of window_gather_kernel
+      cw[t] = v;
+      nw[t] = nz;
+    }
+  }
+}
+
 }  // namespace
 
 extern "C" int ralenet_record_stats(const float* x, int32_t RC, int64_t T, float* stats, void* stream) {
@@ -135,4 +200,27 @@ extern "C" int ralenet_window_scatter(const float* win, const float* x, const fl
   window_scatter_kernel<<<blocks < 1 ? 1 : blocks, RL_NT, 0, (cudaStream_t)stream>>>(win, x, stats, y, C, T, W, stride,
                                                                                      nper, total);
   return rl_check_launch("window_scatter_kernel");
+}
+
+extern "C" int ralenet_record_sample(const rl_sample_args* a, void* stream) {
+  RL_REQUIRE(a, RL_ERR_NULL, "record_sample: args is NULL");
+  RL_REQUIRE(a->records && a->noise && a->snr_levels && a->clean_out && a->noise_out && a->snr_out, RL_ERR_NULL,
+             "record_sample: NULL tensor");
+  RL_REQUIRE(a->R > 0 && a->leads > 0 && a->leads <= 12 && a->N > 0 && a->B > 0 && a->W > 0 && a->stride > 0 &&
+                 a->n_snr >= 1 && a->W <= a->T && a->W <= a->Tn,
+             RL_ERR_SHAPE, "record_sample: unsupported R=%d leads=%d T=%lld N=%d Tn=%lld W=%d stride=%d B=%d n_snr=%d",
+             a->R, a->leads, (long long)a->T, a->N, (long long)a->Tn, a->W, a->stride, a->B, a->n_snr);
+  RL_REQUIRE(a->noise_leads == 1 || a->noise_leads == a->leads, RL_ERR_SHAPE,
+             "record_sample: noise_leads=%d must be 1 or leads=%d", a->noise_leads, a->leads);
+  RL_REQUIRE(a->world > 0 && a->rank >= 0 && a->rank < a->world, RL_ERR_SHAPE, "record_sample: rank=%d world=%d",
+             a->rank, a->world);
+  RL_REQUIRE(!a->meta || (a->T <= INT32_MAX && a->Tn <= INT32_MAX), RL_ERR_SHAPE,
+             "record_sample: meta holds int32 offsets; T=%lld Tn=%lld", (long long)a->T, (long long)a->Tn);
+  const int64_t nper = (a->T - a->W) / a->stride + 1;
+  RL_REQUIRE(nper <= INT32_MAX, RL_ERR_SHAPE, "record_sample: %lld windows per record", (long long)nper);
+  const uint64_t n = (uint64_t)a->R * (uint64_t)nper, spe = n / ((uint64_t)a->world * (uint64_t)a->B);
+  RL_REQUIRE(spe > 0, RL_ERR_SHAPE, "record_sample: %llu grid windows are fewer than world*B=%lld",
+             (unsigned long long)n, (long long)a->world * a->B);
+  rl_launch_pdl(record_sample_kernel, dim3(a->B), dim3(RL_NT), 0, (cudaStream_t)stream, *a, (int)nper, n, spe);
+  return rl_check_launch("record_sample_kernel");
 }

@@ -20,12 +20,6 @@ namespace {
 
 constexpr float FS = 360.f, TWO_PI = 6.283185307179586f;
 
-__device__ __forceinline__ uint64_t mix64(uint64_t z) {
-  z += 0x9e3779b97f4a7c15ull;
-  z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
-  z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
-  return z ^ (z >> 31);
-}
 struct Rng {
   uint64_t base;
   __device__ __forceinline__ float u01(uint32_t stream, uint32_t idx) const {        // (0, 1)

@@ -727,9 +727,10 @@ class FusedTrainer(_HostPipeline):
             self.graph = None             # the captured step changes
 
     def step_synth(self, synth):
-        """one training step on a batch drawn ON THE DEVICE by `synth` (synth_device.DeviceSynth): no host traffic at
-        all; with use_graph the generator is part of the step's CUDA graph and every replay sees new windows.
-        Returns (loss[1], rmse[B], snr[B], out) like step()."""
+        """one training step on a batch drawn ON THE DEVICE by `synth` (synth_device.DeviceSynth for synthetic windows,
+        record_sampler.RecordSampler for windows of real record banks; anything with B, leads, L, device and
+        fill(noisy, clean, counter)): no host traffic at all; with use_graph the generator is part of the step's CUDA
+        graph and every replay sees new windows.  Returns (loss[1], rmse[B], snr[B], out) like step()."""
         self._prepare((synth.B, synth.leads, synth.L), synth.device)
         self._set_synth(synth)
         sx, st_ = self._static
@@ -768,6 +769,7 @@ class FineTuneTrainer(_HostPipeline):
         self.flat = None
         self.graph = None
         self._shape = None
+        self._source = None           # device batch source feeding the step (step_synth)
 
     def _setup(self, device):
         plan: NetPlan = self.core._plan
@@ -829,6 +831,8 @@ class FineTuneTrainer(_HostPipeline):
         st = ctypes.c_void_p(_stream())
         cfg = plan.cfg(B, L, training, True, self._ws)
         a2p, rp = ctypes.c_void_p(self._a2.data_ptr()), ctypes.c_void_p(self._r.data_ptr())
+        if self._source is not None:      # draw this step's batch on the device (batch index = Adam step counter)
+            self._source.fill(self._x, self._t, self.step_dev)
         self.flat_grad.zero_()
         self._conv_fwd(self._x, c1, self._a1, True)
         self._conv_fwd(self._a1, c2, self._a2, True)
@@ -851,7 +855,10 @@ class FineTuneTrainer(_HostPipeline):
         self._keep = dout
         return self._res
 
-    def _run(self):
+    def _run(self, source=None):
+        if source is not self._source:
+            self._source = source
+            self.graph = None             # the captured step changes
         _lib.deterministic_guard("FineTuneTrainer (lead-mixing convolution weight gradients)")
         if not self.use_graph:
             return self._step_impl()
@@ -881,6 +888,17 @@ class FineTuneTrainer(_HostPipeline):
         self._x.copy_(x, non_blocking=True)
         self._t.copy_(target, non_blocking=True)
         return self._run()
+
+    def step_synth(self, source):
+        """one fine-tuning step on a batch drawn ON THE DEVICE by `source` (e.g. record_sampler.RecordSampler on a
+        12-lead bank; anything with B, leads, L, device and fill(noisy, clean, counter)), the counterpart of
+        FusedTrainer.step_synth: the batch index is the Adam step counter, and with use_graph the draw is part of the
+        step's CUDA graph.  Returns (loss[1], rmse[B], snr[B], out) like step()."""
+        cin = self.convs[0].weight.shape[1]
+        if source.leads != cin:
+            raise ValueError(f"FineTuneTrainer.step_synth: the source draws {source.leads} leads, the model takes {cin}")
+        self._prepare((source.B, source.leads, source.L), source.device)
+        return self._run(source)
 
     def _host_static(self, shape):
         self._prepare(shape, self.convs[0].weight.device)

@@ -419,6 +419,29 @@ int ralenet_snr_mix(const float* data, const float* noise, const float* snr_db, 
 int ralenet_synth_windows(float* clean, float* noise, int32_t B, int32_t leads, int32_t L, uint64_t seed,
                           const int32_t* counter_dev, int32_t kind, void* stream);
 
+/* Device-side record sampler (records.cu; SURVEY.md section 8 f3 on real data): training windows cut from a bank of
+ * clean records and paired with windows of a bank of noise records, one CTA per window; mix with ralenet_snr_mix.
+ *   records [R][leads][T] (leads <= 12), stats [R*leads][2] from ralenet_record_stats or NULL (no z-normalisation),
+ *   noise [N][noise_leads][Tn] (noise_leads = 1 or leads; clean lead l reads noise lead l % noise_leads),
+ *   snr_levels [n_snr] dB.  Outputs clean_out / noise_out [B][leads][W] (clean_out z-normalised exactly like
+ *   ralenet_window_gather), snr_out [B] dB, meta [B][4] = (record, offset, noise record, noise offset) or NULL.
+ * The grid of a bank is item = record * nper + k, offset k * stride, nper = (T - W)/stride + 1, n = R * nper items;
+ * spe = n / (world * B) steps per epoch (drop-last).  With c = *counter (0 when NULL), rank r, slot i takes item
+ * perm_e((c % spe) * world * B + r * B + i) of epoch e = c / spe, perm_e a keyed bijection of [0, n) (4-round Feistel
+ * network with cycle walking).  Noise record, noise offset (uniform in [0, Tn - W]) and SNR level are hashed from
+ * (seed, c, r * B + i).  Every draw is a pure function of (seed, c, global slot), so the slices of `world` ranks
+ * concatenate to the batch of world * B windows that one rank would draw.  meta needs T, Tn <= INT32_MAX. */
+typedef struct {
+  const float* records; const float* stats; const float* noise; const float* snr_levels;
+  const int32_t* counter;
+  float* clean_out; float* noise_out; float* snr_out;
+  int32_t* meta;
+  int64_t T, Tn;
+  uint64_t seed;
+  int32_t R, leads, N, noise_leads, n_snr, W, stride, B, rank, world;
+} rl_sample_args;
+int ralenet_record_sample(const rl_sample_args* a, void* stream);
+
 /* Weight-gradient GEMM over the token dimension (used by every *_bwd above; exported for benchmarks):
  *   dW[n*K + k] += sum_m dY[m*ldy + n] * X[m*ldx + k],   db[n] += sum_m dY[m*ldy + n]   (db may be NULL) */
 int ralenet_wgrad(const float* dY, int32_t ldy, const float* X, int32_t ldx, int32_t M, int32_t N, int32_t K,
