@@ -16,7 +16,8 @@
 //   4. partial projection  yp = o_r Wp[:, 32 r : 32 r + 32]^T    UMMA M = 128, N = C, K = 32 -> TMEM columns [96, 96 + C)
 //   5. the NSL partial tiles are reduced through distributed shared memory; + bias + residual -> y
 // so a CTA reads 96 C + 32 C weights for 128 tokens instead of 4 C^2 per window (32x less L2 -> SM traffic at C = 128).
-// Operand staging, the 3-pass tf32 split and completion tracking are those of ffn_umma.cu (umma.cuh).
+// Operand staging, the 3-pass tf32 split, the TMA chunk loop and the cluster reduction are shared with ffn_umma.cu
+// (umma.cuh, tma.cuh).
 #define RL_NT 512
 #define RL_MINB 1
 #include "common.cuh"
@@ -142,65 +143,12 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
   RL_TS(attn_umma, 2);
 
   // 1. x*sqrt(C) + P -> LayerNorm -> A tile (K-major, KT = C) with its tf32 remainder     (transformer.py:386-387)
-  //    A warp owns 8 rows; lane = (row % 8, 16-byte chunk % 4): full sectors from global, contiguous tile stores.
   {
-    constexpr int NI = C / 16;                                // chunks per lane
-    const int rsub = lane & 7, qsub = lane >> 3;
-    const int row = warp * 8 + rsub;
-    const bool ok = row < nvalid;
-    const bool pre = a.flags & RL_F_PRENORM;
     const float sc = sqrtf((float)C);
-    float4 v[NI];
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < NI; ++i) {
-      const int qc = qsub + 4 * i;
-      v[i] = ok ? __ldg(reinterpret_cast<const float4*>(xw + (size_t)row * C) + qc) : make_float4(0.f, 0.f, 0.f, 0.f);
-      if (pre) {
-        const float4 p4 = *reinterpret_cast<const float4*>(s_pe + (row % L) * ASmem<C>::LDPE + 4 * qc);
-        v[i].x = fmaf(v[i].x, sc, p4.x); v[i].y = fmaf(v[i].y, sc, p4.y);
-        v[i].z = fmaf(v[i].z, sc, p4.z); v[i].w = fmaf(v[i].w, sc, p4.w);
-      }
-      s += v[i].x + v[i].y + v[i].z + v[i].w;
-    }
-    RL_TS(attn_umma, 13);                                     // (trace) the x loads have landed
-    float mu = 0.f, rstd = 1.f;
-    if (pre) {
-      s += __shfl_xor_sync(0xffffffffu, s, 8);
-      s += __shfl_xor_sync(0xffffffffu, s, 16);
-      mu = s * (1.0f / C);
-      float q = 0.f;
-#pragma unroll
-      for (int i = 0; i < NI; ++i) {
-        const float d0 = v[i].x - mu, d1 = v[i].y - mu, d2 = v[i].z - mu, d3 = v[i].w - mu;
-        q += d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3;
-      }
-      q += __shfl_xor_sync(0xffffffffu, q, 8);
-      q += __shfl_xor_sync(0xffffffffu, q, 16);
-      rstd = rsqrtf(q * (1.0f / C) + RL_LN_EPS);
-    }
-    RL_TS(attn_umma, 14);                                     // (trace) statistics done
-#pragma unroll
-    for (int i = 0; i < NI; ++i) {
-      const int qc = qsub + 4 * i;
-      float4 u = v[i];
-      if (pre) {
-        const float4 w4 = *reinterpret_cast<const float4*>(s_ln + 4 * qc);
-        const float4 b4 = *reinterpret_cast<const float4*>(s_ln + C + 4 * qc);
-        u.x = fmaf((v[i].x - mu) * rstd, w4.x, b4.x);
-        u.y = fmaf((v[i].y - mu) * rstd, w4.y, b4.y);
-        u.z = fmaf((v[i].z - mu) * rstd, w4.z, b4.z);
-        u.w = fmaf((v[i].w - mu) * rstd, w4.w, b4.w);
-      }
-      if (!ok) u = make_float4(0.f, 0.f, 0.f, 0.f);
-      const int o = rsub * 4 + qc * 32 + warp * (C / 4) * 32;
-      if constexpr (TF32) {
-        *reinterpret_cast<float4*>(sA_hi + o) = umma::rna4(u);
-      } else {
-        *reinterpret_cast<float4*>(sA_hi + o) = u;
-        *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(u);
-      }
-    }
+    umma::stage_rows<C, TF32>(sA_hi, sA_lo, xw, nvalid, a.flags & RL_F_PRENORM, s_ln, [&](float4 v, int row, int qc) {
+      const float4 p4 = *reinterpret_cast<const float4*>(s_pe + (row % L) * ASmem<C>::LDPE + 4 * qc);
+      return make_float4(fmaf(v.x, sc, p4.x), fmaf(v.y, sc, p4.y), fmaf(v.z, sc, p4.z), fmaf(v.w, sc, p4.w));
+    });
   }
   umma::tc_fence_before();
   __syncthreads();
@@ -210,30 +158,8 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
   RL_TS(attn_umma, 3);
 
   // 2. [q | k | v] slice = u [Wq_r ; Wk_r ; Wv_r]^T   (M = TM, N = NQ, K = C) -> TMEM columns [0, NQ)
-  {
-    constexpr uint32_t idesc = umma::idesc_tf32(TM, NQ);
-#pragma unroll
-    for (int j = 0; j < NCHK; ++j) {
-      float* bh = sB + ring.buf() * 2 * NQ * KC;
-      float* bl = bh + NQ * KC;
-      umma::mbar_wait(bars + 2 + (j & 1), (uint32_t)((j >> 1) & 1));
-      tma::derive_lo<RL_NT, TF32>(bh, bl, NQ * KC);
-      umma::fence_async_smem();
-      __syncthreads();
-      if (tid == 0) {
-        umma::tc_fence_after();
-        tma::mma_chunk_3x<KC, TF32>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
-        umma::commit(bars + ring.buf());
-        if (j + 2 < NCHK) {              // refill this buffer once its MMAs have drained
-          ++ring.chunk;
-          ring.wait_last();
-          --ring.chunk;
-          tma_issue_qkv(j + 2);
-        }
-      }
-      ++ring.chunk;
-    }
-  }
+  tma::mma_chunks<NCHK, KC, RL_NT, TF32>(ring, bars + 2, sB, NQ * KC, NQ * KC, tb, sA_hi, sA_lo, C,
+                                         umma::idesc_tf32(TM, NQ), NCHK - 1, tma_issue_qkv);
   // the bias values of epilogue 1 go to registers now; their latency hides behind the MMAs (warp group w / 4 = 0, 1, 2
   // takes q, k, v)
   float4 bias4[CS / 4];
@@ -328,13 +254,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
       const int qc = qsub + 4 * i;
       const float4 o4 = *reinterpret_cast<const float4*>(sq + row * LDS + 4 * qc);
       if (a.o && row < nvalid) *reinterpret_cast<float4*>(a.o + (tok0 + row) * C + CS * r + 4 * qc) = o4;
-      const int o = rsub * 4 + qc * 32 + warp * (CS / 4) * 32;
-      if constexpr (TF32) {
-        *reinterpret_cast<float4*>(sO_hi + o) = umma::rna4(o4);
-      } else {
-        *reinterpret_cast<float4*>(sO_hi + o) = o4;
-        *reinterpret_cast<float4*>(sO_lo + o) = umma::lo4(o4);
-      }
+      umma::store_pair<TF32>(sO_hi, sO_lo, umma::kmajor_off(warp, rsub, qc, CS), o4);
     }
     umma::mbar_wait(bars + 4, 0u);
     tma::derive_lo<RL_NT, TF32>(sW_hi, sW_lo, C * CS);
@@ -354,59 +274,15 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) attn_fwd_umma_kernel(const rl_
 
   // 5. epilogue 2: partial tile -> shared memory [TM][C + 4] (over the dead q / k / v slices), DSMEM reduction:
   //    CTA r finishes rows [r * TM / NSL, (r + 1) * TM / NSL)        y = x + o Wp^T + bp  (transformer.py:320, :405)
-  constexpr int LDP = C + 4;
   float* sp = r0;
-  {
-    const int quad = warp & 3, cgp = warp >> 2;
-    const int row = quad * 32 + lane;
-    constexpr int CW = C / 4;                                 // columns per warp group (16 or 32)
-#pragma unroll
-    for (int c16 = 0; c16 < CW; c16 += 16) {
-      float t0[16];
-      umma::tmem_ld16(umma::tmem_addr(tb, NQ + cgp * CW + c16), t0);
-#pragma unroll
-      for (int i = 0; i < 16; i += 4)
-        *reinterpret_cast<float4*>(sp + row * LDP + cgp * CW + c16 + i) = make_float4(t0[i], t0[i + 1], t0[i + 2], t0[i + 3]);
-    }
-  }
+  umma::tmem_to_smem<C>(sp, tb, NQ);
   umma::tc_fence_before();
-  // rows [r RPC, (r + 1) RPC) are finished here: their bias + residual terms are fetched before the cluster barrier
-  constexpr int RPC = TM / NSL, RIT = RPC * (C / 4) / RL_NT;  // rows finished by this CTA, float4 items per thread
-  static_assert(RPC * (C / 4) % RL_NT == 0, "reduce: items must tile the CTA");
-  float4 add4[RIT];
-#pragma unroll
-  for (int it = 0; it < RIT; ++it) {
-    const int i = tid + it * RL_NT;
-    const int rr = r * RPC + i / (C / 4), c = (i % (C / 4)) * 4;
-    add4[it] = a.bp ? __ldg(reinterpret_cast<const float4*>(a.bp + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
-    if ((a.flags & RL_F_RESIDUAL) && rr < nvalid) {
-      const float4 x4 = __ldg(reinterpret_cast<const float4*>(a.x + (tok0 + rr) * C + c));
-      add4[it].x += x4.x; add4[it].y += x4.y; add4[it].z += x4.z; add4[it].w += x4.w;
-    }
-  }
+  umma::ClusterReduce<TM, C, NSL> red;
+  red.load(r, nvalid, tok0, a.bp, a.x, a.flags & RL_F_RESIDUAL, nullptr);
   RL_TS(attn_umma, 9);
   cluster.sync();
   RL_TS(attn_umma, 10);
-  {
-    const float* part[NSL];
-#pragma unroll
-    for (int q = 0; q < NSL; ++q) part[q] = cluster.map_shared_rank(sp, q);
-#pragma unroll
-    for (int it = 0; it < RIT; ++it) {
-      const int i = tid + it * RL_NT;
-      const int rr = r * RPC + i / (C / 4), c = (i % (C / 4)) * 4;
-      if (rr >= nvalid) continue;
-      const int off = rr * LDP + c;
-      float4 s = *reinterpret_cast<const float4*>(part[0] + off);
-#pragma unroll
-      for (int q = 1; q < NSL; ++q) {
-        const float4 p = *reinterpret_cast<const float4*>(part[q] + off);
-        s.x += p.x; s.y += p.y; s.z += p.z; s.w += p.w;
-      }
-      s.x += add4[it].x; s.y += add4[it].y; s.z += add4[it].z; s.w += add4[it].w;
-      *reinterpret_cast<float4*>(a.y + (tok0 + rr) * C + c) = s;
-    }
-  }
+  red.store(cluster, sp, r, nvalid, tok0, a.y);
   RL_TS(attn_umma, 11);
   cluster.sync();     // nobody may exit while its partial tile is still being read
   if (warp == 0) umma::tmem_dealloc<TMEM_COLS>(tb);
@@ -423,22 +299,7 @@ int launch(const rl_attn_fwd_args& a, cudaStream_t st) {
   if (int rc = rl_tmap_weight(a.wp, C, C, C, C, &tmp)) return rc;             // proj  [C][C]:  all C rows, 32 columns
   auto kernel = attn_fwd_umma_kernel<C, TF32>;
   if (int rc = rl_set_smem(kernel, ASmem<C>::BYTES)) return rc;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(tiles * NSL);
-  cfg.blockDim = dim3(RL_NT);
-  cfg.dynamicSmemBytes = ASmem<C>::BYTES;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = NSL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  rl_prof_pre(st);
-  cudaLaunchKernelEx(&cfg, kernel, a, tmq, tmkv, tmp);
+  rl_launch_pdl_cluster(NSL, kernel, dim3(tiles * NSL), dim3(RL_NT), ASmem<C>::BYTES, st, a, tmq, tmkv, tmp);
   return rl_check_launch("attn_fwd_umma", C, -1, rl_tf32_tag(TF32));
 }
 

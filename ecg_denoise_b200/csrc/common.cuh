@@ -49,21 +49,36 @@ void rl_prof_pre(cudaStream_t st);     // profiling: event right before the next
 
 // Programmatic dependent launch: the kernel may be scheduled while the previous kernel on the stream drains;
 // it must call pdl_wait() before touching global memory.  Captured into CUDA graphs as programmatic edges.
+// cluster > 0: consecutive groups of `cluster` CTAs along x form a thread-block cluster (distributed shared memory).
 template <typename... KArgs, typename... Args>
-static inline void rl_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                 Args... args) {
+static inline void rl_launch_pdl_cluster(int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
+                                         cudaStream_t st, Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute attr[2];
+  int n = 0;
+  if (cluster > 0) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = cluster;
+    attr[n].val.clusterDim.y = 1;
+    attr[n].val.clusterDim.z = 1;
+    ++n;
+  }
+  attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[n].val.programmaticStreamSerializationAllowed = 1;
+  ++n;
   cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  cfg.numAttrs = n;
   rl_prof_pre(st);
   cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);      // errors surface through rl_check_launch()
+}
+template <typename... KArgs, typename... Args>
+static inline void rl_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                 Args... args) {
+  rl_launch_pdl_cluster(0, kernel, grid, block, smem, st, args...);
 }
 // L2 prefetch of tensors that were saved by the forward pass (they sit in HBM by the time the backward reads them):
 // issued before griddepcontrol.wait, the HBM latency passes behind the tail of the preceding kernel and the loads of

@@ -73,18 +73,6 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
       tma::load_2d(dst, &tm2, r_early * TS + (jj - NCH1) * KC, 0, bars + 2 + b);
     }
   };
-  // all threads: wait for chunk jj, derive its remainder tile (same swizzled layout, element-wise; TF32: round in place)
-  auto tma_consume = [&](int jj, int rows) {
-    const int b = jj & 1;
-    umma::mbar_wait(bars + 2 + b, (uint32_t)((jj >> 1) & 1));
-    float4* hi4 = reinterpret_cast<float4*>(sB + b * 2 * FwdSmem<C>::B_FLOATS);
-    float4* lo4 = reinterpret_cast<float4*>(sB + b * 2 * FwdSmem<C>::B_FLOATS + FwdSmem<C>::B_FLOATS);
-    for (int i = threadIdx.x; i < rows * KC / 4; i += RL_NT) {
-      const float4 v = hi4[i];
-      if constexpr (TF32) hi4[i] = umma::rna4(v);
-      else lo4[i] = umma::lo4(v);
-    }
-  };
   if (threadIdx.x == 0) {
     umma::mbar_init(bars, 1);
     umma::mbar_init(bars + 1, 1);
@@ -121,58 +109,8 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
   __syncthreads();                                           // staged LayerNorm affine visible to every warp
   RL_TS(umma, 2);
 
-  // 1. LN2 over the TM tokens -> A tile (K-major, KT = C) with its tf32 remainder.  A warp owns 8 rows; lane =
-  //    (row % 8, 16-byte chunk % 4), so global reads cover full sectors and the tile stores are contiguous.
-  {
-    constexpr int NI = C / 16;                                // chunks per lane
-    const int rsub = lane & 7, qsub = lane >> 3;
-    const int row = warp * 8 + rsub;
-    const bool ok = row < nvalid;
-    float4 v[NI];
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < NI; ++i) {
-      v[i] = ok ? __ldg(reinterpret_cast<const float4*>(xw + (size_t)row * C) + qsub + 4 * i)
-                : make_float4(0.f, 0.f, 0.f, 0.f);
-      s += v[i].x + v[i].y + v[i].z + v[i].w;
-    }
-    float mu = 0.f, rstd = 1.f;
-    if (a.flags & RL_F_PRENORM) {
-      s += __shfl_xor_sync(0xffffffffu, s, 8);
-      s += __shfl_xor_sync(0xffffffffu, s, 16);
-      mu = s * (1.0f / C);
-      float q = 0.f;
-#pragma unroll
-      for (int i = 0; i < NI; ++i) {
-        const float d0 = v[i].x - mu, d1 = v[i].y - mu, d2 = v[i].z - mu, d3 = v[i].w - mu;
-        q += d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3;
-      }
-      q += __shfl_xor_sync(0xffffffffu, q, 8);
-      q += __shfl_xor_sync(0xffffffffu, q, 16);
-      rstd = rsqrtf(q * (1.0f / C) + RL_LN_EPS);
-    }
-#pragma unroll
-    for (int i = 0; i < NI; ++i) {
-      const int qc = qsub + 4 * i;
-      float4 u = v[i];
-      if (a.flags & RL_F_PRENORM) {
-        const float4 w4 = *reinterpret_cast<const float4*>(s_ln + 4 * qc);
-        const float4 b4 = *reinterpret_cast<const float4*>(s_ln + C + 4 * qc);
-        u.x = fmaf((v[i].x - mu) * rstd, w4.x, b4.x);
-        u.y = fmaf((v[i].y - mu) * rstd, w4.y, b4.y);
-        u.z = fmaf((v[i].z - mu) * rstd, w4.z, b4.z);
-        u.w = fmaf((v[i].w - mu) * rstd, w4.w, b4.w);
-        if (!ok) u = make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-      const int o = rsub * 4 + qc * 32 + warp * (C / 4) * 32;
-      if constexpr (TF32) {
-        *reinterpret_cast<float4*>(sA_hi + o) = umma::rna4(u);
-      } else {
-        *reinterpret_cast<float4*>(sA_hi + o) = u;
-        *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(u);
-      }
-    }
-  }
+  // 1. LN2 over the TM tokens -> A tile (K-major, KT = C) with its tf32 remainder
+  umma::stage_rows<C, TF32>(sA_hi, sA_lo, xw, nvalid, a.flags & RL_F_PRENORM, s_ln, [](float4 v, int, int) { return v; });
   umma::tc_fence_before();
   __syncthreads();
   umma::tc_fence_after();
@@ -181,29 +119,9 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
   RL_TS(umma, 3);
 
   // 2. hidden slice: h = u W1[128 r : 128 r + 128]^T   (M = TM, N = TS, K = C) -> TMEM columns [0, TS)
-  {
-    constexpr uint32_t idesc = umma::idesc_tf32(TM, TS);
-#pragma unroll
-    for (int j = 0; j < C / KC; ++j) {
-      float* bh = sB + ring.buf() * 2 * FwdSmem<C>::B_FLOATS;
-      float* bl = bh + FwdSmem<C>::B_FLOATS;
-      tma_consume(j, TS);
-      umma::fence_async_smem();
-      __syncthreads();
-      if (tid == 0) {
-        umma::tc_fence_after();
-        tma::mma_chunk_3x<KC, TF32>(tb, sA_hi, sA_lo, C, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
-        umma::commit(bars + ring.buf());
-        // refill this buffer with chunk j + 2 as soon as its MMAs have drained (TS / KC >= 2: chunk j + 2 always
-        // exists here)
-        ++ring.chunk;
-        ring.wait_last();
-        --ring.chunk;
-        tma_issue(j + 2);
-      }
-      ++ring.chunk;
-    }
-  }
+  constexpr int LAST = NCH1 + TS / KC - 1;                   // last chunk of the weight ring
+  tma::mma_chunks<NCH1, KC, RL_NT, TF32>(ring, bars + 2, sB, FwdSmem<C>::B_FLOATS, TS * KC, tb, sA_hi, sA_lo, C,
+                                         umma::idesc_tf32(TM, TS), LAST, tma_issue);
   RL_TS(umma, 4);
   ring.wait_last();
   umma::tc_fence_after();
@@ -255,114 +173,33 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_fwd_umma_kernel(const rl_f
 #pragma unroll
       for (int i = 0; i < 32; i += 2) gelu2(hv[i], hv[i + 1], hv[i], hv[i + 1]);
     }
-    const int obase = (row & 7) * 4 + (row >> 3) * (TS / 4) * 32;
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const int o = obase + (col0 / 4 + i) * 32;
-      const float4 g = make_float4(hv[4 * i], hv[4 * i + 1], hv[4 * i + 2], hv[4 * i + 3]);
-      if constexpr (TF32) {
-        *reinterpret_cast<float4*>(sA_hi + o) = umma::rna4(g);
-      } else {
-        *reinterpret_cast<float4*>(sA_hi + o) = g;
-        *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(g);
-      }
-    }
+    for (int i = 0; i < 8; ++i)
+      umma::store_pair<TF32>(sA_hi, sA_lo, umma::kmajor_off(row >> 3, row & 7, col0 / 4 + i, TS),
+                             make_float4(hv[4 * i], hv[4 * i + 1], hv[4 * i + 2], hv[4 * i + 3]));
   }
   umma::tc_fence_before();     // the tcgen05.ld reads of the fc1 accumulator precede the barrier below
   RL_TS(umma, 6);
 
   // 4. partial output of this hidden slice: yp = g2 W2[:, 128 r : 128 r + 128]^T  (M = TM, N = C, K = TS)
   //    -> TMEM columns [TS, TS + C)
-  {
-    constexpr uint32_t idesc = umma::idesc_tf32(TM, C);
-#pragma unroll
-    for (int j = 0; j < TS / KC; ++j) {
-      float* bh = sB + ring.buf() * 2 * FwdSmem<C>::B_FLOATS;
-      float* bl = bh + FwdSmem<C>::B_FLOATS;
-      tma_consume(NCH1 + j, C);
-      umma::fence_async_smem();
-      __syncthreads();
-      if (tid == 0) {
-        umma::tc_fence_after();
-        tma::mma_chunk_3x<KC, TF32>(tb + TS, sA_hi, sA_lo, TS, j * KC, bh, bl, idesc, j > 0 ? 1u : 0u);
-        umma::commit(bars + ring.buf());
-        if (j + 2 < TS / KC) {
-          ++ring.chunk;
-          ring.wait_last();
-          --ring.chunk;
-          tma_issue(NCH1 + j + 2);
-        }
-      }
-      ++ring.chunk;
-    }
-  }
+  tma::mma_chunks<TS / KC, KC, RL_NT, TF32>(ring, bars + 2, sB, FwdSmem<C>::B_FLOATS, C * KC, tb + TS, sA_hi, sA_lo, TS,
+                                            umma::idesc_tf32(TM, C), LAST, tma_issue);
   ring.wait_last();
   umma::tc_fence_after();
   RL_TS(umma, 7);
 
   // 5. epilogue 2: partial tile -> shared memory [TM][C + 4] (over the dead g2 tile), DSMEM reduction:
   //    CTA r finishes rows [r * TM / NSL, (r + 1) * TM / NSL)
-  constexpr int LDP = C + 4;
   float* sp = smem;
-  {
-    const int quad = warp & 3, cgp = warp >> 2;
-    const int row = quad * 32 + lane;
-    constexpr int CW = C / 4;                                 // columns per warp group (16 or 32)
-#pragma unroll
-    for (int c16 = 0; c16 < CW; c16 += 16) {
-      float t0[16];
-      umma::tmem_ld16(umma::tmem_addr(tb, TS + cgp * CW + c16), t0);
-#pragma unroll
-      for (int i = 0; i < 16; i += 4)
-        *reinterpret_cast<float4*>(sp + row * LDP + cgp * CW + c16 + i) = make_float4(t0[i], t0[i + 1], t0[i + 2], t0[i + 3]);
-    }
-  }
+  umma::tmem_to_smem<C>(sp, tb, TS);
   umma::tc_fence_before();
-  // rows [r RPC, (r + 1) RPC) are finished here: their bias + residual (+ extra) terms are fetched before the
-  // cluster barrier instead of one round trip per item behind it
-  constexpr int RPC = TM / NSL, RIT = RPC * (C / 4) / RL_NT;  // rows finished by this CTA, float4 items per thread
-  static_assert(RPC * (C / 4) % RL_NT == 0, "reduce: items must tile the CTA");
-  float4 add4[RIT];
-#pragma unroll
-  for (int it = 0; it < RIT; ++it) {
-    const int i = tid + it * RL_NT;
-    const int rr = r * RPC + i / (C / 4), c = (i % (C / 4)) * 4;
-    add4[it] = a.b2 ? __ldg(reinterpret_cast<const float4*>(a.b2 + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
-    if (rr < nvalid) {
-      const size_t g = (tok0 + rr) * C + c;
-      if (a.flags & RL_F_RESIDUAL) {
-        const float4 x4 = __ldg(reinterpret_cast<const float4*>(a.x + g));
-        add4[it].x += x4.x; add4[it].y += x4.y; add4[it].z += x4.z; add4[it].w += x4.w;
-      }
-      if (a.extra) {
-        const float4 e4 = __ldg(reinterpret_cast<const float4*>(a.extra + g));
-        add4[it].x += e4.x; add4[it].y += e4.y; add4[it].z += e4.z; add4[it].w += e4.w;
-      }
-    }
-  }
+  umma::ClusterReduce<TM, C, NSL> red;
+  red.load(r, nvalid, tok0, a.b2, a.x, a.flags & RL_F_RESIDUAL, a.extra);
   RL_TS(umma, 8);
   cluster.sync();
   RL_TS(umma, 9);
-  {
-    const float* part[NSL];
-#pragma unroll
-    for (int q = 0; q < NSL; ++q) part[q] = cluster.map_shared_rank(sp, q);
-#pragma unroll
-    for (int it = 0; it < RIT; ++it) {
-      const int i = tid + it * RL_NT;
-      const int rr = r * RPC + i / (C / 4), c = (i % (C / 4)) * 4;
-      if (rr >= nvalid) continue;
-      const int off = rr * LDP + c;
-      float4 s = *reinterpret_cast<const float4*>(part[0] + off);
-#pragma unroll
-      for (int q = 1; q < NSL; ++q) {
-        const float4 p = *reinterpret_cast<const float4*>(part[q] + off);
-        s.x += p.x; s.y += p.y; s.z += p.z; s.w += p.w;
-      }
-      s.x += add4[it].x; s.y += add4[it].y; s.z += add4[it].z; s.w += add4[it].w;
-      *reinterpret_cast<float4*>(a.y + (tok0 + rr) * C + c) = s;
-    }
-  }
+  red.store(cluster, sp, r, nvalid, tok0, a.y);
   RL_TS(umma, 10);
   cluster.sync();     // nobody may exit while its partial tile is still being read
   if (warp == 0) umma::tmem_dealloc<TMEM_COLS>(tb);
@@ -433,21 +270,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
   if (warp == 0) umma::tmem_alloc<TMEM_COLS>(tmem_slot);
 
   // 1. g tile -> A (K-major, KT = C) with remainder
-  {
-    constexpr int NI = C / 16;
-    const int rsub = lane & 7, qsub = lane >> 3;
-    const int row = warp * 8 + rsub;
-    const bool ok = row < nvalid;
-#pragma unroll
-    for (int i = 0; i < NI; ++i) {
-      const int qc = qsub + 4 * i;
-      const float4 v = ok ? __ldg(reinterpret_cast<const float4*>(gw + (size_t)row * C) + qc)
-                          : make_float4(0.f, 0.f, 0.f, 0.f);
-      const int o = rsub * 4 + qc * 32 + warp * (C / 4) * 32;
-      *reinterpret_cast<float4*>(sA_hi + o) = v;
-      *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(v);
-    }
-  }
+  umma::stage_rows<C, false>(sA_hi, sA_lo, gw, nvalid, false, nullptr, [](float4 v, int, int) { return v; });
   umma::tc_fence_before();
   __syncthreads();
   umma::tc_fence_after();
@@ -506,7 +329,6 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
     }
     ring.wait_last();
     umma::tc_fence_after();
-    const int obase = (row & 7) * 4 + (row >> 3) * (TS / 4) * 32;
 #pragma unroll
     for (int half = 0; half < 2; ++half) {
       float v[16], hh[16], g2v[16];
@@ -549,12 +371,9 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
         }
       }
 #pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int o = obase + (col0 / 4 + 4 * half + i) * 32;
-        const float4 d = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
-        *reinterpret_cast<float4*>(sA_hi + o) = d;
-        *reinterpret_cast<float4*>(sA_lo + o) = umma::lo4(d);
-      }
+      for (int i = 0; i < 4; ++i)
+        umma::store_pair(sA_hi, sA_lo, umma::kmajor_off(row >> 3, row & 7, col0 / 4 + 4 * half + i, TS),
+                         make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]));
     }
     __syncthreads();
     if (part0) {                                             // adjoint of the 3-tap FIR on hidden channel 0
@@ -567,7 +386,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
         const float dg1 = lw0 * dn + lw1 * d + lw2 * dp;
         const float dh = ok ? dg1 * gelu_grad_f(h0) : 0.f;
         if (ok) a.dh[hoff] = dh;
-        const int o = obase + (col0 / 4) * 32;               // element (row, k = 0) of the dh tile
+        const int o = umma::kmajor_off(row >> 3, row & 7, col0 / 4, TS);   // element (row, k = 0) of the dh tile
         sA_hi[o] = dh;
         sA_lo[o] = dh - umma::trunc_tf32(dh);
         a0 = d * ((tl > 0) ? sg10[row - 1] : 0.f);
@@ -614,19 +433,7 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
   // 5. partial tile -> shared memory, DSMEM reduction + LayerNorm backward: CTA r finishes rows [r RPC, (r+1) RPC)
   constexpr int LDP = C + 4;
   float* sp = smem;
-  {
-    const int quad = warp & 3, cgp = warp >> 2;
-    const int row = quad * 32 + lane;
-    constexpr int CW = C / 4;
-#pragma unroll
-    for (int c16 = 0; c16 < CW; c16 += 16) {
-      float t0[16];
-      umma::tmem_ld16(umma::tmem_addr(tb, TS + cgp * CW + c16), t0);
-#pragma unroll
-      for (int i = 0; i < 16; i += 4)
-        *reinterpret_cast<float4*>(sp + row * LDP + cgp * CW + c16 + i) = make_float4(t0[i], t0[i + 1], t0[i + 2], t0[i + 3]);
-    }
-  }
+  umma::tmem_to_smem<C>(sp, tb, TS);
   umma::tc_fence_before();
   cluster.sync();
   {
@@ -641,16 +448,8 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
     const float* xr = a.x + (tok0 + row0) * C;
     const float* gr = gw + (size_t)row0 * C;
     const bool resid = a.flags & RL_F_RESIDUAL;
-    auto du_at4 = [&](int t, int c) {          // four channels of the reduced partial tiles (16-byte DSMEM loads)
-      const int off = (row0 + t) * LDP + c;
-      float4 s = *reinterpret_cast<const float4*>(part[0] + off);
-#pragma unroll
-      for (int q = 1; q < NSL; ++q) {
-        const float4 p = *reinterpret_cast<const float4*>(part[q] + off);
-        s.x += p.x; s.y += p.y; s.z += p.z; s.w += p.w;
-      }
-      return s;
-    };
+    // four channels of the reduced partial tiles
+    auto du_at4 = [&](int t, int c) { return umma::dsmem_sum4<NSL>(part, (row0 + t) * LDP + c); };
     if (a.flags & RL_F_PRENORM) {
       const float* lw = a.ln_w;
       const float* lb = a.ln_b;
@@ -685,29 +484,6 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_umma_kernel(const rl_f
   if (warp == 0) umma::tmem_dealloc<TMEM_COLS>(tb);
 }
 
-template <typename Args>
-int launch_cluster(void (*kernel)(const Args), size_t smem, int grid, int cl, const Args& a, cudaStream_t st,
-                   const char* name, int C) {
-  if (int rc = rl_set_smem(kernel, smem)) return rc;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(RL_NT);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = cl;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  rl_prof_pre(st);
-  cudaLaunchKernelEx(&cfg, kernel, a);
-  return rl_check_launch(name, C);
-}
-
 }  // namespace
 
 template <int C, bool TF32>
@@ -719,22 +495,7 @@ static int launch_fwd(const rl_ffn_fwd_args* a, int tiles, cudaStream_t st) {
   auto kernel = ffn_fwd_umma_kernel<C, TF32>;
   const size_t smem = FwdSmem<C>::BYTES + 64;
   if (int rc = rl_set_smem(kernel, smem)) return rc;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(tiles * NSL);
-  cfg.blockDim = dim3(RL_NT);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = NSL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  rl_prof_pre(st);
-  cudaLaunchKernelEx(&cfg, kernel, *a, tm1, tm2);
+  rl_launch_pdl_cluster(NSL, kernel, dim3(tiles * NSL), dim3(RL_NT), smem, st, *a, tm1, tm2);
   return rl_check_launch("ffn_fwd_umma", C, -1, rl_tf32_tag(TF32));
 }
 
@@ -751,15 +512,18 @@ int rl_ffn_fwd_umma(const rl_ffn_fwd_args* a, cudaStream_t st) {
 template <int C>
 static int launch_bwd(const rl_ffn_bwd_args* a, int tiles, cudaStream_t st, RlDet* det) {
   constexpr int NSL = 4 * C / TS;
-  if (det == nullptr)
-    return launch_cluster(ffn_bwd_umma_kernel<C, false>, BwdSmem<C>::BYTES, tiles * NSL, NSL, *a, st, "ffn_bwd_umma", C);
-  // det: LayerNorm partials one slot per CTA, local-enhancement taps one slot per token tile
+  auto kernel = ffn_bwd_umma_kernel<C, false>;
   rl_ffn_bwd_args d = *a;
-  d.d_ln_w = rl_det_take(det, a->d_ln_w, C, tiles * NSL);
-  d.d_ln_b = rl_det_take(det, a->d_ln_b, C, tiles * NSL);
-  d.d_lew = (a->le_mode == RL_LE_PARTIAL) ? rl_det_take(det, a->d_lew, 3, tiles) : nullptr;
-  RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "ffn_bwd: deterministic-mode workspace too small");
-  return launch_cluster(ffn_bwd_umma_kernel<C, true>, BwdSmem<C>::BYTES, tiles * NSL, NSL, d, st, "ffn_bwd_umma", C);
+  if (det) {     // LayerNorm partials one slot per CTA, local-enhancement taps one slot per token tile
+    d.d_ln_w = rl_det_take(det, a->d_ln_w, C, tiles * NSL);
+    d.d_ln_b = rl_det_take(det, a->d_ln_b, C, tiles * NSL);
+    d.d_lew = (a->le_mode == RL_LE_PARTIAL) ? rl_det_take(det, a->d_lew, 3, tiles) : nullptr;
+    RL_REQUIRE(rl_det_ok(det), RL_ERR_SHAPE, "ffn_bwd: deterministic-mode workspace too small");
+    kernel = ffn_bwd_umma_kernel<C, true>;
+  }
+  if (int rc = rl_set_smem(kernel, BwdSmem<C>::BYTES)) return rc;
+  rl_launch_pdl_cluster(NSL, kernel, dim3(tiles * NSL), dim3(RL_NT), BwdSmem<C>::BYTES, st, d);
+  return rl_check_launch("ffn_bwd_umma", C);
 }
 
 int rl_ffn_bwd_umma(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {

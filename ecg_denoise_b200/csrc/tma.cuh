@@ -87,4 +87,37 @@ __device__ __forceinline__ void derive_lo(float* hi, float* lo, int floats) {
     else l4[i] = umma::lo4(v);
   }
 }
+
+// The TMA-fed chunk loop of one GEMM: D[tmem] (+)= A[:, 0 : NCH * KCW] * B^T, B streamed through the 2-deep weight ring.
+// Chunk jj = ring.chunk lands in buffer b = jj & 1 of ring_mem (hi tile at b * 2 * stage floats, remainder tile
+// `stage` floats after it) and completes the transaction barrier full[b]; `floats` floats land per chunk.  All NT
+// threads wait for the chunk and derive its remainder; thread 0 issues its MMAs, commits them on ring.bar[b] and, once
+// they have drained, refills the buffer through issue(jj + 2) while jj + 2 <= last.
+template <int NCH, int KCW, int NT, bool TF32, typename Issue>
+__device__ __forceinline__ void mma_chunks(umma::Ring& ring, uint64_t* full, float* ring_mem, int stage, int floats,
+                                           uint32_t tmem_d, const float* a_hi, const float* a_lo, int KT_A,
+                                           uint32_t idesc, int last, Issue&& issue) {
+#pragma unroll
+  for (int j = 0; j < NCH; ++j) {
+    const int jj = ring.chunk;
+    float* bh = ring_mem + ring.buf() * 2 * stage;
+    float* bl = bh + stage;
+    umma::mbar_wait(full + (jj & 1), (uint32_t)((jj >> 1) & 1));
+    derive_lo<NT, TF32>(bh, bl, floats);
+    umma::fence_async_smem();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      umma::tc_fence_after();
+      mma_chunk_3x<KCW, TF32>(tmem_d, a_hi, a_lo, KT_A, j * KCW, bh, bl, idesc, j > 0 ? 1u : 0u);
+      umma::commit(ring.bar + ring.buf());
+      if (jj + 2 <= last) {
+        ++ring.chunk;
+        ring.wait_last();
+        --ring.chunk;
+        issue(jj + 2);
+      }
+    }
+    ++ring.chunk;
+  }
+}
 }  // namespace tma

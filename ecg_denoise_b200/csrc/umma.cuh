@@ -1,6 +1,8 @@
 // umma.cuh -- tcgen05 (5th-generation tensor core) building blocks for the wide RA-LENet stages:
 // TMEM allocation, un-swizzled K-major shared-memory matrix descriptors, kind::tf32 MMA issue with the
-// 3-pass split (hi*hi + lo*hi + hi*lo, fp32-grade), mbarrier completion tracking and TMEM -> register loads.
+// 3-pass split (hi*hi + lo*hi + hi*lo, fp32-grade), mbarrier completion tracking and TMEM -> register loads; and
+// the phases the tile kernels share: operand staging into the K-major layout, TMEM -> shared partial tiles and their
+// reduction across a cluster.
 //
 // Facts verified on B200 with tools/umma_probe.cu (gpurun_out/umma_probe1.txt, summarised in profiles/):
 //   * kind::tf32 reads the fp32 container and ignores the low 13 mantissa bits (matches a truncating
@@ -13,6 +15,8 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <cooperative_groups.h>
+#include "common.cuh"
 
 namespace umma {
 
@@ -160,21 +164,172 @@ __device__ __forceinline__ float4 lo4(float4 v) {
   return r;
 }
 
+
 // ---------------------------------------------------------------------------------------------
-// Staging of a ROWS x KC operand block whose contraction index is the ROW of the global matrix (dgrad: B = W^T) into a
-// K-major tile pair (hi = x, lo = x - trunc(x)):   element (n, k) <- src[k * ld + n],  n < ROWS (multiple of 32),
-// k < KC.  A warp reads 32 consecutive n of four consecutive k rows (4 x 128 contiguous bytes) and each lane writes one
-// 16-byte chunk (its n, four k) of the K-major tile.  Split in two halves so that the global loads can be issued long
-// before the tile buffer is free: load() pulls the block into registers, store() splits and writes it.  NT = threads of
-// the CTA.
-template <int ROWS, int KC, int NT>
+// The un-swizzled K-major core-matrix layout of the staged tiles (the `make_desc` strides of mma_chunk_3x: LBO = 128 B,
+// SBO = KT / 4 * 128 B): offset in floats of the 16-byte chunk (row 8 g + r, elements [4 q, 4 q + 4)) of a tile with
+// KT contraction elements per row.
+__device__ __forceinline__ int kmajor_off(int g, int r, int q, int KT) { return r * 4 + q * 32 + g * (KT / 4) * 32; }
+
+// four values of a tile pair at offset o: hi = v, lo = its tf32 remainder; TF32 (single pass): hi = v rounded to tf32
+template <bool TF32 = false>
+__device__ __forceinline__ void store_pair(float* hi, float* lo, int o, float4 v) {
+  if constexpr (TF32) {
+    *reinterpret_cast<float4*>(hi + o) = rna4(v);
+  } else {
+    *reinterpret_cast<float4*>(hi + o) = v;
+    *reinterpret_cast<float4*>(lo + o) = lo4(v);
+  }
+}
+
+// Rows -> A tile: the TM = 128 rows of src (row-major, KT floats per row; rows >= nvalid staged as zeros) into a
+// K-major tile pair with KT elements per row, by the 16 warps of the CTA.  A warp owns 8 rows; lane = (row % 8,
+// 16-byte chunk % 4), so global reads cover full sectors and the tile stores are contiguous.  `norm`: each 16-byte
+// chunk v of row `row` first becomes pre(v, row, chunk), then the row is layer-normalised with the affine
+// s_ln = weight [KT] | bias [KT] staged in shared memory.
+template <int KT, bool TF32, typename Pre>
+__device__ __forceinline__ void stage_rows(float* hi, float* lo, const float* __restrict__ src, int nvalid, bool norm,
+                                           const float* s_ln, Pre pre) {
+  constexpr int NI = KT / 16;                                // chunks per lane
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int rsub = lane & 7, qsub = lane >> 3;
+  const int row = warp * 8 + rsub;
+  const bool ok = row < nvalid;
+  float4 v[NI];
+  float s = 0.f;
+#pragma unroll
+  for (int i = 0; i < NI; ++i) {
+    const int qc = qsub + 4 * i;
+    v[i] = ok ? __ldg(reinterpret_cast<const float4*>(src + (size_t)row * KT) + qc) : make_float4(0.f, 0.f, 0.f, 0.f);
+    if (norm) v[i] = pre(v[i], row, qc);
+    s += v[i].x + v[i].y + v[i].z + v[i].w;
+  }
+  float mu = 0.f, rstd = 1.f;
+  if (norm) {
+    s += __shfl_xor_sync(0xffffffffu, s, 8);
+    s += __shfl_xor_sync(0xffffffffu, s, 16);
+    mu = s * (1.0f / KT);
+    float q = 0.f;
+#pragma unroll
+    for (int i = 0; i < NI; ++i) {
+      const float d0 = v[i].x - mu, d1 = v[i].y - mu, d2 = v[i].z - mu, d3 = v[i].w - mu;
+      q += d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3;
+    }
+    q += __shfl_xor_sync(0xffffffffu, q, 8);
+    q += __shfl_xor_sync(0xffffffffu, q, 16);
+    rstd = rsqrtf(q * (1.0f / KT) + RL_LN_EPS);
+  }
+#pragma unroll
+  for (int i = 0; i < NI; ++i) {
+    const int qc = qsub + 4 * i;
+    float4 u = v[i];
+    if (norm) {
+      const float4 w4 = *reinterpret_cast<const float4*>(s_ln + 4 * qc);
+      const float4 b4 = *reinterpret_cast<const float4*>(s_ln + KT + 4 * qc);
+      u.x = fmaf((v[i].x - mu) * rstd, w4.x, b4.x);
+      u.y = fmaf((v[i].y - mu) * rstd, w4.y, b4.y);
+      u.z = fmaf((v[i].z - mu) * rstd, w4.z, b4.z);
+      u.w = fmaf((v[i].w - mu) * rstd, w4.w, b4.w);
+      if (!ok) u = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    store_pair<TF32>(hi, lo, kmajor_off(warp, rsub, qc, KT), u);
+  }
+}
+
+// Accumulator -> shared memory: the TM = 128 x C fp32 tile at TMEM column col into sp [TM][C + 4].  Warp w reads its
+// lane quadrant w % 4 (row 32 (w % 4) + lane = threadIdx.x % 128) and the C / 4 columns of group w / 4.
+template <int C>
+__device__ __forceinline__ void tmem_to_smem(float* sp, uint32_t tmem_base, int col) {
+  constexpr int LDP = C + 4, CW = C / 4;                     // row stride, columns per warp group (16 or 32)
+  const int row = threadIdx.x & 127, cgp = threadIdx.x >> 7;
+#pragma unroll
+  for (int c16 = 0; c16 < CW; c16 += 16) {
+    float t0[16];
+    tmem_ld16(tmem_addr(tmem_base, col + cgp * CW + c16), t0);
+#pragma unroll
+    for (int i = 0; i < 16; i += 4)
+      *reinterpret_cast<float4*>(sp + row * LDP + cgp * CW + c16 + i) = make_float4(t0[i], t0[i + 1], t0[i + 2], t0[i + 3]);
+  }
+}
+
+// sum of the NSL partial tiles of a cluster (part[q] = tile of CTA rank q, 16-byte DSMEM loads) at offset off
+template <int NSL>
+__device__ __forceinline__ float4 dsmem_sum4(const float* const (&part)[NSL], int off) {
+  float4 s = *reinterpret_cast<const float4*>(part[0] + off);
+#pragma unroll
+  for (int q = 1; q < NSL; ++q) {
+    const float4 p = *reinterpret_cast<const float4*>(part[q] + off);
+    s.x += p.x; s.y += p.y; s.z += p.z; s.w += p.w;
+  }
+  return s;
+}
+
+// Reduction of the partial output tiles [TM][C + 4] of a cluster of NSL CTAs, y = sum of the partials + bias
+// (+ residual) (+ extra): CTA r finishes rows [r RPC, (r + 1) RPC).  load() fetches the bias and residual terms of
+// those rows before the cluster barrier instead of one round trip per item behind it; store() sums and writes them.
+template <int TM, int C, int NSL>
+struct ClusterReduce {
+  static constexpr int RPC = TM / NSL, RIT = RPC * (C / 4) / RL_NT;  // rows finished per CTA, float4 items per thread
+  static_assert(RPC * (C / 4) % RL_NT == 0, "reduce: items must tile the CTA");
+  float4 add4[RIT];
+
+  // bias [C] or NULL; x (added if resid), extra (or NULL): [tokens][C]; rows of the tile start at token tok0
+  __device__ __forceinline__ void load(int r, int nvalid, size_t tok0, const float* bias, const float* x, bool resid,
+                                       const float* extra) {
+#pragma unroll
+    for (int it = 0; it < RIT; ++it) {
+      const int i = threadIdx.x + it * RL_NT;
+      const int rr = r * RPC + i / (C / 4), c = (i % (C / 4)) * 4;
+      add4[it] = bias ? __ldg(reinterpret_cast<const float4*>(bias + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      if (rr < nvalid) {
+        const size_t g = (tok0 + rr) * C + c;
+        if (resid) {
+          const float4 x4 = __ldg(reinterpret_cast<const float4*>(x + g));
+          add4[it].x += x4.x; add4[it].y += x4.y; add4[it].z += x4.z; add4[it].w += x4.w;
+        }
+        if (extra) {
+          const float4 e4 = __ldg(reinterpret_cast<const float4*>(extra + g));
+          add4[it].x += e4.x; add4[it].y += e4.y; add4[it].z += e4.z; add4[it].w += e4.w;
+        }
+      }
+    }
+  }
+  // after the cluster barrier: sp = this CTA's partial tile (the same offset in every CTA of the cluster)
+  __device__ __forceinline__ void store(cooperative_groups::cluster_group& cluster, float* sp, int r, int nvalid,
+                                        size_t tok0, float* y) const {
+    const float* part[NSL];
+#pragma unroll
+    for (int q = 0; q < NSL; ++q) part[q] = cluster.map_shared_rank(sp, q);
+#pragma unroll
+    for (int it = 0; it < RIT; ++it) {
+      const int i = threadIdx.x + it * RL_NT;
+      const int rr = r * RPC + i / (C / 4), c = (i % (C / 4)) * 4;
+      if (rr >= nvalid) continue;
+      float4 s = dsmem_sum4<NSL>(part, rr * (C + 4) + c);
+      s.x += add4[it].x; s.y += add4[it].y; s.z += add4[it].z; s.w += add4[it].w;
+      *reinterpret_cast<float4*>(y + (tok0 + rr) * C + c) = s;
+    }
+  }
+};
+
+// ---------------------------------------------------------------------------------------------
+// Staging of a ROWS x KC operand block whose contraction index is the ROW of the global matrix (dgrad: B = W^T; the
+// weight gradients: both operands, contraction over the tokens) into a K-major tile pair (hi = x, lo = x - trunc(x)):
+// element (n, k) <- src[k * ld + n],  n < ROWS (multiple of 32), k < KC.  A warp reads 32 consecutive n of four
+// consecutive k rows (4 x 128 contiguous bytes) and each lane writes one 16-byte chunk (its n, four k) of the K-major
+// tile.  Split in two halves so that the global loads can be issued long before the tile buffer is free: load() pulls
+// the block into registers, store() splits and writes it.  NT = threads of the CTA.  GUARD: rows n >= rows_valid and
+// k >= m_end - m0 are staged as zeros.
+template <int ROWS, int KC, int NT, bool GUARD = false>
 struct TStage {
   static constexpr int NB = ROWS / 32, NQ = KC / 4, ITEMS = NB * NQ;
   static constexpr int PER = (ITEMS + NT / 32 - 1) / (NT / 32);
   static_assert(ROWS % 32 == 0 && KC % 4 == 0, "TStage: tile shape");
   float4 v[PER];
 
-  __device__ __forceinline__ void load(const float* __restrict__ src, int ld) {
+  // src -> element (n = 0, k = m0)
+  __device__ __forceinline__ void load(const float* __restrict__ src, int ld, int rows_valid = ROWS, int m0 = 0,
+                                       int m_end = KC) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 #pragma unroll
     for (int i = 0; i < PER; ++i) {
@@ -182,8 +337,17 @@ struct TStage {
       v[i] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (item < ITEMS) {
         const int nb = item % NB, q = item / NB;
-        const float* p = src + (size_t)(4 * q) * ld + nb * 32 + lane;
-        v[i] = make_float4(__ldg(p), __ldg(p + ld), __ldg(p + 2 * (size_t)ld), __ldg(p + 3 * (size_t)ld));
+        const int n = nb * 32 + lane, m = m0 + 4 * q;
+        if (!GUARD || n < rows_valid) {
+          const float* p = src + (size_t)m * ld + n;
+          if (!GUARD || m + 3 < m_end) {
+            v[i] = make_float4(__ldg(p), __ldg(p + ld), __ldg(p + 2 * (size_t)ld), __ldg(p + 3 * (size_t)ld));
+          } else {
+            if (m < m_end) v[i].x = __ldg(p);
+            if (m + 1 < m_end) v[i].y = __ldg(p + ld);
+            if (m + 2 < m_end) v[i].z = __ldg(p + 2 * (size_t)ld);
+          }
+        }
       }
     }
   }
@@ -193,14 +357,20 @@ struct TStage {
     for (int i = 0; i < PER; ++i) {
       const int item = wid + i * (NT / 32);
       if (item < ITEMS) {
-        const int nb = item % NB, q = item / NB;
-        const int n = nb * 32 + lane;
-        const int o = (n & 7) * 4 + q * 32 + (n >> 3) * (NQ * 32);
-        *reinterpret_cast<float4*>(hi + o) = v[i];
-        *reinterpret_cast<float4*>(lo + o) = lo4(v[i]);
+        const int n = (item % NB) * 32 + lane;
+        store_pair(hi, lo, kmajor_off(n >> 3, n & 7, item / NB, KC), v[i]);
       }
     }
   }
+  // sum over the staged k of the row this thread holds (every item of a thread has the same row: (NT / 32) % NB == 0)
+  __device__ __forceinline__ float token_sum() const {
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < PER; ++i) s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
+    return s;
+  }
+  __device__ __forceinline__ int my_row() const { return ((threadIdx.x >> 5) % NB) * 32 + (threadIdx.x & 31); }
+  __device__ __forceinline__ bool active() const { return (int)(threadIdx.x >> 5) < ITEMS; }
 };
 
 }  // namespace umma

@@ -46,65 +46,10 @@ struct WuGroup {
   int nprob, M, MC;
 };
 
-// one chunk of an operand: ROWS output rows (or columns) x KC tokens, transposed into a K-major tile pair.
-// A warp reads 32 consecutive rows of four consecutive tokens and each lane owns one 16-byte chunk (its row, four
-// tokens) of the tile (umma::TStage with row / token guards).
+// one chunk of an operand: ROWS output rows (or columns) x KC tokens, transposed into a K-major tile pair; rows
+// beyond the problem and tokens beyond the slice are staged as zeros
 template <int ROWS>
-struct TokStage {
-  static constexpr int NB = ROWS / 32, NQ = KC / 4, ITEMS = NB * NQ, NWARP = RL_NT / 32;
-  static constexpr int PER = (ITEMS + NWARP - 1) / NWARP;
-  static_assert(ROWS % 32 == 0, "TokStage: tile shape");
-  float4 v[PER];
-
-  // src -> first row of the tile at token m0; rows_valid rows, tokens [m0, m_end) exist
-  __device__ __forceinline__ void load(const float* __restrict__ src, int ld, int rows_valid, int m0, int m_end) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) {
-      const int item = wid + i * NWARP;
-      v[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (item < ITEMS) {
-        const int nb = item % NB, q = item / NB;
-        const int n = nb * 32 + lane, m = m0 + 4 * q;
-        if (n < rows_valid) {
-          const float* p = src + (size_t)m * ld + n;
-          if (m + 3 < m_end) {
-            v[i] = make_float4(__ldg(p), __ldg(p + ld), __ldg(p + 2 * (size_t)ld), __ldg(p + 3 * (size_t)ld));
-          } else {
-            if (m < m_end) v[i].x = __ldg(p);
-            if (m + 1 < m_end) v[i].y = __ldg(p + ld);
-            if (m + 2 < m_end) v[i].z = __ldg(p + 2 * (size_t)ld);
-          }
-        }
-      }
-    }
-  }
-  __device__ __forceinline__ void store(float* hi, float* lo) const {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) {
-      const int item = wid + i * NWARP;
-      if (item < ITEMS) {
-        const int nb = item % NB, q = item / NB;
-        const int n = nb * 32 + lane;
-        const int o = (n & 7) * 4 + q * 32 + (n >> 3) * (NQ * 32);
-        *reinterpret_cast<float4*>(hi + o) = v[i];
-        *reinterpret_cast<float4*>(lo + o) =
-            umma::lo4(v[i]);
-      }
-    }
-  }
-  // sum over the staged tokens of the row this thread holds (every item of a thread has the same row:
-  // NWARP % NB == 0)
-  __device__ __forceinline__ float token_sum() const {
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
-    return s;
-  }
-  __device__ __forceinline__ int my_row() const { return ((threadIdx.x >> 5) % NB) * 32 + (threadIdx.x & 31); }
-  __device__ __forceinline__ bool active() const { return (int)(threadIdx.x >> 5) < ITEMS; }
-};
+using TokStage = umma::TStage<ROWS, KC, RL_NT, true>;
 
 template <int TK>
 struct WuSmem {

@@ -63,8 +63,6 @@ buf = (ctypes.c_longlong * (ncta * 16))()
 lib.ralenet_debug_trace_read_attn_umma.argtypes = [ctypes.POINTER(ctypes.c_longlong), ctypes.c_int]
 print("read rc", lib.ralenet_debug_trace_read_attn_umma(buf, ncta * 16))
 full = np.array(buf[:], dtype=np.int64).reshape(ncta, 16)
-print(f"  within PE+LN: x loads landed after {np.median(full[:, 13] - full[:, 2]):.0f}, statistics after "
-      f"{np.median(full[:, 14] - full[:, 13]):.0f}, normalise + tile stores {np.median(full[:, 3] - full[:, 14]):.0f} cycles (thread 0)")
 t = full[:, :13]
 d = np.diff(t, axis=1)
 names = ["prefetch->pdl", "pdl->alloc/init/table", "PE+LN tile", "qkv stage+issue", "wait qkv", "epilogue1 (q,k,v)",
