@@ -36,10 +36,21 @@ __host__ __device__ constexpr int ffn_bwd_swf() {
   return cmax(cmax(WStream<4 * C, C, B_KN>::FLOATS, WStream<C, 4 * C, B_KN>::FLOATS),
               cmax((C <= RL_FW_MAXC) ? 16 * 144 : 0, 32 * C));
 }
+// true: the fc1 / fc2 weight gradients are accumulated inside the data-gradient kernel (narrow stages, C <= 16), which
+// keeps g2 in shared memory for them; false: the kernel writes g2, dh and u to the global scratch and rl_ffn_bwd_wgrad
+// launches the GEMMs.  The depthwise backward of 512-sample windows (WIN = 2) already holds g1 in shared memory: with the
+// g2 tile as well it would need 256 KB (C = 16) / 279 KB (C = 8), more than an SM has, so it takes the GEMM launch.
+__host__ __device__ constexpr bool ffn_bwd_in_cta_wgrad(int C, int WIN, bool dw) {
+  return C <= RL_FW_MAXC && !(dw && WIN == 2);
+}
+bool ffn_bwd_in_cta_wgrad(const rl_ffn_bwd_args* a) {
+  return ffn_bwd_in_cta_wgrad(a->C, a->L * a->C / 2048, a->le_mode == RL_LE_DEPTHWISE);
+}
+
 template <int C>
 size_t ffn_bwd_smem(int L, bool dw) {
-  // narrow stages (C <= 16) keep g2 in shared memory as well for the in-CTA weight gradients
-  return sizeof(float) * (2 * (size_t)L * ld_mk(C) + ((dw ? 2 : 1) + (C <= RL_FW_MAXC ? 1 : 0)) * (size_t)L * ld_mk(4 * C) +
+  const bool fw = ffn_bwd_in_cta_wgrad(C, L * C / 2048, dw);
+  return sizeof(float) * (2 * (size_t)L * ld_mk(C) + ((dw ? 2 : 1) + (fw ? 1 : 0)) * (size_t)L * ld_mk(4 * C) +
                           ffn_bwd_swf<C>() + 3 * (size_t)L + 2 * C + 64);
 }
 
@@ -53,8 +64,8 @@ __global__ void __launch_bounds__(RL_NT, RL_MINB) ffn_bwd_kernel(const rl_ffn_bw
   float* su = sg + L * LDC;               // du (LN2 output gradient)
   float* sd = su + L * LDC;               // df / dh
   float* sh = sd + L * LDH;               // g1 = GELU(h), depthwise mode only
-  constexpr bool FW = (C <= RL_FW_MAXC);          // narrow stages: weight gradients accumulated in-CTA (no wgrad launch)
-  float* sg2 = sh + (DW ? L * LDH : 0);   // g2, narrow stages only
+  constexpr bool FW = ffn_bwd_in_cta_wgrad(C, WIN, DW);   // weight gradients accumulated in-CTA (no wgrad launch)
+  float* sg2 = sh + (DW ? L * LDH : 0);   // g2, in-CTA weight gradients only
   float* sw = sg2 + (FW ? L * LDH : 0);
   float* sg10 = sw + ffn_bwd_swf<C>();    // g1[:,0]
   float* sf0 = sg10 + L;                  // fir(g1[:,0])
@@ -305,8 +316,8 @@ int launch_bwd_det(const rl_ffn_bwd_args* a, cudaStream_t st) {
   return dw ? launch_bwd_one<C, 2, true, DET>(a, st) : launch_bwd_one<C, 2, false, DET>(a, st);
 }
 
-// det: one partial slot per window (CTA) for the in-CTA gradients (LayerNorm, local enhancement; every weight at
-// C <= 16)
+// det: one partial slot per window (CTA) for the in-CTA gradients (LayerNorm, local enhancement; every weight where
+// ffn_bwd_in_cta_wgrad)
 template <int C>
 int launch_bwd(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   if (det == nullptr) return launch_bwd_det<C, false>(a, st);
@@ -316,7 +327,7 @@ int launch_bwd(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   d.d_ln_b = rl_det_take(det, a->d_ln_b, C, B);
   d.d_lew = (a->le_mode == RL_LE_NONE) ? nullptr
                                        : rl_det_take(det, a->d_lew, a->le_mode == RL_LE_DEPTHWISE ? 12 * C : 3, B);
-  if (C <= RL_FW_MAXC) {
+  if (ffn_bwd_in_cta_wgrad(a)) {
     d.d_w1 = rl_det_take(det, a->d_w1, 4 * C * C, B); d.d_b1 = rl_det_take(det, a->d_b1, 4 * C, B);
     d.d_w2 = rl_det_take(det, a->d_w2, 4 * C * C, B); d.d_b2 = rl_det_take(det, a->d_b2, C, B);
   }
@@ -379,12 +390,12 @@ int rl_ffn_bwd_main(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   return RL_ERR_SHAPE;
 }
 
-bool rl_ffn_bwd_has_wgrad(const rl_ffn_bwd_args* a) { return a->C > RL_FW_MAXC && (a->d_w1 || a->d_w2); }
+bool rl_ffn_bwd_has_wgrad(const rl_ffn_bwd_args* a) { return !ffn_bwd_in_cta_wgrad(a) && (a->d_w1 || a->d_w2); }
 
 // weight gradients from (g, g2) and (dh, u); may run on another stream once the main kernel is done
 int rl_ffn_bwd_wgrad(const rl_ffn_bwd_args* a, cudaStream_t st, RlDet* det) {
   const int M = a->B * a->L, C = a->C;
-  if (C <= RL_FW_MAXC) return RL_OK;        // narrow stages accumulate their weight gradients inside the kernel
+  if (ffn_bwd_in_cta_wgrad(a)) return RL_OK;   // accumulated inside the data-gradient kernel
   const RlWgradDesc d[2] = {{a->g, C, a->g2, 4 * C, C, 4 * C, a->d_w2, a->d_b2},
                             {a->dh, 4 * C, a->u, C, 4 * C, C, a->d_w1, a->d_b1}};
   return rl_launch_wgrad_group(d, 2, M, st, det);

@@ -1,6 +1,8 @@
 """Shared helpers for the parity tests (test infrastructure)."""
 from __future__ import annotations
 
+from contextlib import contextmanager
+
 import numpy as np
 import torch
 
@@ -59,3 +61,21 @@ def check_packed(got: torch.Tensor, gold, rtol: float, name: str):
     rms = gnorm / np.sqrt(n_el)
     err = np.max(np.abs(p[2:] - gsamp) / (np.abs(gsamp) + rms + 1e-30))
     assert err <= rtol, f"{name}: sample rel err {err:.3e} > {rtol}"
+
+
+@contextmanager
+def switches(mode):
+    """kernel-selection switches: 'default', 'reg2' (register-tile GEMMs for every group), 'mma' (mma.sync GEMMs)."""
+    from ecg_denoise_b200 import _lib
+    lib = _lib.load()
+    prev_reg, prev_umma = lib.ralenet_set_wgrad_reg(1), lib.ralenet_set_wgrad_umma(1)
+    if mode == "reg2":
+        lib.ralenet_set_wgrad_reg(2)
+    elif mode == "mma":
+        lib.ralenet_set_wgrad_reg(0)
+        lib.ralenet_set_wgrad_umma(0)
+    try:
+        yield
+    finally:
+        lib.ralenet_set_wgrad_reg(prev_reg)
+        lib.ralenet_set_wgrad_umma(prev_umma)

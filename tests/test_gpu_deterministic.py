@@ -12,7 +12,7 @@ import pytest
 import torch
 
 from oracle import synth_weights as SW
-from tests.common import CASES, check_packed, rel_rms_err, unpack_golden
+from tests.common import CASES, check_packed, rel_rms_err, switches, unpack_golden
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-3
@@ -32,24 +32,6 @@ def torch_deterministic(warn_only=False):
         yield
     finally:
         torch.use_deterministic_algorithms(state[0], warn_only=state[1])
-
-
-@contextmanager
-def switches(mode):
-    """kernel-selection switches: 'default', 'reg2' (register-tile GEMMs for every group), 'mma' (mma.sync GEMMs)."""
-    from ecg_denoise_b200 import _lib
-    lib = _lib.load()
-    prev_reg, prev_umma = lib.ralenet_set_wgrad_reg(1), lib.ralenet_set_wgrad_umma(1)
-    if mode == "reg2":
-        lib.ralenet_set_wgrad_reg(2)
-    elif mode == "mma":
-        lib.ralenet_set_wgrad_reg(0)
-        lib.ralenet_set_wgrad_umma(0)
-    try:
-        yield
-    finally:
-        lib.ralenet_set_wgrad_reg(prev_reg)
-        lib.ralenet_set_wgrad_umma(prev_umma)
 
 
 MODELS = {"rw_le_256": ("rw", 1, 256, 256), "rw_le_515": ("rw", 1, 515, 256), "nra512": ("nra", 1, 48, 512)}

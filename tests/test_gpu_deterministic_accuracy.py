@@ -25,8 +25,8 @@ import pytest
 import torch
 
 from oracle import ralenet_oracle as O
-from tests.common import rel_rms_err
-from tests.test_gpu_deterministic import _equal, _inputs, switches, torch_deterministic
+from tests.common import rel_rms_err, switches
+from tests.test_gpu_deterministic import _equal, _inputs, torch_deterministic
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-3
