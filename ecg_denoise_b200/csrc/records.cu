@@ -7,6 +7,8 @@
 // All three are HBM-bound streaming kernels.
 // For training (SURVEY.md 8f-3), record_sample_kernel draws the same z-normalised windows from a record bank in a
 // keyed per-epoch order and pairs each with a window of a noise bank and an SNR level; ralenet_snr_mix does the mix.
+// For evaluation, record_enumerate_kernel walks every (grid window, level) pair of held-out banks once, in order,
+// with a noise pick fixed per pair.
 #include "common.cuh"
 
 namespace {
@@ -116,6 +118,30 @@ __device__ __forceinline__ uint64_t feistel_perm(uint64_t x, uint64_t n, uint64_
   return x;
 }
 
+// Slot i of a drawn batch <- clean window (rec, off) of the record bank, z-normalised with the arithmetic of
+// window_gather_kernel, and noise window (nrec, noff) of the noise bank; clean lead l reads noise lead l % noise_leads.
+// A is rl_sample_args or rl_enum_args (same bank fields).
+template <typename A>
+__device__ __forceinline__ void copy_window_pair(const A& a, int i, int tid, int W, int64_t rec, int64_t off,
+                                                 int64_t nrec, int64_t noff) {
+  for (int l = 0; l < a.leads; ++l) {
+    const size_t rc = (size_t)rec * a.leads + l;
+    const float* xs = a.records + rc * a.T + off;
+    const float* ns = a.noise + ((size_t)nrec * a.noise_leads + l % a.noise_leads) * a.Tn + noff;
+    float mean = 0.f, rstd = 1.f;
+    if (a.stats) { mean = __ldg(a.stats + 2 * rc); rstd = __ldg(a.stats + 2 * rc + 1); }
+    float* cw = a.clean_out + ((size_t)i * a.leads + l) * W;
+    float* nw = a.noise_out + ((size_t)i * a.leads + l) * W;
+    for (int t = tid; t < W; t += RL_NT) {
+      float v = __ldg(xs + t);
+      const float nz = __ldg(ns + t);
+      if (a.stats) v = (v - mean) * rstd;          // the arithmetic of window_gather_kernel
+      cw[t] = v;
+      nw[t] = nz;
+    }
+  }
+}
+
 // one CTA per window; the plan (which record window, which noise window, which SNR level) is computed by every thread
 __global__ void __launch_bounds__(RL_NT) record_sample_kernel(rl_sample_args a, int nper, uint64_t n, uint64_t spe) {
   pdl_wait();                                     // *counter may be the Adam step counter the previous kernel bumped
@@ -139,22 +165,48 @@ __global__ void __launch_bounds__(RL_NT) record_sample_kernel(rl_sample_args a, 
       a.meta[4 * i + 3] = (int32_t)noff;
     }
   }
-  for (int l = 0; l < a.leads; ++l) {
-    const size_t rc = (size_t)rec * a.leads + l;
-    const float* xs = a.records + rc * a.T + off;
-    const float* ns = a.noise + ((size_t)nrec * a.noise_leads + l % a.noise_leads) * a.Tn + noff;
-    float mean = 0.f, rstd = 1.f;
-    if (a.stats) { mean = __ldg(a.stats + 2 * rc); rstd = __ldg(a.stats + 2 * rc + 1); }
-    float* cw = a.clean_out + ((size_t)i * a.leads + l) * W;
-    float* nw = a.noise_out + ((size_t)i * a.leads + l) * W;
-    for (int t = tid; t < W; t += RL_NT) {
-      float v = __ldg(xs + t);
-      const float nz = __ldg(ns + t);
-      if (a.stats) v = (v - mean) * rstd;          // the arithmetic of window_gather_kernel
-      cw[t] = v;
-      nw[t] = nz;
+  copy_window_pair(a, i, tid, W, rec, off, nrec, noff);
+}
+
+// one CTA per slot of the ordered evaluation draw: item e = g * n_snr + lvl of the (grid window, level) set, in
+// order; the noise pick hashes (seed, g, lvl) only.  Slots past the end of the set are zero-filled and marked -1.
+__global__ void __launch_bounds__(RL_NT) record_enumerate_kernel(rl_enum_args a, int nper, uint64_t n_eval) {
+  pdl_wait();                                     // *counter may have been bumped by the previous eval_reduce_kernel
+  pdl_trigger();
+  const int i = blockIdx.x, tid = threadIdx.x, W = a.W;
+  const uint64_t ctr = a.counter ? (uint64_t)(uint32_t)(*a.counter) : 0ull;
+  const uint64_t e = ctr * (uint64_t)a.world * a.B + (uint64_t)a.rank * a.B + i;
+  if (e >= n_eval) {
+    if (tid == 0) {
+      a.snr_out[i] = 0.f;
+      a.level[i] = -1;
+      if (a.meta)
+        for (int k = 0; k < 4; ++k) a.meta[4 * i + k] = -1;
+    }
+    const size_t per = (size_t)a.leads * W;
+    for (size_t t = tid; t < per; t += RL_NT) {
+      a.clean_out[i * per + t] = 0.f;
+      a.noise_out[i * per + t] = 0.f;
+    }
+    return;
+  }
+  const uint64_t g = e / (uint64_t)a.n_snr;
+  const int lvl = (int)(e % (uint64_t)a.n_snr);
+  const int64_t rec = (int64_t)(g / nper), off = (int64_t)(g % nper) * a.stride;
+  const uint64_t hw = mix64(mix64(a.seed ^ mix64(g)) ^ (uint64_t)lvl);
+  const int64_t nrec = (int64_t)(mix64(hw + 1) % (uint64_t)a.N);
+  const int64_t noff = (int64_t)(mix64(hw + 2) % (uint64_t)(a.Tn - W + 1));
+  if (tid == 0) {
+    a.snr_out[i] = __ldg(a.snr_levels + lvl);
+    a.level[i] = lvl;
+    if (a.meta) {
+      a.meta[4 * i] = (int32_t)rec;
+      a.meta[4 * i + 1] = (int32_t)off;
+      a.meta[4 * i + 2] = (int32_t)nrec;
+      a.meta[4 * i + 3] = (int32_t)noff;
     }
   }
+  copy_window_pair(a, i, tid, W, rec, off, nrec, noff);
 }
 
 }  // namespace
@@ -223,4 +275,29 @@ extern "C" int ralenet_record_sample(const rl_sample_args* a, void* stream) {
              (unsigned long long)n, (long long)a->world * a->B);
   rl_launch_pdl(record_sample_kernel, dim3(a->B), dim3(RL_NT), 0, (cudaStream_t)stream, *a, (int)nper, n, spe);
   return rl_check_launch("record_sample_kernel");
+}
+
+extern "C" int ralenet_record_enumerate(const rl_enum_args* a, void* stream) {
+  RL_REQUIRE(a, RL_ERR_NULL, "record_enumerate: args is NULL");
+  RL_REQUIRE(a->records && a->noise && a->snr_levels && a->clean_out && a->noise_out && a->snr_out && a->level,
+             RL_ERR_NULL, "record_enumerate: NULL tensor");
+  RL_REQUIRE(a->R > 0 && a->leads > 0 && a->leads <= 12 && a->N > 0 && a->B > 0 && a->W > 0 && a->stride > 0 &&
+                 a->n_snr >= 1 && a->W <= a->T && a->W <= a->Tn,
+             RL_ERR_SHAPE,
+             "record_enumerate: unsupported R=%d leads=%d T=%lld N=%d Tn=%lld W=%d stride=%d B=%d n_snr=%d", a->R,
+             a->leads, (long long)a->T, a->N, (long long)a->Tn, a->W, a->stride, a->B, a->n_snr);
+  RL_REQUIRE(a->noise_leads == 1 || a->noise_leads == a->leads, RL_ERR_SHAPE,
+             "record_enumerate: noise_leads=%d must be 1 or leads=%d", a->noise_leads, a->leads);
+  RL_REQUIRE(a->world > 0 && a->rank >= 0 && a->rank < a->world, RL_ERR_SHAPE, "record_enumerate: rank=%d world=%d",
+             a->rank, a->world);
+  RL_REQUIRE(a->T <= INT32_MAX && a->Tn <= INT32_MAX, RL_ERR_SHAPE,
+             "record_enumerate: offsets are int32; T=%lld Tn=%lld", (long long)a->T, (long long)a->Tn);
+  const int64_t nper = (a->T - a->W) / a->stride + 1;
+  const uint64_t grid = (uint64_t)a->R * (uint64_t)nper;                              // < 2^62
+  RL_REQUIRE(grid <= (1ull << 62) / (uint64_t)a->n_snr, RL_ERR_SHAPE,
+             "record_enumerate: %llu grid windows x %d levels overflow the item index", (unsigned long long)grid,
+             a->n_snr);
+  const uint64_t n_eval = grid * (uint64_t)a->n_snr;
+  rl_launch_pdl(record_enumerate_kernel, dim3(a->B), dim3(RL_NT), 0, (cudaStream_t)stream, *a, (int)nper, n_eval);
+  return rl_check_launch("record_enumerate_kernel");
 }

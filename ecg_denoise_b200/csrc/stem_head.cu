@@ -409,6 +409,83 @@ __global__ void __launch_bounds__(RL_NT) mse_kernel(const rl_mse_args a) {
   }
 }
 
+// block-wide fp64 sum in a fixed shuffle / warp order (all RL_NT threads must call); result valid in every thread
+__device__ __forceinline__ double block_sum_f64(double v, double* s_red /* >= 32 doubles */) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  __syncthreads();
+  if (lane == 0) s_red[w] = v;
+  __syncthreads();
+  double r = (lane < (RL_NT >> 5)) ? s_red[lane] : 0.0;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) r += __shfl_xor_sync(0xffffffffu, r, o);
+  return r;
+}
+
+// one CTA per window: (1, snr_in, snr_out, rmse) of local_utils/evaluate.py in fp64 -> partials[b][4]
+__global__ void __launch_bounds__(RL_NT) eval_window_kernel(const rl_eval_args a) {
+  pdl_wait();
+  pdl_trigger();
+  __shared__ double s_red[32];
+  const int b = blockIdx.x, tid = threadIdx.x, per = a.per;
+  double* out = a.partials + 4 * (size_t)b;
+  if (__ldg(a.level + b) < 0) {            // tail slot of the evaluation draw: no window
+    if (tid < 4) out[tid] = 0.0;
+    if (tid == 0) {
+      if (a.snr_in) a.snr_in[b] = 0.f;
+      if (a.snr_out) a.snr_out[b] = 0.f;
+      if (a.rmse) a.rmse[b] = 0.f;
+    }
+    return;
+  }
+  const size_t off = (size_t)b * per;
+  double sy = 0.0, se = 0.0, sn = 0.0;
+  for (int i = tid; i < per; i += RL_NT) {
+    const double y = __ldg(a.clean + off + i);
+    const double e = y - (double)__ldg(a.pred + off + i), n = y - (double)__ldg(a.noisy + off + i);
+    sy = fma(y, y, sy);
+    se = fma(e, e, se);
+    sn = fma(n, n, sn);
+  }
+  sy = block_sum_f64(sy, s_red);
+  se = block_sum_f64(se, s_red);
+  sn = block_sum_f64(sn, s_red);
+  if (tid == 0) {
+    const double snr_in = 10.0 * log10(sy / sn), snr_out = 10.0 * log10(sy / se), rmse = sqrt(se / per);
+    out[0] = 1.0;
+    out[1] = snr_in;
+    out[2] = snr_out;
+    out[3] = rmse;
+    if (a.snr_in) a.snr_in[b] = (float)snr_in;
+    if (a.snr_out) a.snr_out[b] = (float)snr_out;
+    if (a.rmse) a.rmse[b] = (float)rmse;
+  }
+}
+
+// one CTA: acc[l][k] += sum over the windows b of level l of partials[b][k], in a fixed order (thread t takes
+// b = t, t + RL_NT, ... in turn, then block_sum_f64); then the batch counter moves on
+__global__ void __launch_bounds__(RL_NT) eval_reduce_kernel(const rl_eval_args a) {
+  pdl_wait();
+  pdl_trigger();
+  __shared__ double s_red[32];
+  for (int l = 0; l < a.n_snr; ++l) {
+    double s[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int b = threadIdx.x; b < a.B; b += RL_NT) {
+      if (__ldg(a.level + b) != l) continue;
+      const double* p = a.partials + 4 * (size_t)b;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) s[k] += p[k];
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const double v = block_sum_f64(s[k], s_red);
+      if (threadIdx.x == 0) a.acc[4 * l + k] += v;
+    }
+  }
+  if (threadIdx.x == 0 && a.counter) *a.counter += 1;
+}
+
 // ---------------------------------------------------------------------------------------------
 // generic small Conv1d ('same', odd K) for the 12-lead wrapper; one CTA per window.
 constexpr int CONV_MAX_CI = 12, CONV_MAX_K = 13;
@@ -651,6 +728,19 @@ extern "C" int ralenet_mse(const rl_mse_args* a, void* stream) {
   RlDet det = {a->partials, (size_t)((a->B + 3) & ~3), 0, {}, 0};     // the per-window sums, added in window order
   rl_det_take(&det, a->loss, 1, a->B);
   return rl_launch_grad_reduce(&det, st);
+}
+
+extern "C" int ralenet_eval_metrics(const rl_eval_args* a, void* stream) {
+  RL_REQUIRE(a, RL_ERR_NULL, "eval_metrics: args is NULL");
+  RL_REQUIRE(a->B > 0 && a->per > 0 && a->n_snr >= 1, RL_ERR_SHAPE, "eval_metrics: B=%d per=%d n_snr=%d", a->B, a->per,
+             a->n_snr);
+  RL_REQUIRE(a->clean && a->noisy && a->pred && a->level && a->partials && a->acc, RL_ERR_NULL,
+             "eval_metrics: NULL tensor");
+  const cudaStream_t st = (cudaStream_t)stream;
+  rl_launch_pdl(eval_window_kernel, dim3(a->B), dim3(RL_NT), 0, st, *a);
+  if (int rc = rl_check_launch("eval_window_kernel")) return rc;
+  rl_launch_pdl(eval_reduce_kernel, dim3(1), dim3(RL_NT), 0, st, *a);
+  return rl_check_launch("eval_reduce_kernel");
 }
 
 // tensor-core implicit-GEMM path for the k = 13 layers of newrale (conv_mma.cu)

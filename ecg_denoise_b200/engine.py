@@ -287,13 +287,17 @@ class _WsLease:
 
     def __del__(self):
         try:
-            if len(self.pool) < 4:
+            if self.pool is not None and len(self.pool) < 4:
                 self.pool.append(self.buf)
         except Exception:      # noqa: BLE001 -- interpreter shutdown
             pass
 
 
 def _lease_ws(plan: NetPlan, nbytes: int, device) -> _WsLease:
+    if torch.cuda.is_current_stream_capturing():
+        # a captured forward keeps using its workspace at every replay, on whatever stream the graph is launched:
+        # the buffer (from the graph's private pool) must never be handed to another forward
+        return _WsLease(torch.empty(nbytes, device=device, dtype=torch.uint8), None)
     # one pool per (plan, stream): a returned buffer is only handed to work enqueued on the same stream, which
     # orders the reuse after the kernels that last touched it
     pool = plan.__dict__.setdefault("_ws_pools", {}).setdefault((str(device), _stream()), [])

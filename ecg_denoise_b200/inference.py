@@ -7,6 +7,7 @@ z-normalisation, the batched eval-mode forward and an overlap-add stitch with ha
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 from typing import Optional
 
@@ -56,6 +57,24 @@ def windows_to_records(win: torch.Tensor, x: torch.Tensor, stats: Optional[torch
     return y
 
 
+@contextlib.contextmanager
+def precision_scope(model, precision: Optional[str]):
+    """for the body: with precision "fp32" or "tf32", that inference_precision on every RA-LENet module inside `model`
+    (e.g. the core of a 12-lead `newrale`), restored afterwards; None changes nothing."""
+    from .model._blocks import _RalenetBase
+    cores = []
+    if precision is not None:
+        check_precision(precision)
+        cores = [(m, m.inference_precision) for m in model.modules() if isinstance(m, _RalenetBase)]
+    try:
+        for m, _ in cores:
+            m.inference_precision = precision
+        yield
+    finally:
+        for m, p in cores:
+            m.inference_precision = p
+
+
 @torch.no_grad()
 def denoise_records(model, records: torch.Tensor, window: int = 256, stride: int = 256, batch: int = 8192,
                     znorm: bool = True, stitch: bool = True, precision: Optional[str] = None):
@@ -64,22 +83,14 @@ def denoise_records(model, records: torch.Tensor, window: int = 256, stride: int
     its own slice of the records -- no communication is needed.
     precision: None keeps the inference_precision of every RA-LENet module inside `model`; "fp32" or "tf32" sets it
     on all of them (e.g. the core of a 12-lead `newrale`) for this call and restores it afterwards."""
-    from .model._blocks import _RalenetBase
-    cores = []
-    if precision is not None:
-        check_precision(precision)
-        cores = [(m, m.inference_precision) for m in model.modules() if isinstance(m, _RalenetBase)]
     was_training = model.training
-    model.eval()
-    try:
-        for m, _ in cores:
-            m.inference_precision = precision
-        win, stats = records_to_windows(records, window, stride, znorm)
-        out = torch.empty_like(win)
-        for i in range(0, win.shape[0], batch):
-            out[i:i + batch] = model(win[i:i + batch])
-        return windows_to_records(out, records, stats, stride) if stitch else out
-    finally:
-        model.train(was_training)
-        for m, p in cores:
-            m.inference_precision = p
+    with precision_scope(model, precision):
+        model.eval()
+        try:
+            win, stats = records_to_windows(records, window, stride, znorm)
+            out = torch.empty_like(win)
+            for i in range(0, win.shape[0], batch):
+                out[i:i + batch] = model(win[i:i + batch])
+            return windows_to_records(out, records, stats, stride) if stitch else out
+        finally:
+            model.train(was_training)

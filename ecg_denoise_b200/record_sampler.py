@@ -34,14 +34,86 @@ def steps_per_epoch(R: int, T: int, window: int, stride: int, batch: int, world:
     return R * windows_per_record(T, window, stride) // (world * batch)
 
 
-def _bank(t, name: str) -> torch.Tensor:
+def _bank(t, name: str, who: str) -> torch.Tensor:
     if not isinstance(t, torch.Tensor) or t.dim() != 3:
-        raise ValueError(f"RecordSampler: {name} must be a 3-D tensor (records, leads, samples), "
+        raise ValueError(f"{who}: {name} must be a 3-D tensor (records, leads, samples), "
                          f"got {getattr(t, 'shape', type(t).__name__)}")
     return t
 
 
-class RecordSampler:
+class _RecordBanks:
+    """What the device batch sources over a clean and a noise record bank share: argument checks (ValueError for
+    shapes and values, before any device work; RalenetError for placement), the per-(record, lead) z-normalisation
+    statistics, the level table, the per-slot noise / level / meta buffers and the C argument struct, whose bank fields
+    rl_sample_args and rl_enum_args have in common.  Subclasses name themselves in _WHO (for messages) and check the
+    size of the grid in _check_grid."""
+    _WHO: str
+
+    def __init__(self, struct: str, records, noise, batch, window, stride, snr_db, znorm, seed, rank, world):
+        who = self._WHO
+        records, noise = _bank(records, "records", who), _bank(noise, "noise", who)
+        R, leads, T = records.shape
+        N, noise_leads, Tn = noise.shape
+        stride = window if stride is None else stride
+        levels = [float(snr_db)] if isinstance(snr_db, (int, float)) else [float(s) for s in snr_db]
+        if world is None or rank is None:
+            dist = torch.distributed.is_available() and torch.distributed.is_initialized()
+            world = (torch.distributed.get_world_size() if dist else 1) if world is None else world
+            rank = (torch.distributed.get_rank() if dist else 0) if rank is None else rank
+        batch, window, stride, world, rank = int(batch), int(window), int(stride), int(world), int(rank)
+        if not 1 <= leads <= 12:
+            raise ValueError(f"{who}: records have {leads} leads; 1 to 12 are supported")
+        if noise_leads not in (1, leads):
+            raise ValueError(f"{who}: noise has {noise_leads} leads; it needs 1 or {leads} (as the records)")
+        if batch < 1 or window < 1 or stride < 1:
+            raise ValueError(f"{who}: batch={batch}, window={window}, stride={stride} must be positive")
+        if window > T or window > Tn:
+            raise ValueError(f"{who}: window {window} is longer than the records ({T}) or the noise ({Tn})")
+        if not levels:
+            raise ValueError(f"{who}: snr_db needs at least one level")
+        if not 0 <= rank < world:
+            raise ValueError(f"{who}: rank {rank} is not in [0, world={world})")
+        self._check_grid(R, windows_per_record(T, window, stride), levels, batch, world)
+        for t, name in ((records, "records"), (noise, "noise")):
+            if not t.is_cuda:
+                raise _lib.RalenetError(f"{who}: {name} is on {t.device}; the banks are read on a CUDA B200 device "
+                                        "(no CPU fallback)")
+            if t.dtype != torch.float32:
+                raise _lib.RalenetError(f"{who}: {name} has dtype {t.dtype}; the kernel reads float32")
+            if not t.is_contiguous():
+                raise _lib.RalenetError(f"{who}: {name} must be contiguous (it is read in place)")
+        if noise.device != records.device:
+            raise _lib.RalenetError(f"{who}: noise is on {noise.device}, records on {records.device}")
+        self.device = records.device
+        _lib.check_device(self.device.index if self.device.index is not None else torch.cuda.current_device())
+
+        self.records, self.noise_bank = records, noise
+        self.B, self.leads, self.L, self.stride, self.seed = batch, leads, window, stride, int(seed)
+        self.rank, self.world = rank, world
+        self.snr_levels = torch.tensor(levels, device=self.device, dtype=torch.float32)
+        lib = _lib.load()
+        self.stats = None
+        if znorm:
+            self.stats = torch.empty(R * leads, 2, device=self.device, dtype=torch.float32)
+            _lib.check(lib.ralenet_record_stats(ctypes.c_void_p(records.data_ptr()), R * leads, ctypes.c_int64(T),
+                                                ctypes.c_void_p(self.stats.data_ptr()), ctypes.c_void_p(_stream())))
+        self.noise = torch.empty(batch, leads, window, device=self.device, dtype=torch.float32)
+        self.snr = torch.empty(batch, device=self.device, dtype=torch.float32)
+        self.meta = torch.empty(batch, 4, device=self.device, dtype=torch.int32)
+        a = _lib.STRUCTS[struct]()
+        a.records, a.noise, a.snr_levels = records.data_ptr(), noise.data_ptr(), self.snr_levels.data_ptr()
+        a.stats = self.stats.data_ptr() if self.stats is not None else None
+        a.noise_out, a.snr_out, a.meta = self.noise.data_ptr(), self.snr.data_ptr(), self.meta.data_ptr()
+        a.T, a.Tn, a.seed = T, Tn, self.seed & 0xFFFFFFFFFFFFFFFF
+        a.R, a.leads, a.N, a.noise_leads, a.n_snr = R, leads, N, noise_leads, len(levels)
+        a.W, a.stride, a.B, a.rank, a.world = window, stride, batch, rank, world
+        self._args = a
+
+    def _check_grid(self, R: int, nper: int, levels: list, batch: int, world: int) -> None:
+        raise NotImplementedError
+
+
+class RecordSampler(_RecordBanks):
     """Training windows drawn on the device from a bank of clean records and a bank of noise records.
 
     records: (R, leads, T) CUDA fp32 contiguous, leads <= 12; noise: (N, noise_leads, Tn) on the same device,
@@ -55,70 +127,19 @@ class RecordSampler:
     `meta` (batch, 4) int32 holds (record, offset, noise record, noise offset) per window and `snr` (batch,) the
     drawn levels in dB.
     """
+    _WHO = "RecordSampler"
 
     def __init__(self, records: torch.Tensor, noise: torch.Tensor, batch: int, window: int = 256,
                  stride: Optional[int] = None, snr_db: Union[float, Sequence[float]] = (-4, -2, 0, 2, 4),
                  znorm: bool = True, seed: int = 2023, rank: Optional[int] = None, world: Optional[int] = None):
-        records, noise = _bank(records, "records"), _bank(noise, "noise")
-        R, leads, T = records.shape
-        N, noise_leads, Tn = noise.shape
-        stride = window if stride is None else stride
-        levels = [float(snr_db)] if isinstance(snr_db, (int, float)) else [float(s) for s in snr_db]
-        if world is None or rank is None:
-            dist = torch.distributed.is_available() and torch.distributed.is_initialized()
-            world = (torch.distributed.get_world_size() if dist else 1) if world is None else world
-            rank = (torch.distributed.get_rank() if dist else 0) if rank is None else rank
-        batch, window, stride, world, rank = int(batch), int(window), int(stride), int(world), int(rank)
-        if not 1 <= leads <= 12:
-            raise ValueError(f"RecordSampler: records have {leads} leads; 1 to 12 are supported")
-        if noise_leads not in (1, leads):
-            raise ValueError(f"RecordSampler: noise has {noise_leads} leads; it needs 1 or {leads} (as the records)")
-        if batch < 1 or window < 1 or stride < 1:
-            raise ValueError(f"RecordSampler: batch={batch}, window={window}, stride={stride} must be positive")
-        if window > T or window > Tn:
-            raise ValueError(f"RecordSampler: window {window} is longer than the records ({T}) or the noise ({Tn})")
-        if not levels:
-            raise ValueError("RecordSampler: snr_db needs at least one level")
-        if not 0 <= rank < world:
-            raise ValueError(f"RecordSampler: rank {rank} is not in [0, world={world})")
-        spe = steps_per_epoch(R, T, window, stride, batch, world)
-        if spe == 0:
-            raise ValueError(f"RecordSampler: the grid has {R * windows_per_record(T, window, stride)} windows, fewer "
-                             f"than one world batch of {world} x {batch}")
-        for t, name in ((records, "records"), (noise, "noise")):
-            if not t.is_cuda:
-                raise _lib.RalenetError(f"RecordSampler: {name} is on {t.device}; the sampler reads its banks on a "
-                                        "CUDA B200 device (no CPU fallback)")
-            if t.dtype != torch.float32:
-                raise _lib.RalenetError(f"RecordSampler: {name} has dtype {t.dtype}; the kernel reads float32")
-            if not t.is_contiguous():
-                raise _lib.RalenetError(f"RecordSampler: {name} must be contiguous (it is read in place)")
-        if noise.device != records.device:
-            raise _lib.RalenetError(f"RecordSampler: noise is on {noise.device}, records on {records.device}")
-        self.device = records.device
-        _lib.check_device(self.device.index if self.device.index is not None else torch.cuda.current_device())
+        super().__init__("rl_sample_args", records, noise, batch, window, stride, snr_db, znorm, seed, rank, world)
 
-        self.records, self.noise_bank = records, noise
-        self.B, self.leads, self.L, self.stride, self.seed = batch, leads, window, stride, int(seed)
-        self.rank, self.world, self.steps_per_epoch = rank, world, spe
-        self.snr_levels = torch.tensor(levels, device=self.device, dtype=torch.float32)
-        lib = _lib.load()
-        self.stats = None
-        if znorm:
-            self.stats = torch.empty(R * leads, 2, device=self.device, dtype=torch.float32)
-            _lib.check(lib.ralenet_record_stats(ctypes.c_void_p(records.data_ptr()), R * leads, ctypes.c_int64(T),
-                                                ctypes.c_void_p(self.stats.data_ptr()), ctypes.c_void_p(_stream())))
-        self.noise = torch.empty(batch, leads, window, device=self.device, dtype=torch.float32)
-        self.snr = torch.empty(batch, device=self.device, dtype=torch.float32)
-        self.meta = torch.empty(batch, 4, device=self.device, dtype=torch.int32)
-        a = _lib.STRUCTS["rl_sample_args"]()
-        a.records, a.noise, a.snr_levels = records.data_ptr(), noise.data_ptr(), self.snr_levels.data_ptr()
-        a.stats = self.stats.data_ptr() if self.stats is not None else None
-        a.noise_out, a.snr_out, a.meta = self.noise.data_ptr(), self.snr.data_ptr(), self.meta.data_ptr()
-        a.T, a.Tn, a.seed = T, Tn, self.seed & 0xFFFFFFFFFFFFFFFF
-        a.R, a.leads, a.N, a.noise_leads, a.n_snr = R, leads, N, noise_leads, len(levels)
-        a.W, a.stride, a.B, a.rank, a.world = window, stride, batch, rank, world
-        self._args = a
+    def _check_grid(self, R, nper, levels, batch, world):
+        spe = R * nper // (world * batch)
+        if spe == 0:
+            raise ValueError(f"RecordSampler: the grid has {R * nper} windows, fewer than one world batch of "
+                             f"{world} x {batch}")
+        self.steps_per_epoch = spe
 
     def _counter(self, counter) -> Optional[torch.Tensor]:
         if counter is None or isinstance(counter, torch.Tensor):

@@ -442,6 +442,47 @@ typedef struct {
 } rl_sample_args;
 int ralenet_record_sample(const rl_sample_args* a, void* stream);
 
+/* Ordered evaluation draw over held-out banks (records.cu), the device side of the per-epoch test loop
+ * (denoise_train.py:66-81 over the test loader; the reference's test sets are one noisy copy per intensity,
+ * dict_data/{m4,m2,0,p2,p4}).  Same banks, statistics, outputs and layouts as rl_sample_args; one CTA per slot.
+ * The evaluation set is every grid window at every level: item e = g * n_snr + lvl, g = record * nper + k the grid
+ * window in record-major order (the order of ralenet_window_gather), n_eval = R * nper * n_snr items.  With
+ * c = *counter (0 when NULL), slot i of rank r takes e = c * world * B + r * B + i: no shuffle, no drop-last, and the
+ * ranks together cover the set exactly once.  Noise record and noise offset are hashed from (seed, g, lvl) alone, so
+ * every run, epoch and rank split sees the same noisy test set.  A slot with e >= n_eval writes zeroed clean and noise
+ * windows, snr_out = 0, meta = (-1, -1, -1, -1) and level = -1.  level [B]: level index of the slot (valid = level >= 0).
+ * Mix with ralenet_snr_mix.  Offsets must fit int32 (T, Tn <= INT32_MAX), like meta. */
+typedef struct {
+  const float* records; const float* stats; const float* noise; const float* snr_levels;
+  const int32_t* counter;
+  float* clean_out; float* noise_out; float* snr_out;
+  int32_t* meta; int32_t* level;
+  int64_t T, Tn;
+  uint64_t seed;
+  int32_t R, leads, N, noise_leads, n_snr, W, stride, B, rank, world;
+} rl_enum_args;
+int ralenet_record_enumerate(const rl_enum_args* a, void* stream);
+
+/* Evaluation metrics of one batch (local_utils/evaluate.py:27-29, 49-51 per window, summed per level as
+ * denoise_train.py:100-101 reports them).  For window b with level[b] >= 0, over all `per` elements (leads x samples),
+ * in fp64:  snr_out = 10 log10(sum y^2 / sum (y - pred)^2),  snr_in = the same with noisy in place of pred,
+ * rmse = sqrt(mean((y - pred)^2)), y = clean.  Optional per-window outputs snr_in / snr_out / rmse [B] (float; 0 for
+ * windows with level < 0).  acc [n_snr][4] += (count, sum snr_in, sum snr_out, sum rmse) per level: the windows'
+ * values go through partials [B][4] (fp64 scratch) and one CTA adds them in a fixed order, so the whole evaluation
+ * is bit-reproducible (no floating-point atomics).  Windows with level < 0 or >= n_snr add nothing.  counter (device
+ * int32, may be NULL) is incremented after the sums, so a captured draw + forward + metrics step advances by itself
+ * (as ralenet_adam_dev does with the step count). */
+typedef struct {
+  const float* clean; const float* noisy; const float* pred;   /* [B][per] each                            */
+  const int32_t* level;                                        /* [B]                                      */
+  float* snr_in; float* snr_out; float* rmse;                  /* [B] each or NULL                         */
+  double* partials;                                            /* [B][4] scratch                           */
+  double* acc;                                                 /* [n_snr][4] (+=)                          */
+  int32_t* counter;                                            /* or NULL                                  */
+  int32_t B, per, n_snr, _pad;
+} rl_eval_args;
+int ralenet_eval_metrics(const rl_eval_args* a, void* stream);
+
 /* Weight-gradient GEMM over the token dimension (used by every *_bwd above; exported for benchmarks):
  *   dW[n*K + k] += sum_m dY[m*ldy + n] * X[m*ldx + k],   db[n] += sum_m dY[m*ldy + n]   (db may be NULL) */
 int ralenet_wgrad(const float* dY, int32_t ldy, const float* X, int32_t ldx, int32_t M, int32_t N, int32_t K,
