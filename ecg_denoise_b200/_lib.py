@@ -113,6 +113,9 @@ def load():
     lib.ralenet_pconv1.argtypes = [P, P, P, I, I, I, I, P]
     lib.ralenet_pconv1_wgrad.argtypes = [P, P, P, I, I, I, P]
     lib.ralenet_wgrad.argtypes = [P, I, P, I, I, I, I, P, P, P]
+    lib.ralenet_conv1d_slab_bytes.restype = ctypes.c_uint64
+    lib.ralenet_conv1d_slab_bytes.argtypes = [I] * 4
+    lib.ralenet_conv1d_bwd_det.argtypes = [P, P, ctypes.c_uint64, P]
     lib.ralenet_synth_windows.argtypes = [P, P, I, I, I, ctypes.c_uint64, P, I, P]
     lib.ralenet_comm_bytes.restype = ctypes.c_uint64
     lib.ralenet_comm_bytes.argtypes = [ctypes.c_uint64]
@@ -142,8 +145,9 @@ def deterministic_guard(what: str) -> None:
     if not torch.are_deterministic_algorithms_enabled():
         return
     msg = (f"{what} does not have a deterministic implementation, but you set "
-           "'torch.use_deterministic_algorithms(True)'. The whole-network paths (ralenet modules, FusedTrainer on one "
-           "GPU) are deterministic under that flag; see INTEGRATION.md section 4.")
+           "'torch.use_deterministic_algorithms(True)'. The whole-network paths (ralenet and newrale modules, "
+           "FusedTrainer and FineTuneTrainer on one GPU) are deterministic under that flag; see INTEGRATION.md "
+           "section 4.")
     if torch.is_deterministic_algorithms_warn_only_enabled():
         import warnings
         warnings.warn(msg)

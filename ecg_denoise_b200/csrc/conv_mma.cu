@@ -143,7 +143,9 @@ __global__ void __launch_bounds__(RL_NT) conv13_fwd_mma_kernel(const rl_conv_fwd
   }
 }
 
-template <int NTO, int NTI>     // column tiles of the forward GEMM (Cout) and of the dgrad GEMM (Cin)
+// DET: d_w / d_b are partial slabs [B][Cout*Cin*13] / [B][Cout] (grad_add): every element of a window's dW is one
+// element of one warp tile, every element of its db the sum of one warp, so the slot of a CTA is its window
+template <int NTO, int NTI, bool DET>     // column tiles of the forward GEMM (Cout) and of the dgrad GEMM (Cin)
 __global__ void __launch_bounds__(RL_NT) conv13_bwd_mma_kernel(const rl_conv_bwd_args a) {
   extern __shared__ __align__(16) float smem[];
   const int L = a.L, Ci = a.Cin, Co = a.Cout, LP = L + 2 * PAD;
@@ -204,6 +206,7 @@ __global__ void __launch_bounds__(RL_NT) conv13_bwd_mma_kernel(const rl_conv_bwd
 
   // 3. wgrad: dW[o][(i,k)] += sum_t dc[o][t] x[i][t+k-6]: one 16 x 8 tile of dW per warp step, K = L
   if (a.d_w) {
+    float* const d_w = grad_slot<DET>(a.d_w, (size_t)Co * Kt, blockIdx.x);
     for (int nt = warp; nt < KP / 8; nt += RL_NT / 32) {
       float acc[4] = {0.f, 0.f, 0.f, 0.f};
       const int ob = s.offA[nt * 8 + g];                    // B(k = t', n = (i,k)) = x[i][t' + k]
@@ -219,17 +222,19 @@ __global__ void __launch_bounds__(RL_NT) conv13_bwd_mma_kernel(const rl_conv_bwd
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         const int o = g + (e >> 1) * 8, n = nt * 8 + 2 * t + (e & 1);
-        if (o < Co && n < Kt) atomicAdd(a.d_w + o * Kt + n, acc[e]);
+        if (o < Co && n < Kt) grad_add<DET>(d_w + o * Kt + n, acc[e]);
       }
     }
-    if (a.d_b)
+    if (a.d_b) {
+      float* const d_b = grad_slot<DET>(a.d_b, Co, blockIdx.x);
       for (int o = warp; o < Co; o += RL_NT / 32) {
         float sum = 0.f;
         for (int m = lane; m < L; m += 32) sum += s.sdc[o * LP + PAD + m];
 #pragma unroll
         for (int sft = 16; sft > 0; sft >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, sft);
-        if (lane == 0) atomicAdd(a.d_b + o, sum);
+        if (lane == 0) grad_add<DET>(d_b + o, sum);
       }
+    }
   }
 }
 
@@ -267,19 +272,22 @@ int rl_conv13_fwd_mma(const rl_conv_fwd_args* a, cudaStream_t st) {
   return rl_check_launch("conv13_fwd_mma_kernel", a->Cin, a->Cout);
 }
 
-template <int NTO, int NTI>
+template <int NTO, int NTI, bool DET>
 static int launch_bwd(const rl_conv_bwd_args* a, size_t smem, cudaStream_t st) {
-  if (int rc = rl_set_smem(conv13_bwd_mma_kernel<NTO, NTI>, smem)) return rc;
-  conv13_bwd_mma_kernel<NTO, NTI><<<a->B, RL_NT, smem, st>>>(*a);
+  if (int rc = rl_set_smem(conv13_bwd_mma_kernel<NTO, NTI, DET>, smem)) return rc;
+  conv13_bwd_mma_kernel<NTO, NTI, DET><<<a->B, RL_NT, smem, st>>>(*a);
   return RL_OK;
 }
 
-int rl_conv13_bwd_mma(const rl_conv_bwd_args* a, cudaStream_t st) {
+template <bool DET>
+static int launch_bwd(const rl_conv_bwd_args* a, size_t smem, cudaStream_t st) {
+  if (a->Cout <= 8) return a->Cin <= 8 ? launch_bwd<1, 1, DET>(a, smem, st) : launch_bwd<1, 2, DET>(a, smem, st);
+  return a->Cin <= 8 ? launch_bwd<2, 1, DET>(a, smem, st) : launch_bwd<2, 2, DET>(a, smem, st);
+}
+
+int rl_conv13_bwd_mma(const rl_conv_bwd_args* a, cudaStream_t st, bool det) {
   const size_t smem = sizeof(float) * smem_floats(a->L, a->Cin, true);
   rl_prof_pre(st);
-  int rc;
-  if (a->Cout <= 8) rc = a->Cin <= 8 ? launch_bwd<1, 1>(a, smem, st) : launch_bwd<1, 2>(a, smem, st);
-  else rc = a->Cin <= 8 ? launch_bwd<2, 1>(a, smem, st) : launch_bwd<2, 2>(a, smem, st);
-  if (rc) return rc;
+  if (int rc = det ? launch_bwd<true>(a, smem, st) : launch_bwd<false>(a, smem, st)) return rc;
   return rl_check_launch("conv13_bwd_mma_kernel", a->Cin, a->Cout);
 }

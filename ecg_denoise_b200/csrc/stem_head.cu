@@ -516,6 +516,9 @@ __global__ void __launch_bounds__(RL_NT) conv1d_fwd_kernel(const rl_conv_fwd_arg
   }
 }
 
+// DET: d_w / d_b are partial slabs [B][Cout*Cin*K] / [B][Cout] (grad_add); one thread sums each element of a
+// window's dW and db, so the slot of a CTA is its window
+template <bool DET>
 __global__ void __launch_bounds__(RL_NT) conv1d_bwd_kernel(const rl_conv_bwd_args a) {
   extern __shared__ __align__(16) float smem[];
   const int L = a.L, Ci = a.Cin, Co = a.Cout, K = a.K, pad = a.K / 2, LP = L + 2 * pad;
@@ -561,20 +564,23 @@ __global__ void __launch_bounds__(RL_NT) conv1d_bwd_kernel(const rl_conv_bwd_arg
     }
   }
   if (a.d_w) {  // dW[o][i][k] += sum_t dc[o][t] x[i][t+k-pad]
+    float* const d_w = grad_slot<DET>(a.d_w, (size_t)Co * Ci * K, blockIdx.x);
     for (int idx = tid; idx < Co * Ci * K; idx += RL_NT) {
       const int k = idx % K, i = (idx / K) % Ci, o = idx / (K * Ci);
       const float* dr = sdc + o * LP + pad;
       const float* xr = sx + i * LP + k;
       float s = 0.f;
       for (int t = 0; t < L; ++t) s = fmaf(dr[t], xr[t], s);
-      atomicAdd(a.d_w + idx, s);
+      grad_add<DET>(d_w + idx, s);
     }
-    if (a.d_b)
+    if (a.d_b) {
+      float* const d_b = grad_slot<DET>(a.d_b, Co, blockIdx.x);
       for (int o = tid; o < Co; o += RL_NT) {
         float s = 0.f;
         for (int t = 0; t < L; ++t) s += sdc[o * LP + pad + t];
-        atomicAdd(a.d_b + o, s);
+        grad_add<DET>(d_b + o, s);
       }
+    }
   }
 }
 
@@ -746,7 +752,7 @@ extern "C" int ralenet_eval_metrics(const rl_eval_args* a, void* stream) {
 // tensor-core implicit-GEMM path for the k = 13 layers of newrale (conv_mma.cu)
 bool rl_conv13_eligible(int L, int Ci, int Co, int K);
 int rl_conv13_fwd_mma(const rl_conv_fwd_args* a, cudaStream_t st);
-int rl_conv13_bwd_mma(const rl_conv_bwd_args* a, cudaStream_t st);
+int rl_conv13_bwd_mma(const rl_conv_bwd_args* a, cudaStream_t st, bool det);
 
 static int conv_check(int B, int L, int Ci, int Co, int K, size_t* smem, bool bwd) {
   RL_REQUIRE(B > 0 && L > 0 && L <= 8192 && Ci > 0 && Co > 0 && Ci <= CONV_MAX_CI && Co <= CONV_MAX_CI && K % 2 == 1 &&
@@ -770,16 +776,45 @@ extern "C" int ralenet_conv1d_fwd(const rl_conv_fwd_args* a, void* stream) {
   return rl_check_launch("conv1d_fwd_kernel");
 }
 
+template <bool DET>
+static int conv1d_bwd_launch(const rl_conv_bwd_args* a, size_t smem, cudaStream_t st) {
+  if (rl_conv13_eligible(a->L, a->Cin, a->Cout, a->K)) return rl_conv13_bwd_mma(a, st, DET);
+  if (int rc = rl_set_smem(conv1d_bwd_kernel<DET>, smem)) return rc;
+  rl_prof_pre(st);
+  conv1d_bwd_kernel<DET><<<a->B, RL_NT, smem, st>>>(*a);
+  return rl_check_launch("conv1d_bwd_kernel");
+}
+
 extern "C" int ralenet_conv1d_bwd(const rl_conv_bwd_args* a, void* stream) {
   RL_REQUIRE(a, RL_ERR_NULL, "conv1d_bwd: args is NULL");
   size_t smem = 0;
   if (int rc = conv_check(a->B, a->L, a->Cin, a->Cout, a->K, &smem, true)) return rc;
   RL_REQUIRE(a->dy && a->x && a->w, RL_ERR_NULL, "conv1d_bwd: NULL tensor");
-  if (rl_conv13_eligible(a->L, a->Cin, a->Cout, a->K)) return rl_conv13_bwd_mma(a, (cudaStream_t)stream);
-  if (int rc = rl_set_smem(conv1d_bwd_kernel, smem)) return rc;
-  rl_prof_pre((cudaStream_t)stream);
-  conv1d_bwd_kernel<<<a->B, RL_NT, smem, (cudaStream_t)stream>>>(*a);
-  return rl_check_launch("conv1d_bwd_kernel");
+  return conv1d_bwd_launch<false>(a, smem, (cudaStream_t)stream);
+}
+
+extern "C" uint64_t ralenet_conv1d_slab_bytes(int32_t B, int32_t Cin, int32_t Cout, int32_t K) {
+  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0) return 0;
+  const uint64_t nw = (uint64_t)B * Cout * Cin * K, nb = (uint64_t)B * Cout;   // rl_det_take's 16-byte rounding
+  return sizeof(float) * (((nw + 3) & ~(uint64_t)3) + ((nb + 3) & ~(uint64_t)3));
+}
+
+extern "C" int ralenet_conv1d_bwd_det(const rl_conv_bwd_args* a, float* slab, uint64_t slab_bytes, void* stream) {
+  RL_REQUIRE(a, RL_ERR_NULL, "conv1d_bwd_det: args is NULL");
+  size_t smem = 0;
+  if (int rc = conv_check(a->B, a->L, a->Cin, a->Cout, a->K, &smem, true)) return rc;
+  RL_REQUIRE(a->dy && a->x && a->w && slab, RL_ERR_NULL, "conv1d_bwd_det: NULL tensor or slab");
+  const uint64_t need = ralenet_conv1d_slab_bytes(a->B, a->Cin, a->Cout, a->K);
+  RL_REQUIRE(slab_bytes >= need, RL_ERR_SHAPE, "conv1d_bwd_det: slab of %llu bytes, %llu needed",
+             (unsigned long long)slab_bytes, (unsigned long long)need);
+  const cudaStream_t st = (cudaStream_t)stream;
+  RlDet det = {slab, (size_t)(slab_bytes / sizeof(float)), 0, {}, 0};
+  rl_conv_bwd_args d = *a;                     // one partial slot per window (CTA)
+  d.d_w = rl_det_take(&det, a->d_w, (size_t)a->Cout * a->Cin * a->K, a->B);
+  d.d_b = a->d_w ? rl_det_take(&det, a->d_b, a->Cout, a->B) : nullptr;   // the kernels write d_b only with d_w
+  RL_REQUIRE(rl_det_ok(&det), RL_ERR_SHAPE, "conv1d_bwd_det: slab too small");
+  if (int rc = conv1d_bwd_launch<true>(&d, smem, st)) return rc;
+  return rl_launch_grad_reduce(&det, st);
 }
 
 extern "C" int ralenet_adam(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1,

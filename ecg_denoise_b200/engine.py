@@ -761,13 +761,22 @@ class FineTuneTrainer(_HostPipeline):
     pre-allocated buffers -- no autograd graph, no per-tensor optimizer, one flat Adam -- so the whole step
     (forward, loss + metrics, data gradients through the frozen core, conv weight gradients, Adam) replays from ONE
     CUDA graph.  The core stays in whatever mode `model.rale.training` says (model.train() puts its BatchNorm in
-    batch-statistics mode and updates its running statistics, exactly like the reference's frozen core)."""
+    batch-statistics mode and updates its running statistics, exactly like the reference's frozen core).
+
+    deterministic: True = bit-reproducible steps (loss, gradients, BatchNorm sums, Adam trajectory): the frozen core
+    runs its RL_NET_DETERMINISTIC backward, the loss is summed in window order and the four convolutions write their
+    weight gradients to per-window partial slabs reduced in window order (ralenet_conv1d_bwd_det); None = follow
+    torch.are_deterministic_algorithms_enabled() at construction."""
 
     def __init__(self, model: nn.Module, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8,
-                 use_graph: bool = False):
+                 use_graph: bool = False, deterministic: Optional[bool] = None):
         from . import ops
         self.ops, self.model, self.core = ops, model, model.rale
         self.lr, self.betas, self.eps, self.use_graph = lr, betas, eps, use_graph
+        if deterministic is None:
+            deterministic = torch.are_deterministic_algorithms_enabled()
+        self.deterministic = bool(deterministic)
+        self.net_flags = _lib.RL_NET_DETERMINISTIC if self.deterministic else 0
         self.convs = [model.conv1, model.conv2, model.conv3, model.conv4]
         self.slope = float(model.relu.negative_slope)
         self.flat = None
@@ -807,7 +816,15 @@ class FineTuneTrainer(_HostPipeline):
         self._x, self._t = f(Cin), f(Cin)
         self._a1, self._a2, self._r, self._a3, self._out = f(6), f(2), f(2), f(6), f(Cin)
         self._da3, self._dr, self._da2, self._da1 = f(6), f(2), f(2), f(6)
-        self._ws = torch.empty(workspace_bytes(B, L, True), device=device, dtype=torch.uint8)
+        self._ws = torch.empty(workspace_bytes(B, L, True, self.net_flags), device=device, dtype=torch.uint8)
+        self._loss_partials = self._slabs = None
+        if self.deterministic:
+            self._loss_partials = torch.empty(B, device=device, dtype=torch.float32)
+            # one slab per layer: no reuse between the four backward calls, whatever their launch order
+            self._slabs = {}
+            for c in self.convs:
+                Co, Ci, K = c.weight.shape
+                self._slabs[id(c)] = self.ops.conv1d_slab(B, Ci, Co, K, device)
         self._shape = tuple(shape)
         self.graph = None
 
@@ -825,7 +842,10 @@ class FineTuneTrainer(_HostPipeline):
         a.dy, a.x, a.w, a.b = dy.data_ptr(), x.data_ptr(), conv.weight.data_ptr(), conv.bias.data_ptr()
         a.dx = dx.data_ptr() if dx is not None else None
         a.d_w, a.d_b = conv.weight.grad.data_ptr(), conv.bias.grad.data_ptr()
-        _lib.call("ralenet_conv1d_bwd", a, _stream())
+        if self._slabs is not None:
+            self.ops.conv1d_bwd_det(a, self._slabs[id(conv)])
+        else:
+            _lib.call("ralenet_conv1d_bwd", a, _stream())
 
     def _step_impl(self):
         plan: NetPlan = self.core._plan
@@ -833,7 +853,7 @@ class FineTuneTrainer(_HostPipeline):
         B, _, L = self._x.shape
         training = self.core.training
         st = ctypes.c_void_p(_stream())
-        cfg = plan.cfg(B, L, training, True, self._ws)
+        cfg = plan.cfg(B, L, training, True, self._ws, self.net_flags)
         a2p, rp = ctypes.c_void_p(self._a2.data_ptr()), ctypes.c_void_p(self._r.data_ptr())
         if self._source is not None:      # draw this step's batch on the device (batch index = Adam step counter)
             self._source.fill(self._x, self._t, self.step_dev)
@@ -845,7 +865,7 @@ class FineTuneTrainer(_HostPipeline):
         _call("ralenet_net_fwd", ctypes.byref(cfg), ctypes.byref(plan.P), a2p, rp, st)
         self._conv_fwd(self._r, c3, self._a3, True)
         self._conv_fwd(self._a3, c4, self._out, False)
-        loss, dout, rmse, snr = self.ops.mse_loss_metrics(self._out, self._t)
+        loss, dout, rmse, snr = self.ops.mse_loss_metrics(self._out, self._t, partials=self._loss_partials)
         self._conv_bwd(dout, self._a3, c4, self._da3, False)
         self._conv_bwd(self._da3, self._r, c3, self._dr, True)
         _call("ralenet_net_bwd", ctypes.byref(cfg), ctypes.byref(plan.P), ctypes.byref(plan.G), a2p,
@@ -863,7 +883,8 @@ class FineTuneTrainer(_HostPipeline):
         if source is not self._source:
             self._source = source
             self.graph = None             # the captured step changes
-        _lib.deterministic_guard("FineTuneTrainer (lead-mixing convolution weight gradients)")
+        if not self.deterministic:
+            _lib.deterministic_guard("FineTuneTrainer constructed with deterministic=False")
         if not self.use_graph:
             return self._step_impl()
         if self.graph is None:

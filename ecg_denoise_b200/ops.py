@@ -296,11 +296,14 @@ class Conv1dFn(torch.autograd.Function):
         _lib.call("ralenet_conv1d_fwd", a, _stream())
         ctx.save_for_backward(x, w, b)
         ctx.meta = (act, slope)
+        # torch.use_deterministic_algorithms(True) at forward time selects the deterministic backward (as in RalenetFn)
+        ctx.det = torch.are_deterministic_algorithms_enabled()
         return y
 
     @staticmethod
     def backward(ctx, dy):
-        _lib.deterministic_guard("Conv1dFn backward (parameter gradients accumulated with atomics)")
+        if not ctx.det:
+            _lib.deterministic_guard("Conv1dFn backward of a forward run without torch.use_deterministic_algorithms(True)")
         x, w, b = ctx.saved_tensors
         act, slope = ctx.meta
         B, Ci, L = x.shape
@@ -312,8 +315,22 @@ class Conv1dFn(torch.autograd.Function):
         d_b = torch.zeros_like(b) if (b is not None and nig[2]) else None
         a = _fill("rl_conv_bwd_args", B=B, L=L, Cin=Ci, Cout=Co, K=K, act=int(act), slope=slope, dy=dy, x=x, w=w,
                   b=_p(b), dx=_p(dx), d_w=_p(d_w), d_b=_p(d_b))
-        _lib.call("ralenet_conv1d_bwd", a, _stream())
+        if ctx.det:
+            conv1d_bwd_det(a, conv1d_slab(B, Ci, Co, K, x.device))
+        else:
+            _lib.call("ralenet_conv1d_bwd", a, _stream())
         return dx, d_w, d_b, None, None
+
+
+def conv1d_slab(B: int, Ci: int, Co: int, K: int, device) -> torch.Tensor:
+    """partial-slab scratch of the deterministic convolution backward (ralenet_conv1d_slab_bytes, float32)."""
+    n = int(_lib.load().ralenet_conv1d_slab_bytes(B, Ci, Co, K))
+    return torch.empty(n // 4, device=device, dtype=torch.float32)
+
+
+def conv1d_bwd_det(a, slab: torch.Tensor) -> None:
+    """ralenet_conv1d_bwd_det: the convolution backward with window-ordered weight / bias gradient sums."""
+    _lib.check(_lib.load().ralenet_conv1d_bwd_det(ctypes.byref(a), slab.data_ptr(), slab.numel() * 4, _stream()))
 
 
 # ------------------------------------------------------------------------------------------------

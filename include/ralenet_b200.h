@@ -291,6 +291,16 @@ typedef struct {
 } rl_conv_bwd_args;
 int ralenet_conv1d_fwd(const rl_conv_fwd_args* a, void* stream);
 int ralenet_conv1d_bwd(const rl_conv_bwd_args* a, void* stream);
+/* deterministic twin of ralenet_conv1d_bwd: same kernels and the same += semantics of d_w / d_b, but every window
+ * stores its weight and bias gradients into its own slot of a partial slab in `slab` (caller-owned scratch of at least
+ * ralenet_conv1d_slab_bytes bytes, any content), and a reduction kernel on the same stream adds the slots in window
+ * order.  The result is bit-identical from run to run for a fixed build, shape and ralenet_set_conv_mma setting,
+ * whatever the scheduling.  dx is a plain store in both functions and equal between them.  Like ralenet_conv1d_bwd,
+ * d_b is only written when d_w is given.  RL_ERR_NULL for a NULL slab, RL_ERR_SHAPE for a short one.
+ * ralenet_conv1d_slab_bytes = 4 * (B*Cout*Cin*K + B*Cout) floats, each of the two regions rounded up to 16 bytes
+ * (0 for a non-positive size). */
+uint64_t ralenet_conv1d_slab_bytes(int32_t B, int32_t Cin, int32_t Cout, int32_t K);
+int ralenet_conv1d_bwd_det(const rl_conv_bwd_args* a, float* slab, uint64_t slab_bytes, void* stream);
 /* k = 13 layers: 1 (default) = implicit-GEMM tensor-core kernels (conv_mma.cu), 0 = scalar FMA kernels (stem_head.cu).
  * Same function; A/B switch, initial value from RALENET_CONV_MMA.  Returns the previous setting. */
 int ralenet_set_conv_mma(int on);
